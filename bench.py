@@ -2,6 +2,7 @@
 """Benchmark of the nexoclom hot path on B200 (see DESIGN.md section 6).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--packets P] [--impl reference]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic packets: rewind the
 resident initial state, K2 adaptive integration, K4 radiance image (800x800) --
@@ -14,6 +15,17 @@ buffers: Output(inputs, n, X0=<pinned host columns>) -> ModelImage.  The other k
 path ride along as flat `config` keys: K1 (warm), K4 on an all-live state, K3 on configs[2],
 K5 for 1e5 lines of sight incl. its host preparation, and -- at N > 1 -- an assertion that
 the all-reduced product of two shards equals the single-rank product.
+
+`--dump-outputs DIR` writes what the last timed step computed, so that two builds can be
+compared output for output (the inputs depend only on the arguments): `image.npy` and
+`packet_counts.npy` (the 800x800 radiance image and packet counts of one step, all ranks),
+`step_totals.npy` (attempted, accepted steps of rank 0's K2) and, for a fixed seeded sample of
+at most 2^18 of rank 0's packets, `packet_ids.npy`, `final_state.npy` (time, x, y, z, vx, vy,
+vz, frac) and the per-packet `attempted_steps.npy` / `accepted_steps.npy`.  All float64,
+under 34 MB in all.  `image` is the image accumulated over the K timed steps divided by K, and
+K4 adds with atomics in no fixed order: it matches between runs and builds only to rounding,
+not bit for bit (compare it with a relative tolerance); the other arrays of a build repeat
+exactly.
 """
 import argparse
 import json
@@ -26,6 +38,10 @@ import time
 import numpy as np
 
 REPO = os.path.dirname(os.path.abspath(__file__))
+# the bench leaves the source tree untouched (it may be read-only): no bytecode caches there,
+# in this process or in the worker processes it spawns
+sys.dont_write_bytecode = True
+os.environ['PYTHONDONTWRITEBYTECODE'] = '1'
 sys.path.insert(0, REPO)
 sys.path.insert(0, os.path.join(REPO, 'tests'))
 
@@ -207,6 +223,27 @@ def synthetic_los(nlos, seed=1):
     return np.ascontiguousarray(np.concatenate([x_sc, bore])), np.ascontiguousarray(dplan)
 
 
+DUMP_SAMPLE = 1 << 18        # packets of the final state written by --dump-outputs
+DUMP_SEED = 12345
+
+
+def dump_outputs(dest, eng, img, cnt, steps, first_id):
+    """What the last of `steps` timed steps computed, as float64 .npy files in `dest` (see the
+    module docstring).  The engine still holds that step's final state and step counts; the
+    context-owned image summed the same packets once per step."""
+    n = eng.n
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, min(n, DUMP_SAMPLE), replace=False))
+    state = eng.export_state()
+    att, acc = eng.export_stats()
+    out = {'image': img / steps, 'packet_counts': cnt // steps,
+           'step_totals': [int(att.sum(dtype=np.int64)), int(acc.sum(dtype=np.int64))],
+           'packet_ids': first_id + idx, 'final_state': state[:, idx].T,
+           'attempted_steps': att[idx], 'accepted_steps': acc[idx]}
+    os.makedirs(dest, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(dest, name + '.npy'), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def run_gpu(args):
     import torch
     import torch.distributed as dist
@@ -345,6 +382,8 @@ def run_gpu(args):
     live_hits = int(cnt_run.sum())
     extras['image_hits_per_step_all_ranks'] = live_hits // args.steps
     x0_dev_cols = None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, img_run, cnt_run, args.steps, first_id)
 
     # ---- multi-rank product check: all-reduced == recomputed on rank 0 ------------------
     if world > 1:
@@ -687,7 +726,13 @@ def main():
                     help='packets per GPU of the configs[2] leg (361 steps each; 1e8 / 8 GPUs)')
     ap.add_argument('--check-packets', type=int, default=200_000,
                     help='packets per shard of the multi-rank product check')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step computed to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs writes the products of the GPU path (--impl b200)')
     if args.impl == 'reference':
         return run_reference(args)
     return run_gpu(args)

@@ -1,18 +1,22 @@
 """The reference's own boundary regression (tests/unit_tests/Initial_state/
-test_input_classes.py:17-143), restated against THIS package's Input class and run on the
-reference's own inputfiles where they lie (tests/test_data/inputfiles/*.input; build
-container only -- skipped where /root/reference is absent).  Also test_SSObject.py:6-34."""
+test_input_classes.py:17-143), restated against THIS package's Input class.  The per-group
+cases read tests/golden/inputfiles/*.input, which carry the settings that test's inputfiles
+(tests/test_data/inputfiles/) are asserted to hold; the reference's whole inputfile directory
+and its surface map are read where the reference source tree is present (refimport.REF, as
+for the other cross-checks against the reference).  Also test_SSObject.py:6-34."""
 import os
 
 import numpy as np
 import pytest
 
+import refimport
 from nexoclom_b200 import Input, SSObject
 from nexoclom_b200.units import Quantity
 
-INPUTS = os.path.join(os.environ.get('NEXOCLOM_REFERENCE', '/root/reference'), 'tests',
-                      'test_data', 'inputfiles')
-pytestmark = pytest.mark.skipif(not os.path.isdir(INPUTS), reason='reference tree not present')
+INPUTS = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'inputfiles')
+REF_INPUTS = os.path.join(refimport.REF, 'tests', 'test_data', 'inputfiles')
+needs_reference = pytest.mark.skipif(not os.path.isdir(REF_INPUTS),
+                                     reason='reference tree not present')
 
 
 def rad(v):
@@ -82,10 +86,11 @@ def test_spatial_dist():
                        'latitude': (rad(0), rad(0.79)), 'exobase': 2.1})
 
 
+@needs_reference
 def test_every_reference_inputfile_parses():
-    for fn in sorted(os.listdir(INPUTS)):
+    for fn in sorted(os.listdir(REF_INPUTS)):
         if fn.endswith('.input'):
-            inp = Input(os.path.join(INPUTS, fn))
+            inp = Input(os.path.join(REF_INPUTS, fn))
             assert inp.geometry.planet.object is not None, fn
 
 
@@ -100,7 +105,7 @@ def test_ssobject():
     assert io.type == 'Moon' and io.orbits == 'Jupiter' and io.GM.value < 0
 
 
-MAPFILE = os.path.join(os.path.dirname(INPUTS), 'surface_maps', 'Orbit3576.Ca.pkl')
+MAPFILE = os.path.join(os.path.dirname(REF_INPUTS), 'surface_maps', 'Orbit3576.Ca.pkl')
 
 
 @pytest.mark.skipif(not os.path.exists(MAPFILE), reason='reference surface map not present')
@@ -115,7 +120,7 @@ def test_surface_map_source_with_the_references_own_map(tmp_path):
     from nexoclom_b200.runsetup import RunSetup
     from nexoclom_b200.sourcemap import SourceMap
     from oracle import initial_state
-    src = open(os.path.join(INPUTS, 'Ca.surfacemap.maxwellian.input')).read()
+    src = open(os.path.join(REF_INPUTS, 'Ca.surfacemap.maxwellian.input')).read()
     f = tmp_path / 'map.input'
     f.write_text(src + f'\nSpatialDist.mapfile = {MAPFILE}\n')
     setup = RunSetup(Input(str(f)))
