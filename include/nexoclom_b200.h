@@ -283,6 +283,19 @@ int nx_los_used_fill(nx_ctx* ctx, long long n, long long nlos, const double* los
                      const double* dist_from_plan, const nx_los_params* lp,
                      const long long* used_offsets, uint32_t* used_indices);
 
+/* ---- K7: number density at sample points (ModelDensity) ------------------------
+ * Over the rows of the bound packet table (or the slab), float32-rounded, frac == 0 rows
+ * dropped: a row is a member of ball i when d2 <= radius[i]^2, with dx = x - pts[i] etc. and
+ * d2 = (dx*dx + dy*dy) + dz*dz, every operation an IEEE float64 op rounded to nearest.
+ * pts[3*npts] SoA: x[npts], y[npts], z[npts] in R_p (the frame of Output.X);
+ * radius[npts] > 0 in R_p.  ADDS to the caller's buffers (several tables can be summed):
+ * s1[i] += sum frac, s2[i] += sum frac^2, count[i] += member rows.  Counts are exact; the
+ * sums are atomics, so their last bits depend on the order of the additions.
+ * Resets the candidate pairs nx_los_accumulate_counted keeps for nx_los_used_fill.        */
+int nx_density_accumulate(nx_ctx* ctx, long long n, long long npts, const double* pts,
+                          const double* radius, double* s1, double* s2,
+                          unsigned long long* count);
+
 /* ---- K6: source maps (data_simulation/make_source_map.py:11-175) ----------------
  * Whole-planet and per-grid-point (haversine ball of radius smear_radius*cos(lat_point),
  * sklearn BallTree.query_radius) histograms of the initial states.  All arrays are host

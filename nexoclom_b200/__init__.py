@@ -2,17 +2,18 @@
 
 Public API mirrors the reference's ``nexoclom/__init__.py:9-14``.  Importing the
 package needs neither PostgreSQL nor astropy; creating an ``Output`` /
-``ModelImage`` / ``LOSResult`` needs the built CUDA library and a GPU (there is
-no CPU fallback).
+``ModelImage`` / ``ModelDensity`` / ``LOSResult`` needs the built CUDA library and a
+GPU (there is no CPU fallback).
 """
 from .Input import Input
 from .Output import Output
 from .ModelImage import ModelImage
+from .ModelDensity import ModelDensity
 from .LOSResult import LOSResult
 from .LOSResultFitted import LOSResultFitted
 from .solarsystem import SSObject
 from .input_classes import InputError
 
-__all__ = ['Input', 'Output', 'ModelImage', 'LOSResult', 'LOSResultFitted', 'SSObject',
-           'InputError']
+__all__ = ['Input', 'Output', 'ModelImage', 'ModelDensity', 'LOSResult', 'LOSResultFitted',
+           'SSObject', 'InputError']
 __version__ = '0.1.0'

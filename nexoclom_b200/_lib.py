@@ -152,6 +152,8 @@ def load():
                              c_u32_p],
         'nx_los_used': [vp, i64, i64, c_double_p, c_double_p, C.POINTER(LosParams), c_i64_p,
                         c_i64_p, c_u32_p],
+        'nx_density_accumulate': [vp, i64, i64, c_double_p, c_double_p, c_double_p, c_double_p,
+                                  C.POINTER(u64)],
         'nx_source_map': [vp, i64, C.POINTER(SourceMapParams)] + [c_double_p] * 9 +
                          [c_double_p] * 4 + [c_i64_p] * 2 + [c_double_p] * 4,
         'nx_state_device_ptr': [vp, C.c_int, C.POINTER(vp)],

@@ -118,7 +118,7 @@ struct nx_ctx {
   // grow-only device scratch, one slot per temporary of the product calls: no cudaMalloc /
   // cudaFree (an implicit device synchronisation each) on the calls LOSResult / ModelImage
   // make once per output file, and nothing to leak on an error path
-  struct Scratch { void* p = nullptr; size_t bytes = 0; } scr[24];
+  struct Scratch { void* p = nullptr; size_t bytes = 0; } scr[32];
   int img_nx = 0, img_nz = 0;  // shape of the context-owned image scratch (nx_image_begin)
   void* pinned = nullptr;      // grow-only pinned staging for small D2H results (image, LOS columns)
   size_t pinned_bytes = 0;
@@ -268,8 +268,9 @@ static int alloc_los_work(nx_ctx* ctx, long long n) {
 
 enum { SCR_IMG, SCR_CNT, SCR_LOS, SCR_DIST, SCR_RAD, SCR_NP, SCR_INC, SCR_NBALL, SCR_LADDER,
        SCR_WID2, SCR_ORDER, SCR_NUSED, SCR_CURSOR, SCR_OFF, SCR_IDX, SCR_SM_IN, SCR_SM_PTS,
-       SCR_SM_OUT, SCR_SM_CNT, SCR_TMP, SCR_IMG_OUT, SCR_DD, SCR_KEY, SCR_NSLOTS };
-static_assert(SCR_NSLOTS <= 24, "nx_ctx::scr is too small");
+       SCR_SM_OUT, SCR_SM_CNT, SCR_TMP, SCR_IMG_OUT, SCR_DD, SCR_KEY, SCR_DENS_IN, SCR_DENS_OUT,
+       SCR_DENS_IDX, SCR_NSLOTS };
+static_assert(SCR_NSLOTS <= 32, "nx_ctx::scr is too small");
 static int scratch_bytes(nx_ctx* ctx, int slot, size_t bytes, void** out) {
   nx_ctx::Scratch& sc = ctx->scr[slot];
   if (bytes > sc.bytes) {
@@ -1625,6 +1626,90 @@ int nx_los_used(nx_ctx* ctx, long long n, long long nlos, const double* los,
       cudaMemcpyAsync(used_indices, d_idx, (size_t)total * sizeof(unsigned), cudaMemcpyDeviceToHost, ctx->stream);
     cudaError_t e = cudaStreamSynchronize(ctx->stream);
     if (e != cudaSuccess) { ctx->err = cudaGetErrorString(e); r = -(int)e; }
+  }
+  return r;
+}
+
+// ---- K7: number density at sample points (ModelDensity) ------------------------------------
+// The rows go through K5's cell grid (built again here, with the f32 records: this resets the
+// candidate pairs K5 keeps, which ENTER drops); the points are processed in Morton order of
+// 0.4 R_p cells over +-6.4 R_p, so that warps that run together stream the same cells.
+int nx_density_accumulate(nx_ctx* ctx, long long n, long long npts, const double* pts,
+                          const double* radius, double* s1, double* s2,
+                          unsigned long long* count) {
+  ENTER(ctx);
+  if (n < 0 || npts < 0) { ctx->err = "nx_density_accumulate: negative size"; return -1; }
+  if (n > resident_rows(ctx)) { ctx->err = "n exceeds resident packets"; return -1; }
+  if (n >= (1LL << 32)) { ctx->err = "more than 2^32 packets per GPU"; return -1; }
+  if (n == 0 || npts == 0) return 0;
+  if (!pts || !radius || !s1 || !s2 || !count) { ctx->err = "nx_density_accumulate: null argument"; return -1; }
+  for (long long i = 0; i < npts; ++i) {
+    if (!std::isfinite(pts[i]) || !std::isfinite(pts[npts + i]) || !std::isfinite(pts[2 * npts + i]) ||
+        !std::isfinite(radius[i]) || !(radius[i] > 0.0)) {
+      ctx->err = "nx_density_accumulate: points and radii must be finite, radii > 0";
+      return -1;
+    }
+  }
+  { int r0 = materialize(ctx); if (r0) return r0; }
+  // Morton order (counting sort of 15-bit keys)
+  std::vector<unsigned> key((size_t)npts), order((size_t)npts), hist(NX_LOS_KEY_BINS + 1, 0u);
+  for (long long i = 0; i < npts; ++i) {
+    unsigned k = 0;
+    for (int a = 0; a < 3; ++a) {
+      double v = (pts[a * npts + i] + 6.4) / 0.4;
+      v = v < 0.0 ? 0.0 : (v > 31.0 ? 31.0 : v);
+      const unsigned q = (unsigned)v;
+      for (int b = 0; b < 5; ++b) k |= ((q >> b) & 1u) << (3 * b + a);
+    }
+    key[i] = k;
+    ++hist[k + 1];
+  }
+  for (int k = 0; k < NX_LOS_KEY_BINS; ++k) hist[k + 1] += hist[k];
+  for (long long i = 0; i < npts; ++i) order[hist[key[i]]++] = (unsigned)i;
+
+  const size_t np = (size_t)npts;
+  const size_t nb = np < (size_t)NX_DENSITY_BATCH ? np : (size_t)NX_DENSITY_BATCH;
+  double *d_in = nullptr, *d_out = nullptr;
+  unsigned* d_idx = nullptr;
+  SCR(SCR_DENS_IN, d_in, 4 * np);                   // x, y, z, radius
+  SCR(SCR_DENS_OUT, d_out, 3 * np);                 // s1, s2, count (u64)
+  SCR(SCR_DENS_IDX, d_idx, np + 6 * nb + 2 * nb + 2);   // order, box, nitem, item_off, cursor
+  unsigned* d_order = d_idx;
+  int* d_box = reinterpret_cast<int*>(d_idx + np);
+  unsigned* d_nitem = d_idx + np + 6 * nb;
+  unsigned* d_off = d_nitem + nb;
+  unsigned* d_cursor = d_off + nb + 1;
+  double* d_s1 = d_out;
+  double* d_s2 = d_out + np;
+  unsigned long long* d_cnt = reinterpret_cast<unsigned long long*>(d_out + 2 * np);
+  CK(cudaMemcpyAsync(d_in, pts, 3 * np * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(d_in + 3 * np, radius, np * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(d_order, order.data(), np * sizeof(unsigned), cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemsetAsync(d_out, 0, 3 * np * sizeof(double), ctx->stream));
+  int r = alloc_los_work(ctx, n);
+  if (r == 0) r = begin_timed(ctx);
+  int nlaunch = 6;
+  if (r == 0) {
+    LosParams lp{};
+    lp.round_f32 = 1;
+    lp.skip_dead = 1;
+    cudaError_t e = launch_los_grid_build(ctx->stream, ctx->device, state_cols(ctx), n, lp, ctx->losw);
+    if (e == cudaSuccess)
+      e = launch_density(ctx->stream, ctx->device, ctx->losw, npts, d_in, d_in + 3 * np, d_order,
+                         d_box, d_nitem, d_off, d_cursor, d_s1, d_s2, d_cnt, &nlaunch);
+    if (e != cudaSuccess) { ctx->err = cudaGetErrorString(e); r = -(int)e; }
+  }
+  if (r == 0) r = end_timed(ctx, nlaunch);
+  if (r == 0) {
+    std::vector<double> out(3 * np);
+    CK(cudaMemcpyAsync(out.data(), d_out, 3 * np * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    const unsigned long long* c = reinterpret_cast<const unsigned long long*>(out.data() + 2 * np);
+    for (size_t i = 0; i < np; ++i) {
+      s1[i] += out[i];
+      s2[i] += out[np + i];
+      count[i] += c[i];
+    }
   }
   return r;
 }

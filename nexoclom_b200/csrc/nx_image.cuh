@@ -226,4 +226,17 @@ NX_HD double los_weight(const LosRay& L, const LosParams& lp, const GTables& G,
   return mul_rn(wt, lit ? 1.0 : 0.0);
 }
 
+// ---------------------------------------------------------------------------
+// Number density (K7): is the saved row (x, y, z), float32 values widened to double, inside
+// the ball of radius r around p?  d2 = (dx*dx + dy*dy) + dz*dz <= r*r, every operation an
+// IEEE float64 op rounded to nearest, no contraction: NumPy's order for
+// ((X - p)**2).sum(axis=1) <= r**2 on a float64 copy of the float32 columns.
+// ---------------------------------------------------------------------------
+NX_HD bool density_member(double x, double y, double z, double px, double py, double pz,
+                          double r) {
+  const double dx = sub_rn(x, px), dy = sub_rn(y, py), dz = sub_rn(z, pz);
+  const double d2 = add_rn(add_rn(mul_rn(dx, dx), mul_rn(dy, dy)), mul_rn(dz, dz));
+  return d2 <= mul_rn(r, r);
+}
+
 }  // namespace nx

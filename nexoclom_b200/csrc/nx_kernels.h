@@ -94,6 +94,16 @@ cudaError_t launch_los_resolve(cudaStream_t st, LosGridWork& w, unsigned long lo
                                unsigned long long* nused, const long long* used_off,
                                unsigned long long* used_cursor, unsigned* used_idx);
 
+// K7 number density over the grid launch_los_grid_build made with round_f32 = 1 (F32
+// records): pts SoA with stride npts, order = the points' processing order; box[6 * B],
+// nitem[B], item_off[B + 1] scratch for B = min(npts, 2^20) points, cursor one u32.
+// s1 / s2 / count are added to.
+cudaError_t launch_density(cudaStream_t st, int device, const LosGridWork& w, long long npts,
+                           const double* pts, const double* rad, const unsigned* order,
+                           int* box, unsigned* nitem, unsigned* item_off, unsigned* cursor,
+                           double* s1, double* s2, unsigned long long* count, int* nlaunch);
+#define NX_DENSITY_BATCH (1 << 20)  // points per plan / scan / query round (item ids fit u32)
+
 // per-call preparation of the lines of sight on the device (nx_los_grid.cu)
 #define NX_LOS_KEY_BINS 32768
 cudaError_t launch_los_prepare(cudaStream_t st, const double* los, long long nlos, double outeredge,

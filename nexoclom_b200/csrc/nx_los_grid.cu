@@ -712,4 +712,145 @@ cudaError_t launch_los_resolve(cudaStream_t st, LosGridWork& w, unsigned long lo
   return cudaGetLastError();
 }
 
+// ---------------------------------------------------------------------------
+// K7: number density, sums over the saved rows inside a ball around every sample point
+// (ModelDensity).  The rows are the ones K5 reads (float32-rounded, frac == 0 dropped), in
+// the same cell order, so the grid is launch_los_grid_build's.
+//   k_density_plan: per point (in the host's Morton order) the cell box of [p - r, p + r]
+//                   per axis (cell_of is monotone: an index range per axis) and the number
+//                   of work items, one per 32 (ix, iy) columns of the box;
+//   scan          : the three K5 scan kernels turn the item counts into item offsets;
+//   k_density     : persistent warps take items from a ticket counter; lane c of the warp
+//                   finds the packet range of column c of the item (the z cells of the box),
+//                   then the warp streams the ranges, coalesced, through the exact membership
+//                   test (nx_image.cuh: density_member) and adds S1 = sum frac,
+//                   S2 = sum frac^2 and the member count of the item to the point's totals
+//                   with f64 / u64 atomics.  A ball near the planet spans hundreds of columns
+//                   and most of the packets: its items spread over many warps instead of
+//                   keeping one warp busy after the others are done.
+// ---------------------------------------------------------------------------
+#define NX_DENSITY_WARPS 8
+#define NX_DENSITY_MINBLOCKS 4      // <= 64 registers: 32 resident warps per SM
+#define NX_DENSITY_COLS 32          // (ix, iy) columns per work item (one per lane)
+
+__global__ void __launch_bounds__(256)
+k_density_plan(long long npts, long long stride, const double* __restrict__ pts,
+               const double* __restrict__ rad, const unsigned* __restrict__ order, LosGrid g,
+               int* __restrict__ box, unsigned* __restrict__ nitem) {
+  const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= npts) return;
+  const long long i = order[j];
+  const double p[3] = {pts[i], pts[stride + i], pts[2 * stride + i]};
+  // a member's |x - p| can exceed r by the rounding of d2: pad the box by far more
+  const double rr = rad[i] * (1.0 + 1e-9) + 1e-12;
+  int lo[3], hi[3];
+  bool empty = !(rr > 0.0);
+#pragma unroll
+  for (int a = 0; a < 3; ++a) {
+    if (p[a] - rr > g.half || p[a] + rr < -g.half) empty = true;       // outside the packet cube
+    lo[a] = cell_of(p[a] - rr, g);
+    hi[a] = cell_of(p[a] + rr, g);
+  }
+#pragma unroll
+  for (int a = 0; a < 3; ++a) { box[6 * j + 2 * a] = lo[a]; box[6 * j + 2 * a + 1] = hi[a]; }
+  const unsigned ncol = (unsigned)((hi[0] - lo[0] + 1) * (hi[1] - lo[1] + 1));
+  nitem[j] = empty ? 0u : (ncol + NX_DENSITY_COLS - 1) / NX_DENSITY_COLS;
+}
+
+__global__ void __launch_bounds__(32 * NX_DENSITY_WARPS, NX_DENSITY_MINBLOCKS)
+k_density(LosSorted S, LosGrid g, const unsigned* __restrict__ start, long long npts,
+          const int* __restrict__ box, const unsigned* __restrict__ item_off,
+          const unsigned* __restrict__ nitems, const unsigned* __restrict__ order, long long stride,
+          const double* __restrict__ pts, const double* __restrict__ rad, double* __restrict__ s1,
+          double* __restrict__ s2, unsigned long long* __restrict__ count,
+          unsigned* __restrict__ cursor) {
+  const unsigned lane = threadIdx.x & 31u;
+  const float4* __restrict__ recs = reinterpret_cast<const float4*>(S.pos);
+  const float* __restrict__ fracs = reinterpret_cast<const float*>(S.frac);
+  const unsigned total = *nitems;
+  for (;;) {
+    unsigned t = 0;
+    if (lane == 0) t = atomicAdd(cursor, 1u);
+    t = __shfl_sync(FULL_MASK, t, 0);
+    if (t >= total) return;
+    // the point of item t: the last slot j with item_off[j] <= t (item_off[npts] = total > t)
+    long long lo = 0, hi = npts;
+    while (hi - lo > 1) {
+      const long long mid = (lo + hi) >> 1;
+      if (__ldg(item_off + mid) <= t) lo = mid; else hi = mid;
+    }
+    const long long j = lo;
+    const long long i = order[j];
+    const double px = pts[i], py = pts[stride + i], pz = pts[2 * stride + i], r = rad[i];
+    const int ix0 = box[6 * j], ix1 = box[6 * j + 1], iy0 = box[6 * j + 2], iy1 = box[6 * j + 3];
+    const int iz0 = box[6 * j + 4], iz1 = box[6 * j + 5];
+    const int ny = iy1 - iy0 + 1, ncol = (ix1 - ix0 + 1) * ny;
+    const int c0 = (int)(t - item_off[j]) * NX_DENSITY_COLS;
+    const int c = c0 + (int)lane;
+    unsigned p0v = 0u, p1v = 0u;
+    if (c < ncol) {
+      const unsigned row = (unsigned)(((ix0 + c / ny) * g.G + iy0 + c % ny) * g.G);
+      p0v = __ldg(start + row + iz0);
+      p1v = __ldg(start + row + iz1 + 1);
+    }
+    const int nc = min(NX_DENSITY_COLS, ncol - c0);
+    double a1 = 0.0, a2 = 0.0;
+    unsigned m = 0;
+    for (int k = 0; k < nc; ++k) {
+      const unsigned p0 = __shfl_sync(FULL_MASK, p0v, k), p1 = __shfl_sync(FULL_MASK, p1v, k);
+      for (unsigned qb = p0; qb < p1; qb += 64) {
+        const unsigned q0 = qb + lane, q1 = q0 + 32u;
+        float4 ra, rb;
+        if (q0 < p1) ra = __ldg(recs + q0);
+        if (q1 < p1) rb = __ldg(recs + q1);
+        if (q0 < p1 && density_member(ra.x, ra.y, ra.z, px, py, pz, r)) {
+          const double f = (double)__ldg(fracs + q0);
+          a1 += f; a2 += f * f; ++m;           // f * f: exact (24-bit mantissas)
+        }
+        if (q1 < p1 && density_member(rb.x, rb.y, rb.z, px, py, pz, r)) {
+          const double f = (double)__ldg(fracs + q1);
+          a1 += f; a2 += f * f; ++m;
+        }
+      }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      a1 += __shfl_xor_sync(FULL_MASK, a1, o);
+      a2 += __shfl_xor_sync(FULL_MASK, a2, o);
+      m += __shfl_xor_sync(FULL_MASK, m, o);
+    }
+    if (lane == 0 && m) {
+      atomicAdd(s1 + i, a1);
+      atomicAdd(s2 + i, a2);
+      atomicAdd(count + i, (unsigned long long)m);
+    }
+  }
+}
+
+cudaError_t launch_density(cudaStream_t st, int device, const LosGridWork& w, long long npts,
+                           const double* pts, const double* rad, const unsigned* order,
+                           int* box, unsigned* nitem, unsigned* item_off, unsigned* cursor, double* s1,
+                           double* s2, unsigned long long* count, int* nlaunch) {
+  int sms = 148;
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+  cudaError_t e;
+  for (long long first = 0; first < npts; first += NX_DENSITY_BATCH) {
+    const long long nb = npts - first < NX_DENSITY_BATCH ? npts - first : NX_DENSITY_BATCH;
+    k_density_plan<<<(unsigned)((nb + 255) / 256), 256, 0, st>>>(nb, npts, pts, rad, order + first,
+                                                                  w.grid, box, nitem);
+    // item counts -> offsets; item_off[nb] = the item total
+    const int nsb = (int)((nb + NX_SCAN_ELEMS - 1) / NX_SCAN_ELEMS);
+    k_scan_partial<<<nsb, 1024, 0, st>>>(nitem, item_off, w.block_sum, (int)nb);
+    k_scan_top<<<1, 1024, 0, st>>>(w.block_sum, nsb, w.total);
+    k_scan_add<<<nsb, 1024, 0, st>>>(item_off, w.block_sum, (int)nb, w.total);
+    if ((e = cudaMemsetAsync(cursor, 0, sizeof(unsigned), st)) != cudaSuccess) return e;
+    // the item total stays on the device: the warps read it, the host does not wait for it
+    k_density<<<(unsigned)sms * NX_DENSITY_MINBLOCKS, 32 * NX_DENSITY_WARPS, 0, st>>>(
+        w.sorted, w.grid, w.start, nb, box, item_off, w.total, order + first, npts, pts, rad, s1,
+        s2, count, cursor);
+    if (nlaunch) *nlaunch += 5;
+  }
+  return cudaGetLastError();
+}
+
 }  // namespace nx

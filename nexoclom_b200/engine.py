@@ -491,6 +491,25 @@ class Engine:
             C.byref(los_params), C.c_void_p(rad_dev), C.c_void_p(npk_dev),
             C.c_void_p(inc_dev)), 'nx_los_accumulate_dev')
 
+    def density_accumulate(self, points, radius, s1, s2, count, n=None):
+        """K7 of the bound packet table (or the slab): ADDS to ``s1`` (sum of frac), ``s2``
+        (sum of frac**2) and ``count`` (member rows) of every ball.  ``points``: (npts, 3) in
+        R_p; ``radius``: (npts,) in R_p; ``s1`` / ``s2`` float64 and ``count`` int64 arrays of
+        length npts, C-contiguous (updated in place)."""
+        n = self.n if n is None else n
+        pts = np.ascontiguousarray(np.asarray(points, dtype=np.float64).T)
+        rad = as_f64(radius)
+        npts = len(rad)
+        if pts.shape != (3, npts):
+            raise ValueError('points must be (npts, 3) with one radius per point')
+        for a, dt in ((s1, np.float64), (s2, np.float64), (count, np.int64)):
+            if not (isinstance(a, np.ndarray) and a.dtype == dt and a.flags.c_contiguous and
+                    a.shape == (npts,)):
+                raise TypeError('s1 / s2 must be float64 and count int64 arrays of length npts')
+        self._check(self.lib.nx_density_accumulate(
+            self.ctx, int(n), npts, dptr(pts), dptr(rad), dptr(s1), dptr(s2),
+            count.ctypes.data_as(C.POINTER(C.c_ulonglong))), 'nx_density_accumulate')
+        return s1, s2, count
 
     def source_map(self, params, longitude, latitude, speed_kms, altitude, azimuth, frac,
                    point_lon, point_lat, point_radius):
