@@ -283,6 +283,26 @@ int nx_los_used_fill(nx_ctx* ctx, long long n, long long nlos, const double* los
                      const double* dist_from_plan, const nx_los_params* lp,
                      const long long* used_offsets, uint32_t* used_indices);
 
+/* ---- Doppler line profiles along lines of sight (LOSSpectrum) ------------------
+ * The hits of nx_los_accumulate (same test, same rows, same weight w) binned by the velocity
+ * of the row along the boresight, v = ((vx*bx + vy*by) + vz*bz) * vscale [km/s, planet rest
+ * frame, positive = receding], every operation float64 rounded to nearest; vx, vy, vz are
+ * float32-rounded when lp->round_f32.  Bins follow np.histogram on edges = linspace(vmin,
+ * vmax, nbins + 1) (vmax belongs to the last bin).  Always runs the cell-grid search; more
+ * than 2^32 packets per GPU are rejected.                                                  */
+typedef struct nx_spectrum_params {
+  double vmin, vmax;      /* km/s; edges = linspace(vmin, vmax, nbins + 1)          */
+  double vscale;          /* km/s per R_p/s (the planet radius in km)               */
+  int32_t nbins;          /* >= 1                                                   */
+  int32_t reserved;
+} nx_spectrum_params;
+/* spectrum / counts: row-major (nlos, nbins + 2); column 0 = v < vmin, 1..nbins = bins,
+ * nbins + 1 = v > vmax.  Overwritten (like nx_los_accumulate).  Resets the candidate pairs
+ * nx_los_accumulate_counted keeps for nx_los_used_fill.                                 */
+int nx_los_spectrum(nx_ctx* ctx, long long n, long long nlos, const double* los,
+                    const double* dist_from_plan, const nx_los_params* lp,
+                    const nx_spectrum_params* sp, double* spectrum, long long* counts);
+
 /* ---- K7: number density at sample points (ModelDensity) ------------------------
  * Over the rows of the bound packet table (or the slab), float32-rounded, frac == 0 rows
  * dropped: a row is a member of ball i when d2 <= radius[i]^2, with dx = x - pts[i] etc. and

@@ -2,7 +2,8 @@
 
 Public API mirrors the reference's ``nexoclom/__init__.py:9-14``.  Importing the
 package needs neither PostgreSQL nor astropy; creating an ``Output`` /
-``ModelImage`` / ``ModelDensity`` / ``LOSResult`` needs the built CUDA library and a
+``ModelImage`` / ``ModelDensity`` / ``LOSResult`` /
+``LOSSpectrum`` needs the built CUDA library and a
 GPU (there is no CPU fallback).
 """
 from .Input import Input
@@ -10,10 +11,11 @@ from .Output import Output
 from .ModelImage import ModelImage
 from .ModelDensity import ModelDensity
 from .LOSResult import LOSResult
+from .LOSSpectrum import LOSSpectrum
 from .LOSResultFitted import LOSResultFitted
 from .solarsystem import SSObject
 from .input_classes import InputError
 
-__all__ = ['Input', 'Output', 'ModelImage', 'ModelDensity', 'LOSResult', 'LOSResultFitted',
-           'SSObject', 'InputError']
+__all__ = ['Input', 'Output', 'ModelImage', 'ModelDensity', 'LOSResult', 'LOSSpectrum',
+           'LOSResultFitted', 'SSObject', 'InputError']
 __version__ = '0.1.0'

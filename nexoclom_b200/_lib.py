@@ -78,6 +78,14 @@ class LosParams(C.Structure):
     ]
 
 
+class SpectrumParams(C.Structure):
+    """Mirror of ``nx_spectrum_params``."""
+    _fields_ = [
+        ('vmin', C.c_double), ('vmax', C.c_double), ('vscale', C.c_double),
+        ('nbins', C.c_int32), ('reserved', C.c_int32),
+    ]
+
+
 class SourceMapParams(C.Structure):
     """Mirror of ``nx_source_map_params``."""
     _fields_ = [
@@ -152,6 +160,8 @@ def load():
                              c_u32_p],
         'nx_los_used': [vp, i64, i64, c_double_p, c_double_p, C.POINTER(LosParams), c_i64_p,
                         c_i64_p, c_u32_p],
+        'nx_los_spectrum': [vp, i64, i64, c_double_p, c_double_p, C.POINTER(LosParams),
+                            C.POINTER(SpectrumParams), c_double_p, c_i64_p],
         'nx_density_accumulate': [vp, i64, i64, c_double_p, c_double_p, c_double_p, c_double_p,
                                   C.POINTER(u64)],
         'nx_source_map': [vp, i64, C.POINTER(SourceMapParams)] + [c_double_p] * 9 +

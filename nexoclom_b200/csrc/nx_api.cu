@@ -269,7 +269,7 @@ static int alloc_los_work(nx_ctx* ctx, long long n) {
 enum { SCR_IMG, SCR_CNT, SCR_LOS, SCR_DIST, SCR_RAD, SCR_NP, SCR_INC, SCR_NBALL, SCR_LADDER,
        SCR_WID2, SCR_ORDER, SCR_NUSED, SCR_CURSOR, SCR_OFF, SCR_IDX, SCR_SM_IN, SCR_SM_PTS,
        SCR_SM_OUT, SCR_SM_CNT, SCR_TMP, SCR_IMG_OUT, SCR_DD, SCR_KEY, SCR_DENS_IN, SCR_DENS_OUT,
-       SCR_DENS_IDX, SCR_NSLOTS };
+       SCR_DENS_IDX, SCR_SPEC, SCR_NSLOTS };
 static_assert(SCR_NSLOTS <= 32, "nx_ctx::scr is too small");
 static int scratch_bytes(nx_ctx* ctx, int slot, size_t bytes, void** out) {
   nx_ctx::Scratch& sc = ctx->scr[slot];
@@ -1350,7 +1350,7 @@ static void los_prepare(const double* los, long long nlos, const LosParams& lp,
 static int los_run(nx_ctx* ctx, long long n, long long nlos, const double* los_dev,
                    const double* dist_dev, const LosParams& lp, double* rad_dev,
                    unsigned long long* np_dev, unsigned char* inc_dev,
-                   unsigned long long* nused_dev = nullptr) {
+                   unsigned long long* nused_dev = nullptr, const LosSpectrum* spec = nullptr) {
   { int r0 = materialize(ctx); if (r0) return r0; }
   static const bool timing = std::getenv("NX_LOS_TIMING") != nullptr;     // developer aid
   const auto tp0 = std::chrono::steady_clock::now();
@@ -1360,7 +1360,7 @@ static int los_run(nx_ctx* ctx, long long n, long long nlos, const double* los_d
                    std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tp0).count());
   };
   // candidate generation: brute force for small problems, cell grid otherwise
-  const bool use_grid = ctx->los_mode == 2 || nused_dev ||      // (`used` counts: grid path only)
+  const bool use_grid = ctx->los_mode == 2 || nused_dev || spec ||   // (`used` counts, spectra: grid path only)
                         (ctx->los_mode == 0 && (double)n * (double)nlos > 2e9 && n < (1LL << 32));
   const bool want_order = use_grid && ctx->los_order && nlos >= 1024;
   // per-line preparation on the device; the host only turns the longest boresight distance
@@ -1407,7 +1407,7 @@ static int los_run(nx_ctx* ctx, long long n, long long nlos, const double* los_d
       if (e == cudaSuccess)
         e = launch_los_grid(ctx->stream, ctx->losw, nlos, los_dev, dist_dev, d_nball, d_ladder,
                             d_wid2, lp, lc, ctx->gtables, rad_dev, np_dev, inc_dev, nused_dev,
-                            nullptr, nullptr, nullptr, d_order, nused_dev ? &kept : nullptr);
+                            nullptr, nullptr, nullptr, d_order, nused_dev ? &kept : nullptr, spec);
       if (e == cudaSuccess && kept) {
         ctx->los_kept.np = kept; ctx->los_kept.n = n; ctx->los_kept.nlos = nlos;
         ctx->los_kept.bound = ctx->bound; ctx->los_kept.lc = lc;
@@ -1626,6 +1626,67 @@ int nx_los_used(nx_ctx* ctx, long long n, long long nlos, const double* los,
       cudaMemcpyAsync(used_indices, d_idx, (size_t)total * sizeof(unsigned), cudaMemcpyDeviceToHost, ctx->stream);
     cudaError_t e = cudaStreamSynchronize(ctx->stream);
     if (e != cudaSuccess) { ctx->err = cudaGetErrorString(e); r = -(int)e; }
+  }
+  return r;
+}
+
+// ---- Doppler line profiles (LOSSpectrum): K5's hits binned by line-of-sight velocity -------
+int nx_los_spectrum(nx_ctx* ctx, long long n, long long nlos, const double* los,
+                    const double* dist_from_plan, const nx_los_params* lp_,
+                    const nx_spectrum_params* sp_, double* spectrum, long long* counts) {
+  ENTER(ctx);
+  if (!lp_ || !sp_) { ctx->err = "nx_los_spectrum: null argument"; return -1; }
+  if (n < 0 || nlos < 0) { ctx->err = "nx_los_spectrum: negative size"; return -1; }
+  if (n > resident_rows(ctx)) { ctx->err = "n exceeds resident packets"; return -1; }
+  if (n >= (1LL << 32)) { ctx->err = "more than 2^32 packets per GPU"; return -1; }
+  const nx_spectrum_params sp = *sp_;
+  if (sp.nbins < 1) { ctx->err = "nx_los_spectrum: nbins must be >= 1"; return -1; }
+  if (!std::isfinite(sp.vmin) || !std::isfinite(sp.vmax) || !(sp.vmin < sp.vmax)) {
+    ctx->err = "nx_los_spectrum: vmin < vmax, both finite, required";
+    return -1;
+  }
+  if (!std::isfinite(sp.vscale)) { ctx->err = "nx_los_spectrum: vscale must be finite"; return -1; }
+  const long long ncol = (long long)sp.nbins + 2;
+  if ((double)nlos * (double)ncol >= 2147483648.0) {
+    ctx->err = "nx_los_spectrum: nlos * (nbins + 2) must be < 2^31";
+    return -1;
+  }
+  LosParams lp;
+  std::memcpy(&lp, lp_, sizeof(lp));
+  if (lp.quantity != 1) { ctx->err = "Other quantities not set up."; return -1; }
+  if (ctx->gtables.n == 0) { ctx->err = "no g-value tables uploaded"; return -1; }
+  const size_t ncell = (size_t)(nlos * ncol);
+  if (nlos == 0) return 0;
+  if (!los || !dist_from_plan || !spectrum || !counts) { ctx->err = "nx_los_spectrum: null argument"; return -1; }
+  if (n == 0) {
+    std::memset(spectrum, 0, ncell * sizeof(double));
+    std::memset(counts, 0, ncell * sizeof(long long));
+    return 0;
+  }
+  double *d_los = nullptr, *d_dist = nullptr, *d_spec = nullptr;
+  SCR(SCR_LOS, d_los, 6 * (size_t)nlos);
+  SCR(SCR_DIST, d_dist, (size_t)nlos);
+  SCR(SCR_SPEC, d_spec, 2 * ncell);                 // sums, then the u64 counts
+  LosSpectrum spec;
+  const StateCols P = state_cols(ctx);
+  spec.vx = P.c[4];
+  spec.vz = P.c[6];
+  spec.vmin = sp.vmin;
+  spec.vmax = sp.vmax;
+  spec.step = (sp.vmax - sp.vmin) / sp.nbins;       // np.linspace's step
+  spec.vscale = sp.vscale;
+  spec.nbins = sp.nbins;
+  spec.sum = d_spec;
+  spec.count = reinterpret_cast<unsigned long long*>(d_spec + ncell);
+  CK(cudaMemcpyAsync(d_los, los, 6 * (size_t)nlos * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(d_dist, dist_from_plan, (size_t)nlos * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemsetAsync(d_spec, 0, 2 * ncell * sizeof(double), ctx->stream));
+  int r = los_run(ctx, n, nlos, d_los, d_dist, lp, nullptr, nullptr, nullptr, nullptr, &spec);
+  if (r == 0) {
+    static_assert(sizeof(long long) == sizeof(unsigned long long), "");
+    CK(cudaMemcpyAsync(spectrum, d_spec, ncell * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(counts, d_spec + ncell, ncell * sizeof(long long), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
   }
   return r;
 }

@@ -227,6 +227,24 @@ NX_HD double los_weight(const LosRay& L, const LosParams& lp, const GTables& G,
 }
 
 // ---------------------------------------------------------------------------
+// Doppler spectra (LOSSpectrum): the velocity of a hit row along the boresight, in km/s,
+// positive away from the observer, v = ((vx*bx + vy*by) + vz*bz) * vscale, every operation an
+// IEEE float64 op rounded to nearest (vscale = R_p in km).
+// ---------------------------------------------------------------------------
+NX_HD double los_doppler(double vx, double vy, double vz, double bx, double by, double bz,
+                         double vscale) {
+  return mul_rn(add_rn(add_rn(mul_rn(vx, bx), mul_rn(vy, by)), mul_rn(vz, bz)), vscale);
+}
+// Spectrum column of v for edges = np.linspace(vmin, vmax, nbins + 1), step = (vmax - vmin) /
+// nbins: 0 below vmin, 1 + the np.histogram bin inside [vmin, vmax] (vmax in the last bin),
+// nbins + 1 above vmax (NaN included).
+NX_HD int spectrum_column(double v, int nbins, double vmin, double vmax, double step) {
+  if (v < vmin) return 0;
+  if (!(v <= vmax)) return nbins + 1;
+  return hist_bin(v, nbins, vmin, vmax, step) + 1;
+}
+
+// ---------------------------------------------------------------------------
 // Number density (K7): is the saved row (x, y, z), float32 values widened to double, inside
 // the ball of radius r around p?  d2 = (dx*dx + dy*dy) + dz*dz <= r*r, every operation an
 // IEEE float64 op rounded to nearest, no contraction: NumPy's order for

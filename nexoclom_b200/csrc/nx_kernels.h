@@ -76,6 +76,18 @@ struct LosGridWork {
   long long batch_hint = 0;    // lines of sight per batch that half-filled `pairs` last time
   unsigned long long pairs_cap_fixed = 0;   // option "los_pair_cap" (tests: force several batches)
 };
+// Doppler spectrum of the hits instead of the per-line sums (nx_los_spectrum): the exact test
+// and the weight stay K5's; every hit adds its weight and 1 to column spectrum_column(v) of its
+// line (row-major (nlos, nbins + 2)).  vx / vz are columns 4 and 6 of the packet table, read
+// at the hit's row (vy is in the sorted record).
+struct LosSpectrum {
+  const double* vx;
+  const double* vz;
+  double vmin, vmax, step, vscale;
+  int nbins;
+  double* sum;
+  unsigned long long* count;
+};
 cudaError_t launch_los_grid_build(cudaStream_t st, int device, StateCols P, long long n,
                                   const LosParams& lp, LosGridWork& w);
 cudaError_t launch_los_grid(cudaStream_t st, LosGridWork& w, long long nlos,
@@ -85,7 +97,8 @@ cudaError_t launch_los_grid(cudaStream_t st, LosGridWork& w, long long nlos,
                             unsigned long long* npack, unsigned char* included,
                             unsigned long long* nused = nullptr, const long long* used_off = nullptr,
                             unsigned long long* used_cursor = nullptr, unsigned* used_idx = nullptr,
-                            const unsigned* order = nullptr, unsigned long long* kept_pairs = nullptr);
+                            const unsigned* order = nullptr, unsigned long long* kept_pairs = nullptr,
+                            const LosSpectrum* spec = nullptr);
 cudaError_t launch_los_resolve(cudaStream_t st, LosGridWork& w, unsigned long long np, long long nlos,
                                const double* los, const double* dist_plan, const int* nball,
                                const double* ladder, const double* wid2, const LosParams& lp,

@@ -374,7 +374,9 @@ k_los_candidates(LosSorted S, LosGrid g, const unsigned* __restrict__ start, lon
 }
 
 // ---- 4. exact membership + weight, one thread per candidate pair -----------------------
-template <bool F32>
+// SPEC: the Doppler spectrum variant (nx_los_spectrum) -- the same test and weight, added to
+// the hit's (line, velocity column) cell of sp instead of the per-line sums.
+template <bool F32, bool SPEC>
 __global__ void __launch_bounds__(256)
 k_los_resolve(LosSorted S, const uint2* __restrict__ pairs, unsigned long long npairs,
               long long nlos, const double* __restrict__ los,
@@ -383,7 +385,8 @@ k_los_resolve(LosSorted S, const uint2* __restrict__ pairs, unsigned long long n
               LosConsts lc, GTables G, double* __restrict__ radiance,
               unsigned long long* __restrict__ npack, unsigned char* __restrict__ included,
               unsigned long long* __restrict__ nused, const long long* __restrict__ used_off,
-              unsigned long long* __restrict__ used_cursor, unsigned* __restrict__ used_idx) {
+              unsigned long long* __restrict__ used_cursor, unsigned* __restrict__ used_idx,
+              LosSpectrum sp) {
   typedef typename LosRec<F32>::type RecT;
   const unsigned lane = threadIdx.x & 31u;
   const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
@@ -396,6 +399,7 @@ k_los_resolve(LosSorted S, const uint2* __restrict__ pairs, unsigned long long n
     unsigned l = 0xffffffffu;
     double w = 0.0;
     bool hit = false;
+    unsigned cell = 0xffffffffu;       // SPEC: l * (nbins + 2) + velocity column of a hit
     if (valid) {
       const uint2 pr = pairs[i];
       l = pr.x;
@@ -413,10 +417,38 @@ k_los_resolve(LosSorted S, const uint2* __restrict__ pairs, unsigned long long n
         const double fr = F32 ? (double)reinterpret_cast<const float*>(S.frac)[q] : S.frac[q];
         w = los_weight(L, lp, G, lc.sin_dphi, fr, r.w, losrad, dist);
         const unsigned pidx = S.idx[q];
-        if (included) included[pidx] = 1;
-        if (w > 0.0 && used_idx)               // `used` packets (compute_iteration.py:210-211)
-          used_idx[used_off[l] + atomicAdd(&used_cursor[l], 1ull)] = pidx;
+        if (SPEC) {
+          // vx, vz gathered from the table at the hit's row (the records carry x, y, z, vy only)
+          double vx = sp.vx[pidx], vz = sp.vz[pidx];
+          if (lp.round_f32) { vx = round_f32(vx); vz = round_f32(vz); }
+          const double v = los_doppler(vx, r.w, vz, L.bx, L.by, L.bz, sp.vscale);
+          cell = l * (unsigned)(sp.nbins + 2) +
+                 (unsigned)spectrum_column(v, sp.nbins, sp.vmin, sp.vmax, sp.step);
+        } else {
+          if (included) included[pidx] = 1;
+          if (w > 0.0 && used_idx)               // `used` packets (compute_iteration.py:210-211)
+            used_idx[used_off[l] + atomicAdd(&used_cursor[l], 1ull)] = pidx;
+        }
       }
+    }
+    if (SPEC) {
+      // Pairs of one line are adjacent but their velocity columns are not: the lanes with equal
+      // cells combine (the lowest lane adds the group's weights in lane order) before the
+      // global f64 / u64 atomics.
+      const unsigned hitm = __ballot_sync(FULL_MASK, hit);
+      if (hitm) {
+        const unsigned grp = __match_any_sync(FULL_MASK, cell);
+        double acc = 0.0;
+        for (int k = 0; k < 32; ++k) {
+          const double wk = __shfl_sync(FULL_MASK, w, k);
+          if ((grp >> k) & 1u) acc += wk;
+        }
+        if (hit && lane == (unsigned)(__ffs(grp) - 1)) {
+          atomicAdd(&sp.count[cell], (unsigned long long)__popc(grp));
+          if (acc != 0.0) atomicAdd(&sp.sum[cell], acc);
+        }
+      }
+      continue;
     }
     // pairs of one line of sight sit next to each other in the list: one atomic per run of
     // equal l within the warp (segmented reduction over the lanes, in lane order)
@@ -454,6 +486,33 @@ k_los_resolve(LosSorted S, const uint2* __restrict__ pairs, unsigned long long n
 }
 
 // ---- host-side launch sequence ------------------------------------------------------
+// k_los_resolve over np pairs in w.pairs: records F32 or not, spectrum (spec) or per-line sums
+static void launch_resolve_pairs(cudaStream_t st, LosGridWork& w, unsigned long long np, long long nlos,
+                                 const double* los, const double* dist_plan, const int* nball,
+                                 const double* ladder, const double* wid2, const LosParams& lp,
+                                 const LosConsts& lc, const GTables& G, double* radiance,
+                                 unsigned long long* npack, unsigned char* included,
+                                 unsigned long long* nused, const long long* used_off,
+                                 unsigned long long* used_cursor, unsigned* used_idx,
+                                 const LosSpectrum* spec) {
+  int sms = 148, dev = 0;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  long long rb = (long long)((np + 255) / 256);
+  if (rb > (long long)sms * 16) rb = (long long)sms * 16;
+  const LosSpectrum sp = spec ? *spec : LosSpectrum{};
+#define NX_RESOLVE(F32, SPEC)                                                                  \
+  k_los_resolve<F32, SPEC><<<(unsigned)rb, 256, 0, st>>>(                                      \
+      w.sorted, w.pairs, np, nlos, los, dist_plan, nball, ladder, wid2, lp, lc, G, radiance,   \
+      npack, included, nused, used_off, used_cursor, used_idx, sp)
+  if (spec) {
+    if (lp.round_f32) NX_RESOLVE(true, true); else NX_RESOLVE(false, true);
+  } else {
+    if (lp.round_f32) NX_RESOLVE(true, false); else NX_RESOLVE(false, false);
+  }
+#undef NX_RESOLVE
+}
+
 cudaError_t launch_los_grid_build(cudaStream_t st, int device, StateCols P, long long n,
                                   const LosParams& lp, LosGridWork& w) {
   int sms = 148;
@@ -505,7 +564,8 @@ cudaError_t launch_los_grid(cudaStream_t st, LosGridWork& w, long long nlos,
                             unsigned long long* npack, unsigned char* included,
                             unsigned long long* nused, const long long* used_off,
                             unsigned long long* used_cursor, unsigned* used_idx,
-                            const unsigned* order, unsigned long long* kept_pairs) {
+                            const unsigned* order, unsigned long long* kept_pairs,
+                            const LosSpectrum* spec) {
   // Lines of sight go through in batches sized so that the candidate pairs of a batch fit the
   // pair buffer (about half full: the size of the next batch follows the pairs per line of
   // sight seen so far); a batch that overflows is repeated with half as many lines.
@@ -540,18 +600,9 @@ cudaError_t launch_los_grid(cudaStream_t st, LosGridWork& w, long long nlos,
       batch = fit > 1 ? fit : 1;
       continue;
     }
-    if (np) {
-      long long rb = (long long)((np + 255) / 256);
-      if (rb > (long long)sms * 16) rb = (long long)sms * 16;
-      if (lp.round_f32)
-        k_los_resolve<true><<<(unsigned)rb, 256, 0, st>>>(w.sorted, w.pairs, np, nlos, los, dist_plan, nball,
-                                                          ladder, wid2, lp, lc, G, radiance, npack, included,
-                                                          nused, used_off, used_cursor, used_idx);
-      else
-        k_los_resolve<false><<<(unsigned)rb, 256, 0, st>>>(w.sorted, w.pairs, np, nlos, los, dist_plan, nball,
-                                                           ladder, wid2, lp, lc, G, radiance, npack, included,
-                                                           nused, used_off, used_cursor, used_idx);
-    }
+    if (np)
+      launch_resolve_pairs(st, w, np, nlos, los, dist_plan, nball, ladder, wid2, lp, lc, G, radiance,
+                           npack, included, nused, used_off, used_cursor, used_idx, spec);
     // one batch covered every line of sight: its pairs stay valid in w.pairs
     if (kept_pairs) *kept_pairs = (first == 0 && cnt == nlos) ? np : 0ull;
     const bool whole = first == 0 && cnt == nlos;      // the whole sweep fitted one batch
@@ -696,19 +747,8 @@ cudaError_t launch_los_resolve(cudaStream_t st, LosGridWork& w, unsigned long lo
                                unsigned long long* nused, const long long* used_off,
                                unsigned long long* used_cursor, unsigned* used_idx) {
   if (!np) return cudaSuccess;
-  int sms = 148, dev = 0;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  long long rb = (long long)((np + 255) / 256);
-  if (rb > (long long)sms * 16) rb = (long long)sms * 16;
-  if (lp.round_f32)
-    k_los_resolve<true><<<(unsigned)rb, 256, 0, st>>>(w.sorted, w.pairs, np, nlos, los, dist_plan, nball,
-                                                      ladder, wid2, lp, lc, G, radiance, npack, included,
-                                                      nused, used_off, used_cursor, used_idx);
-  else
-    k_los_resolve<false><<<(unsigned)rb, 256, 0, st>>>(w.sorted, w.pairs, np, nlos, los, dist_plan, nball,
-                                                       ladder, wid2, lp, lc, G, radiance, npack, included,
-                                                       nused, used_off, used_cursor, used_idx);
+  launch_resolve_pairs(st, w, np, nlos, los, dist_plan, nball, ladder, wid2, lp, lc, G, radiance,
+                       npack, included, nused, used_off, used_cursor, used_idx, nullptr);
   return cudaGetLastError();
 }
 
