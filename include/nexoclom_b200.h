@@ -303,6 +303,28 @@ int nx_los_spectrum(nx_ctx* ctx, long long n, long long nlos, const double* los,
                     const double* dist_from_plan, const nx_los_params* lp,
                     const nx_spectrum_params* sp, double* spectrum, long long* counts);
 
+/* ---- Doppler-resolved image cubes (ModelImageCube) -----------------------------
+ * K4's rows, pixel and weight (nx_image_add: same rows, occulted / shadowed rows counted with
+ * w = 0) with a velocity axis: v = ((vx*M[3] + vy*M[4]) + vz*M[5]) * sp->vscale [km/s], every
+ * operation float64 rounded to nearest, M the observer rotation of ip (row 1: the observer sits
+ * at -y_obs, so v > 0 recedes; planet rest frame); vx, vy, vz float32-rounded when
+ * ip->round_f32.  Columns as nx_los_spectrum: 0 = v < vmin, 1..nbins = np.histogram on
+ * linspace(vmin, vmax, nbins + 1), nbins + 1 = v > vmax (NaN included).  Layout row-major
+ * (nx, nz, nbins + 2), so the sum over the last axis is K4's image and counts.
+ * begin allocates and zeroes the context-owned cube (f64 sums + i64 counts, 16 B per cell;
+ * nx * nz * (nbins + 2) < 2^31), add bins the bound packet table (or the slab) into it (any
+ * number of tables; checks dims, the velocity axis, g-tables for radiance and n before any
+ * launch), fetch copies the raw sums and counts to the host (either may be NULL; page-locked
+ * destinations receive the DMA directly), allreduce_total is the one collective of a sharded
+ * cube (*total rides along, as nx_image_allreduce_total), end releases the device buffers.
+ * None of these touch the image scratch or the candidate pairs nx_los_used_fill reads.      */
+int nx_cube_begin(nx_ctx* ctx, int nx, int nz, int nbins);
+int nx_cube_add(nx_ctx* ctx, long long n, const nx_image_params* ip,
+                const nx_spectrum_params* sp);
+int nx_cube_fetch(nx_ctx* ctx, double* cube, long long* counts);
+int nx_cube_allreduce_total(nx_ctx* ctx, nx_comm* comm, double* total);
+int nx_cube_end(nx_ctx* ctx);
+
 /* ---- K7: number density at sample points (ModelDensity) ------------------------
  * Over the rows of the bound packet table (or the slab), float32-rounded, frac == 0 rows
  * dropped: a row is a member of ball i when d2 <= radius[i]^2, with dx = x - pts[i] etc. and

@@ -58,40 +58,12 @@ class _Hist2d:
 
 class ModelImage(ModelResult):
     def __init__(self, inputs, params, overwrite=False, distribute=None, device=None):
-        from .sharding import local_device, allreduce_sum, nccl_comm
+        from .sharding import allreduce_sum, nccl_comm
         super().__init__(inputs, params)
         self.type = 'image'
-        self.origin = self.params.get('origin', inputs.geometry.planet)
-        self.unit = def_unit('R_' + self.origin.object, 'length',
-                             float(self.origin.radius.value) * 1e3)
-        R = lambda v: Quantity(v, self.unit)      # noqa: E731
-
-        dimtemp = self.params.get('dims', '800,800').split(',')
-        self.dims = [int(dimtemp[0]), int(dimtemp[1])]
-        centtemp = self.params.get('center', '0,0').split(',')
-        self.center = [R(float(centtemp[0])), R(float(centtemp[1]))]
-        widtemp = self.params.get('width', '8,8').split(',')
-        self.width = [R(float(widtemp[0])), R(float(widtemp[1]))]
-        self.subobslongitude = Quantity(float(self.params.get('subobslongitude', '0')), 'rad')
-        self.subobslatitude = Quantity(float(self.params.get('subobslatitude', np.pi / 2)),
-                                       'rad')
-
+        self._image_geometry(inputs, device)
         self.image = np.zeros(self.dims)
         self.packet_image = np.zeros(self.dims)
-        self.blimits = None
-        immin = tuple(float(c) - float(w) / 2 for c, w in zip(self.center, self.width))
-        immax = tuple(float(c) + float(w) / 2 for c, w in zip(self.center, self.width))
-        self.xrange = [R(immin[0]), R(immax[0])]
-        self.zrange = [R(immin[1]), R(immax[1])]
-        scale = tuple(float(w) / d for w, d in zip(self.width, self.dims))
-        r_cm = float(self.origin.radius.value) * 1e5
-        self.Apix = Quantity((scale[0] * r_cm) * (scale[1] * r_cm), 'cm2')
-        self._device = local_device() if device is None else device
-        xr = [float(x) for x in self.xrange]
-        zr = [float(z) for z in self.zrange]
-        axes = _Hist2d(None, xr, zr, self.dims)
-        self.xaxis = R(axes.x)
-        self.zaxis = R(axes.y)
 
         # Every output file of this rank is binned into ONE image that stays on the device
         # (the reference adds the per-file histograms on the host, ModelImage.py:92-99) ...
@@ -124,6 +96,41 @@ class ModelImage(ModelResult):
                 *self.dims, self.atoms_per_packet)
         if comm is None:
             allreduce_sum(self.image, self.packet_image)       # gloo (CPU tests of the host logic)
+
+    def _image_geometry(self, inputs, device):
+        """The image plane from ``params`` (host only; ModelImageCube shares it): origin, unit,
+        dims, center, width, sub-observer point, xrange / zrange, Apix, xaxis / zaxis and the
+        device."""
+        from .sharding import local_device
+        self.origin = self.params.get('origin', inputs.geometry.planet)
+        self.unit = def_unit('R_' + self.origin.object, 'length',
+                             float(self.origin.radius.value) * 1e3)
+        R = lambda v: Quantity(v, self.unit)      # noqa: E731
+
+        dimtemp = self.params.get('dims', '800,800').split(',')
+        self.dims = [int(dimtemp[0]), int(dimtemp[1])]
+        centtemp = self.params.get('center', '0,0').split(',')
+        self.center = [R(float(centtemp[0])), R(float(centtemp[1]))]
+        widtemp = self.params.get('width', '8,8').split(',')
+        self.width = [R(float(widtemp[0])), R(float(widtemp[1]))]
+        self.subobslongitude = Quantity(float(self.params.get('subobslongitude', '0')), 'rad')
+        self.subobslatitude = Quantity(float(self.params.get('subobslatitude', np.pi / 2)),
+                                       'rad')
+
+        self.blimits = None
+        immin = tuple(float(c) - float(w) / 2 for c, w in zip(self.center, self.width))
+        immax = tuple(float(c) + float(w) / 2 for c, w in zip(self.center, self.width))
+        self.xrange = [R(immin[0]), R(immax[0])]
+        self.zrange = [R(immin[1]), R(immax[1])]
+        scale = tuple(float(w) / d for w, d in zip(self.width, self.dims))
+        r_cm = float(self.origin.radius.value) * 1e5
+        self.Apix = Quantity((scale[0] * r_cm) * (scale[1] * r_cm), 'cm2')
+        self._device = local_device() if device is None else device
+        xr = [float(x) for x in self.xrange]
+        zr = [float(z) for z in self.zrange]
+        axes = _Hist2d(None, xr, zr, self.dims)
+        self.xaxis = R(axes.x)
+        self.zaxis = R(axes.y)
 
     def image_rotation(self):
         return image_rotation(self.subobslongitude, self.subobslatitude)

@@ -2,13 +2,14 @@
 
 Public API mirrors the reference's ``nexoclom/__init__.py:9-14``.  Importing the
 package needs neither PostgreSQL nor astropy; creating an ``Output`` /
-``ModelImage`` / ``ModelDensity`` / ``LOSResult`` /
+``ModelImage`` / ``ModelImageCube`` / ``ModelDensity`` / ``LOSResult`` /
 ``LOSSpectrum`` needs the built CUDA library and a
 GPU (there is no CPU fallback).
 """
 from .Input import Input
 from .Output import Output
 from .ModelImage import ModelImage
+from .ModelImageCube import ModelImageCube
 from .ModelDensity import ModelDensity
 from .LOSResult import LOSResult
 from .LOSSpectrum import LOSSpectrum
@@ -16,6 +17,6 @@ from .LOSResultFitted import LOSResultFitted
 from .solarsystem import SSObject
 from .input_classes import InputError
 
-__all__ = ['Input', 'Output', 'ModelImage', 'ModelDensity', 'LOSResult', 'LOSSpectrum',
-           'LOSResultFitted', 'SSObject', 'InputError']
+__all__ = ['Input', 'Output', 'ModelImage', 'ModelImageCube', 'ModelDensity', 'LOSResult',
+           'LOSSpectrum', 'LOSResultFitted', 'SSObject', 'InputError']
 __version__ = '0.1.0'

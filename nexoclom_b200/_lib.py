@@ -162,6 +162,11 @@ def load():
                         c_i64_p, c_u32_p],
         'nx_los_spectrum': [vp, i64, i64, c_double_p, c_double_p, C.POINTER(LosParams),
                             C.POINTER(SpectrumParams), c_double_p, c_i64_p],
+        'nx_cube_begin': [vp, C.c_int, C.c_int, C.c_int],
+        'nx_cube_add': [vp, i64, C.POINTER(ImageParams), C.POINTER(SpectrumParams)],
+        'nx_cube_fetch': [vp, c_double_p, c_i64_p],
+        'nx_cube_allreduce_total': [vp, vp, C.POINTER(C.c_double)],
+        'nx_cube_end': [vp],
         'nx_density_accumulate': [vp, i64, i64, c_double_p, c_double_p, c_double_p, c_double_p,
                                   C.POINTER(u64)],
         'nx_source_map': [vp, i64, C.POINTER(SourceMapParams)] + [c_double_p] * 9 +

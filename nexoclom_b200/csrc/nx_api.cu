@@ -120,6 +120,10 @@ struct nx_ctx {
   // make once per output file, and nothing to leak on an error path
   struct Scratch { void* p = nullptr; size_t bytes = 0; } scr[32];
   int img_nx = 0, img_nz = 0;  // shape of the context-owned image scratch (nx_image_begin)
+  // context-owned image cube (nx_cube_begin .. nx_cube_end): ncell + 1 f64 sums (the last
+  // slot rides with the all-reduce), then ncell u64 counts, one allocation freed by end
+  int cube_nx = 0, cube_nz = 0, cube_nbins = 0;
+  double* cube = nullptr;
   void* pinned = nullptr;      // grow-only pinned staging for small D2H results (image, LOS columns)
   size_t pinned_bytes = 0;
   unsigned* cmp_tiles = nullptr;     // compaction scratch (tile counts)
@@ -412,6 +416,7 @@ int nx_ctx_destroy(nx_ctx* ctx) {
   cudaFree(ctx->pipe_scalars); cudaFree(ctx->pipe_hist);
   cudaFree(ctx->scalars); cudaFree(ctx->status); cudaFree(ctx->cmp_tiles);
   for (auto& sc : ctx->scr) cudaFree(sc.p);
+  cudaFree(ctx->cube);
   cudaFree(ctx->squeue); cudaFreeHost(ctx->seq_host);
   if (ctx->pinned) cudaFreeHost(ctx->pinned);
   if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
@@ -1689,6 +1694,112 @@ int nx_los_spectrum(nx_ctx* ctx, long long n, long long nlos, const double* los,
     CK(cudaStreamSynchronize(ctx->stream));
   }
   return r;
+}
+
+// ---- Doppler-resolved image cubes (ModelImageCube) -----------------------------------------
+// The cube has its own allocation, released by nx_cube_end: an 800 x 800 x 100 cube is 0.5 GB per
+// plane, too much to keep in grow-only scratch after the product is fetched.  No ENTER: like
+// nx_image_add, nothing here changes what the line-of-sight kernels read, so the candidate
+// pairs nx_los_accumulate_counted keeps stay valid.
+static long long cube_cells(const nx_ctx* ctx) {
+  return (long long)ctx->cube_nx * ctx->cube_nz * (ctx->cube_nbins + 2);
+}
+
+int nx_cube_end(nx_ctx* ctx) {
+  CK(cudaSetDevice(ctx->device));
+  if (ctx->cube) {
+    CK(cudaStreamSynchronize(ctx->stream));
+    CK(cudaFree(ctx->cube));
+  }
+  ctx->cube = nullptr;
+  ctx->cube_nx = ctx->cube_nz = ctx->cube_nbins = 0;
+  return 0;
+}
+
+int nx_cube_begin(nx_ctx* ctx, int nx_, int nz_, int nbins) {
+  CK(cudaSetDevice(ctx->device));
+  if (nx_ < 1 || nz_ < 1 || nbins < 1) { ctx->err = "nx_cube_begin: bad dims"; return -1; }
+  if ((double)nx_ * nz_ * ((double)nbins + 2) >= 2147483648.0) {
+    ctx->err = "nx_cube_begin: nx * nz * (nbins + 2) must be < 2^31";
+    return -1;
+  }
+  const long long ncell = (long long)nx_ * nz_ * (nbins + 2);
+  if (!ctx->cube || ncell != cube_cells(ctx)) {
+    int r = nx_cube_end(ctx);
+    if (r) return r;
+    CK(dev_malloc(&ctx->cube, (size_t)(2 * ncell + 1) * sizeof(double)));
+  }
+  ctx->cube_nx = nx_; ctx->cube_nz = nz_; ctx->cube_nbins = nbins;
+  CK(cudaMemsetAsync(ctx->cube, 0, (size_t)(2 * ncell + 1) * sizeof(double), ctx->stream));
+  return 0;
+}
+
+int nx_cube_add(nx_ctx* ctx, long long n, const nx_image_params* ip_,
+                const nx_spectrum_params* sp_) {
+  CK(cudaSetDevice(ctx->device));
+  if (!ctx->cube) { ctx->err = "nx_cube_begin not called"; return -1; }
+  if (!ip_ || !sp_) { ctx->err = "nx_cube_add: null argument"; return -1; }
+  ImageParams ip;
+  std::memcpy(&ip, ip_, sizeof(ip));
+  const nx_spectrum_params sp = *sp_;
+  if (ip.nx != ctx->cube_nx || ip.nz != ctx->cube_nz || sp.nbins != ctx->cube_nbins) {
+    ctx->err = "nx_cube_add: dims or nbins differ from nx_cube_begin";
+    return -1;
+  }
+  if (!std::isfinite(sp.vmin) || !std::isfinite(sp.vmax) || !(sp.vmin < sp.vmax)) {
+    ctx->err = "nx_cube_add: vmin < vmax, both finite, required";
+    return -1;
+  }
+  if (!std::isfinite(sp.vscale)) { ctx->err = "nx_cube_add: vscale must be finite"; return -1; }
+  if (ip.quantity == 1 && ctx->gtables.n == 0) {
+    ctx->err = "radiance cube requested but no g-value tables uploaded";
+    return -1;
+  }
+  if (n < 0 || n > resident_rows(ctx)) { ctx->err = "n exceeds resident packets"; return -1; }
+  if (n == 0) return 0;
+  CubeAxis ax;
+  ax.vmin = sp.vmin;
+  ax.vmax = sp.vmax;
+  ax.step = (sp.vmax - sp.vmin) / sp.nbins;         // np.linspace's step
+  ax.vscale = sp.vscale;
+  ax.nbins = sp.nbins;
+  const long long ncell = cube_cells(ctx);
+  int r;
+  if ((r = materialize(ctx))) return r;
+  if ((r = begin_timed(ctx))) return r;
+  CK(launch_image_cube(ctx->stream, ctx->device, state_cols(ctx), n, ip, ctx->gtables, ax,
+                       ctx->cube, reinterpret_cast<unsigned long long*>(ctx->cube + ncell + 1)));
+  return end_timed(ctx, 1);
+}
+
+int nx_cube_fetch(nx_ctx* ctx, double* cube, long long* counts) {
+  CK(cudaSetDevice(ctx->device));
+  if (!ctx->cube) { ctx->err = "nx_cube_begin not called"; return -1; }
+  const size_t bytes = (size_t)cube_cells(ctx) * 8;
+  // page-locked destinations (nx_host_alloc) get the DMA directly; pageable ones are staged by
+  // the driver (a pinned staging buffer of the context, grow-only, would outlive the cube)
+  if (cube) CK(cudaMemcpyAsync(cube, ctx->cube, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  if (counts)
+    CK(cudaMemcpyAsync(counts, ctx->cube + cube_cells(ctx) + 1, bytes, cudaMemcpyDeviceToHost,
+                       ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  return 0;
+}
+
+// The one collective of a sharded cube: sums and counts of every rank of `comm`, in place, with
+// *total riding in the slot after the sums (as nx_image_allreduce_total).
+int nx_cube_allreduce_total(nx_ctx* ctx, nx_comm* comm, double* total) {
+  CK(cudaSetDevice(ctx->device));
+  if (!ctx->cube) { ctx->err = "nx_cube_begin not called"; return -1; }
+  if (!total) { ctx->err = "nx_cube_allreduce_total: null total"; return -1; }
+  const long long ncell = cube_cells(ctx);
+  CK(cudaMemcpyAsync(ctx->cube + ncell, total, sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+  int r = nx_allreduce(comm, ctx->cube, ncell + 1, NX_DTYPE_F64, ctx->stream);
+  if (r == 0) r = nx_allreduce(comm, ctx->cube + ncell + 1, ncell, NX_DTYPE_I64, ctx->stream);
+  if (r) { ctx->err = std::string("nx_cube_allreduce_total: ") + nx_comm_last_error(); return r; }
+  CK(cudaMemcpyAsync(total, ctx->cube + ncell, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  return 0;
 }
 
 // ---- K7: number density at sample points (ModelDensity) ------------------------------------

@@ -1283,6 +1283,74 @@ k_image_accumulate_tile(StateCols P, long long n, ImageParams ip, GTables Gg, Im
 }
 
 // ---------------------------------------------------------------------------
+// Image cube (ModelImageCube): K4's pixel and weight (image_packet_fast, unchanged) with a
+// velocity axis.  v = los_doppler along row 1 of the observer rotation (the observer sits at
+// -y_obs, so v > 0 recedes), column = spectrum_column (np.histogram on linspace(vmin, vmax,
+// nbins + 1), 0 below, nbins + 1 above).  Streams x,y,z,vx,vy,vz,frac (56 B/row) and adds
+// one f64 RED (w != 0) and one u64 RED at pixel * (nbins + 2) + column.  The host keeps
+// nx * nz * (nbins + 2) below 2^31, so a cell index fits an int.
+// ---------------------------------------------------------------------------
+__device__ __forceinline__ void cube_one(const ImageParams& ip, const GTables& G,
+                                         const ImageSteps& t, const CubeAxis& ax, double x,
+                                         double y, double z, double vx, double vy, double vz,
+                                         double f, double* cube, unsigned long long* counts) {
+  if (ip.skip_dead && !(f > 0.0)) return;
+  double w;
+  const int pix = image_packet_fast(ip, G, t, x, y, z, vy, f, w);
+  if (pix < 0) return;
+  if (ip.round_f32) { vx = round_f32(vx); vy = round_f32(vy); vz = round_f32(vz); }
+  const double v = los_doppler(vx, vy, vz, ip.M[3], ip.M[4], ip.M[5], ax.vscale);
+  const int cell = pix * (ax.nbins + 2) + spectrum_column(v, ax.nbins, ax.vmin, ax.vmax, ax.step);
+  if (w != 0.0) atomicAdd(&cube[cell], w);
+  atomicAdd(&counts[cell], 1ull);
+}
+
+// Two rows per thread and iteration; the seven loads of the next pair are issued before the
+// current pair is binned (as k_image_accumulate)
+__global__ void __launch_bounds__(256)
+k_image_cube(StateCols P, long long n, ImageParams ip, GTables Gg, CubeAxis ax,
+             double* __restrict__ cube, unsigned long long* __restrict__ counts) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  GTables G;
+  stage_gtables(Gg, G, smem_raw);
+  __syncthreads();
+  const ImageSteps isteps = image_steps(ip);
+  const long long npair = n >> 1;
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  const double2* __restrict__ C2[7];
+#pragma unroll
+  for (int k = 0; k < 7; ++k) C2[k] = reinterpret_cast<const double2*>(P.c[k + 1]);
+  long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  double2 a[7];
+  if (i < npair) {
+#pragma unroll
+    for (int k = 0; k < 7; ++k) a[k] = __ldcs(C2[k] + i);
+  }
+  while (i < npair) {
+    const long long j = i + stride;
+    double2 b[7];
+#pragma unroll
+    for (int k = 0; k < 7; ++k) b[k] = a[k];
+    if (j < npair) {
+#pragma unroll
+      for (int k = 0; k < 7; ++k) b[k] = __ldcs(C2[k] + j);
+    }
+    cube_one(ip, G, isteps, ax, a[0].x, a[1].x, a[2].x, a[3].x, a[4].x, a[5].x, a[6].x, cube,
+             counts);
+    cube_one(ip, G, isteps, ax, a[0].y, a[1].y, a[2].y, a[3].y, a[4].y, a[5].y, a[6].y, cube,
+             counts);
+#pragma unroll
+    for (int k = 0; k < 7; ++k) a[k] = b[k];
+    i = j;
+  }
+  if ((n & 1) && blockIdx.x == 0 && threadIdx.x == 0) {
+    const long long q = n - 1;
+    cube_one(ip, G, isteps, ax, P.c[1][q], P.c[2][q], P.c[3][q], P.c[4][q], P.c[5][q], P.c[6][q],
+             P.c[7][q], cube, counts);
+  }
+}
+
+// ---------------------------------------------------------------------------
 // K5: lines of sight.  One LOS per thread (ray constants in registers), packet
 // positions staged through shared memory in tiles; every thread of the block
 // reads the same packet (smem broadcast) and runs the conservative cone reject;
@@ -1709,6 +1777,25 @@ cudaError_t launch_image_accumulate(cudaStream_t st, int device, StateCols P, lo
   const long long need = ((n >> 1) + 255) / 256;
   if (need < blocks) blocks = need > 0 ? need : 1;
   k_image_accumulate<<<(unsigned)blocks, 256, smem, st>>>(P, n, ip, G, image, counts);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_image_cube(cudaStream_t st, int device, StateCols P, long long n,
+                              const ImageParams& ip, const GTables& G, const CubeAxis& ax,
+                              double* cube, unsigned long long* counts) {
+  const size_t smem = gtables_smem_bytes(G);
+  if (smem > 48 * 1024) {
+    cudaError_t e = cudaFuncSetAttribute(k_image_cube, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)smem);
+    if (e != cudaSuccess) return e;
+  }
+  int per_sm = 1;
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_image_cube, 256, smem);
+  if (per_sm < 1) per_sm = 1;
+  long long blocks = (long long)per_sm * sm_count(device);
+  const long long need = ((n >> 1) + 255) / 256;
+  if (need < blocks) blocks = need > 0 ? need : 1;
+  k_image_cube<<<(unsigned)blocks, 256, smem, st>>>(P, n, ip, G, ax, cube, counts);
   return cudaGetLastError();
 }
 

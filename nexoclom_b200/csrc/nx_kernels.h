@@ -177,6 +177,15 @@ cudaError_t launch_integrate_constant(cudaStream_t st, int device, StateCols In,
 cudaError_t launch_image_accumulate(cudaStream_t st, int device, StateCols P, long long n,
                                     const ImageParams& ip, const GTables& G, double* image,
                                     unsigned long long* counts, int mode = 0);
+// Velocity axis of an image cube (ModelImageCube): edges = linspace(vmin, vmax, nbins + 1),
+// step = (vmax - vmin) / nbins, vscale = R_p in km; cell = pixel * (nbins + 2) + column
+struct CubeAxis {
+  double vmin, vmax, step, vscale;
+  int nbins;
+};
+cudaError_t launch_image_cube(cudaStream_t st, int device, StateCols P, long long n,
+                              const ImageParams& ip, const GTables& G, const CubeAxis& ax,
+                              double* cube, unsigned long long* counts);
 cudaError_t launch_los_accumulate(cudaStream_t st, int device, StateCols P, long long n,
                                   long long nlos, const double* los, const double* dist_plan,
                                   const int* nball, const double* ladder, const double* wid2,

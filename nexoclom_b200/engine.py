@@ -512,6 +512,44 @@ class Engine:
                                              cnt.ctypes.data_as(_lib.c_i64_p)), 'nx_los_spectrum')
         return spec, cnt
 
+    def cube_begin(self, nx, nz, nbins):
+        """Allocate and zero the context-owned image cube: (nx, nz, nbins + 2) f64 sums and
+        int64 counts (16 B per cell) until ``cube_end``."""
+        self._check(self.lib.nx_cube_begin(self.ctx, int(nx), int(nz), int(nbins)),
+                    'nx_cube_begin')
+
+    def cube_add(self, image_params, vmin, vmax, nbins, vscale, n=None):
+        """K4's rows, pixels and weights of the bound packet table (or the slab) binned into the
+        cube by their velocity along the observer's line of sight (``vscale`` km/s per R_p/s),
+        on ``np.linspace(vmin, vmax, nbins + 1)``; column 0 holds v < vmin, nbins + 1 v > vmax."""
+        n = self.n if n is None else n
+        sp = SpectrumParams()
+        sp.vmin, sp.vmax, sp.vscale, sp.nbins = float(vmin), float(vmax), float(vscale), int(nbins)
+        self._check(self.lib.nx_cube_add(self.ctx, int(n), C.byref(image_params), C.byref(sp)),
+                    'nx_cube_add')
+
+    def cube_fetch(self, nx, nz, nbins):
+        """(sums, counts), both (nx, nz, nbins + 2), float64 and int64, in page-locked arrays."""
+        pool = _pinned_pool(self.lib)
+        shape = (int(nx), int(nz), int(nbins) + 2)
+        cube = pool.array(shape)
+        cnt = pool.array(shape, dtype=np.int64)
+        self._check(self.lib.nx_cube_fetch(self.ctx, dptr(cube), cnt.ctypes.data_as(_lib.c_i64_p)),
+                    'nx_cube_fetch')
+        return cube, cnt
+
+    def cube_allreduce_total(self, comm, total):
+        """Sum the cube's sums and counts over the ranks of ``comm`` in place, with one scalar
+        riding along; returns the summed scalar."""
+        v = C.c_double(float(total))
+        self._check(self.lib.nx_cube_allreduce_total(self.ctx, comm, C.byref(v)),
+                    'nx_cube_allreduce_total')
+        return v.value
+
+    def cube_end(self):
+        """Release the cube's device memory."""
+        self._check(self.lib.nx_cube_end(self.ctx), 'nx_cube_end')
+
     def density_accumulate(self, points, radius, s1, s2, count, n=None):
         """K7 of the bound packet table (or the slab): ADDS to ``s1`` (sum of frac), ``s2``
         (sum of frac**2) and ``count`` (member rows) of every ball.  ``points``: (npts, 3) in
