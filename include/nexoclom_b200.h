@@ -205,6 +205,22 @@ int nx_integrate_adaptive_host(nx_ctx* ctx, long long n, const double* const* co
                                unsigned long long* attempted_steps,
                                unsigned long long* accepted_steps);
 
+/* K2 with surface bounce (an extension: the reference's adaptive driver asserts 'Not set up'
+ * unless stickcoef == 1, Output.py:309-315).  An accepted step that ends inside the planet
+ * goes through K3's surface interaction (bouncepackets.py: back-trace to r = 1, rebound speed,
+ * cosine-law direction, accommodation, constant or temperature-dependent sticking) with the
+ * deviates uniform_pair(seed, first_id + i, STREAM_BOUNCE, 2k) and (.., 2k + 1), k = the
+ * packet's accepted steps counting this one; then moon impact, escape (r^2 > outeredge),
+ * vanish and time = 0 for a dead packet as in K3.  Results do not depend on the launch
+ * geometry, the packet order or the number of GPUs.  Perfect sticking gives exactly
+ * nx_integrate_adaptive's results.  Preconditions of nx_integrate_constant: tables uploaded,
+ * the accommodation spline when accomfactor > 0.  `bounces` receives the number of surface
+ * interactions of the run.                                                                  */
+int nx_integrate_adaptive_bounce(nx_ctx* ctx, long long n, uint64_t seed, uint64_t first_id,
+                                 unsigned long long* attempted_steps,
+                                 unsigned long long* accepted_steps,
+                                 unsigned long long* bounces);
+
 /* ---- K3: constant-step driver with bounce (Output.py:368-455, bouncepackets.py)
  * Optional fused per-step image accumulation (image_dev / counts_dev device
  * pointers, may be NULL) and optional dense trajectory sink traj_host

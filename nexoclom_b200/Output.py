@@ -153,8 +153,18 @@ class Output:
     # ------------------------------------------------------------------
     def variable_step_size_driver(self, eng, host_cols=None):
         """Adaptive driver on the GPU (K2).  Semantics of reference
-        Output.py:221-366, including quirks Q1-Q9 (see DESIGN.md)."""
-        if host_cols is not None:
+        Output.py:221-366, including quirks Q1-Q9 (see DESIGN.md).  Extension: a surface that
+        does not absorb every packet (stickcoef < 1, temperature-dependent sticking) makes the
+        packets bounce (K3's surface interaction, deviates keyed by ``seed`` and the packet
+        id); ``bounces`` counts the surface interactions of the run."""
+        p = eng.params
+        self.bounces = 0
+        if not (p.sticktype == 0 and p.stickcoef == 1.0):
+            if host_cols is not None:
+                eng.import_state(host_cols)
+            self.attempted_steps, self.accepted_steps, self.bounces = eng.integrate_adaptive_bounce(
+                self.seed, self.first_id, self.npackets)
+        elif host_cols is not None:
             self.attempted_steps, self.accepted_steps = eng.integrate_adaptive_host(
                 host_cols, nchunks=16)
         else:

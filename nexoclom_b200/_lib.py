@@ -138,6 +138,8 @@ def load():
         'nx_integrate_adaptive': [vp, i64, C.POINTER(u64), C.POINTER(u64)],
         'nx_integrate_adaptive_host': [vp, i64, C.POINTER(c_double_p), C.c_int, C.POINTER(u64),
                                        C.POINTER(u64)],
+        'nx_integrate_adaptive_bounce': [vp, i64, u64, u64, C.POINTER(u64), C.POINTER(u64),
+                                         C.POINTER(u64)],
         'nx_integrate_constant': [vp, i64, u64, u64, C.POINTER(ImageParams), vp, vp,
                                   c_double_p, C.POINTER(u64)],
         'nx_image_accumulate': [vp, i64, C.POINTER(ImageParams), c_double_p, c_i64_p],

@@ -820,6 +820,25 @@ static int check_status(nx_ctx* ctx) {
   return v;
 }
 
+// K2 over the resident packets (ctx->scalars: [0] queue, [1] attempted, [2] accepted,
+// [3] bounces), longest first when ordering is on, inside the caller's timed section.
+// S != nullptr: packets bounce (nx_integrate_adaptive_bounce); the cost model then budgets
+// every packet's remaining time, since reaching the surface no longer ends its flight.
+static int adaptive_resident(nx_ctx* ctx, long long n, const Spline2D* S, uint64_t seed,
+                             uint64_t first_id) {
+  const bool order = ctx->order_packets && n >= 4096;
+  const bool to_surface = !S || perfect_sticking(ctx->params);
+  if (order)
+    CK(launch_cost_order(ctx->stream, ctx->device, in_cols(ctx), n, ctx->params,
+                         ctx->order_packets, ctx->cost, ctx->hist, ctx->perm, to_surface));
+  CK(launch_integrate_adaptive(ctx->stream, ctx->device, in_cols(ctx), state_cols(ctx), n,
+                               ctx->params,
+                               ctx->radpres.view, ctx->radpres.fast,
+                               order ? ctx->perm : nullptr, ctx->scalars, ctx->scalars + 1,
+                               ctx->att, ctx->acc, ctx->status, S, seed, first_id));
+  return end_timed(ctx, order ? 4 : 1);
+}
+
 int nx_integrate_adaptive(nx_ctx* ctx, long long n, unsigned long long* attempted,
                           unsigned long long* accepted) {
   ENTER(ctx);
@@ -857,16 +876,7 @@ int nx_integrate_adaptive(nx_ctx* ctx, long long n, unsigned long long* attempte
                                           ctx->scalars + 1, ctx->att, ctx->acc, ctx->status));
       if ((r = end_timed(ctx, 1))) return r;
     } else {
-      const bool order = ctx->order_packets && n >= 4096;
-      if (order)
-        CK(launch_cost_order(ctx->stream, ctx->device, in_cols(ctx), n, ctx->params,
-                             ctx->order_packets, ctx->cost, ctx->hist, ctx->perm));
-      CK(launch_integrate_adaptive(ctx->stream, ctx->device, in_cols(ctx), state_cols(ctx), n,
-                                   ctx->params,
-                                   ctx->radpres.view, ctx->radpres.fast,
-                                   order ? ctx->perm : nullptr, ctx->scalars, ctx->scalars + 1,
-                                   ctx->att, ctx->acc, ctx->status));
-      if ((r = end_timed(ctx, order ? 4 : 1))) return r;
+      if ((r = adaptive_resident(ctx, n, nullptr, 0, 0))) return r;
     }
     ctx->fresh = false;
   }
@@ -876,6 +886,35 @@ int nx_integrate_adaptive(nx_ctx* ctx, long long n, unsigned long long* attempte
   if (r < 0) return r;
   if (attempted) *attempted = h[1];
   if (accepted) *accepted = h[2];
+  return r;
+}
+
+int nx_integrate_adaptive_bounce(nx_ctx* ctx, long long n, uint64_t seed, uint64_t first_id,
+                                 unsigned long long* attempted, unsigned long long* accepted,
+                                 unsigned long long* bounces) {
+  ENTER(ctx);
+  if (!ctx->have_params) { ctx->err = "nx_tables_upload not called"; return -1; }
+  ctx->bound = nullptr;            // integrators work on the slab
+  if (n > ctx->cap) { ctx->err = "n exceeds resident packets"; return -1; }
+  const RunParams& p = ctx->params;
+  if (!perfect_sticking(p) && p.accomfactor != 0.0 && !ctx->spl_c) {
+    ctx->err = "accommodation enabled but no speed spline uploaded";
+    return -1;
+  }
+  CK(cudaMemsetAsync(ctx->scalars, 0, 8 * sizeof(unsigned long long), ctx->stream));
+  int r;
+  if (n > 0) {
+    if ((r = begin_timed(ctx))) return r;
+    if ((r = adaptive_resident(ctx, n, &ctx->spline, seed, first_id))) return r;
+    ctx->fresh = false;
+  }
+  unsigned long long h[4] = {0, 0, 0, 0};
+  CK(cudaMemcpyAsync(h, ctx->scalars, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
+  r = check_status(ctx);
+  if (r < 0) return r;
+  if (attempted) *attempted = h[1];
+  if (accepted) *accepted = h[2];
+  if (bounces) *bounces = h[3];
   return r;
 }
 

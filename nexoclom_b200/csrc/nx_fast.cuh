@@ -306,15 +306,17 @@ NX_HD void fast_stages(const RunParams& p, const FastTable& T, const double* s, 
 
 // One attempted adaptive step, fast arithmetic.  Same contract as
 // adaptive_attempt<>(): s[0..7] = time,x,y,z,vx,vy,vz,frac; returns AttemptFlags.
-template <int GR, int RP, int LOSS, int MO = 0>
+// BOUNCE, S, seed, id, k: as in adaptive_attempt<>().
+template <int GR, int RP, int LOSS, int MO = 0, bool BOUNCE = false>
 NX_HD int adaptive_attempt_fast(const RunParams& p, const FastTable& T, double* s,
-                                double& step) {
+                                double& step, const Spline2D* S = nullptr, uint64_t seed = 0,
+                                uint64_t id = 0, uint32_t k = 0) {
   const double res = p.resolution;
   const double resv = 0.1 * res;
   const double h = fmin(s[0], step);
   double nx[6], d[6], fn, delta_f, moon_end[2] = {0.0, 0.0};
   fast_stages<GR, RP, LOSS, true, MO>(p, T, s, h, nx, fn, d, delta_f, moon_end);
-  const double px = nx[0], py = nx[1], pz = nx[2], vx = nx[3], vy = nx[4], vz = nx[5];
+  double px = nx[0], py = nx[1], pz = nx[2], vx = nx[3], vy = nx[4], vz = nx[5];
   // accept  <=>  every delta_j < scale_j  (== max_j fl(delta_j/scale_j) < 1).  The
   // quotient itself (Newton reciprocal, ~2^-40) only sizes the next step after a
   // reject and screens the "no error" case (Q4); it is formed for every lane so
@@ -348,7 +350,16 @@ NX_HD int adaptive_attempt_fast(const RunParams& p, const FastTable& T, double* 
     const double r2 = fma(pz, pz, fma(py, py, px * px));
     double f = fn;
     if (fn < 0.0) flags |= ATT_NEG_FRAC;
-    if (r2 < 1.0) f = 0.0;                 // impact, stickcoef == 1 (Q6)
+    if (r2 < 1.0) {
+      if (BOUNCE && !perfect_sticking(p)) {  // bounce, then K3's tests on the new state
+        double b[8] = {0.0, px, py, pz, vx, vy, vz, fn};
+        adaptive_surface<true>(p, *S, b, r2, seed, id, k);
+        px = b[1]; py = b[2]; pz = b[3]; vx = b[4]; vy = b[5]; vz = b[6]; f = b[7];
+        flags |= ATT_BOUNCED;
+      } else {
+        f = 0.0;                           // impact, stickcoef == 1 (Q6)
+      }
+    }
     if (MO) {                              // impact on the moon
       const double dx = px - moon_end[0], dy = py - moon_end[1];
       if (fma(pz, pz, fma(dy, dy, dx * dx)) < p.moon_r2[0]) f = 0.0;
@@ -368,27 +379,31 @@ NX_HD int adaptive_attempt_fast(const RunParams& p, const FastTable& T, double* 
 }
 
 // runtime dispatch over the compile-time force / loss combinations
+template <bool BOUNCE = false>
 NX_HD int adaptive_attempt_fast_rt(const RunParams& p, const FastTable& T, double* s,
-                                   double& step) {
+                                   double& step, const Spline2D* S = nullptr, uint64_t seed = 0,
+                                   uint64_t id = 0, uint32_t k = 0) {
+#define NX_ARGS p, T, s, step, S, seed, id, k
   if (p.nmoons == 1 && p.gravity) {
     if (p.radpres) {
-      if (p.loss_mode == LOSS_PHOTO) return adaptive_attempt_fast<1, 1, LOSS_PHOTO, 1>(p, T, s, step);
-      if (p.loss_mode == LOSS_LIFETIME) return adaptive_attempt_fast<1, 1, LOSS_LIFETIME, 1>(p, T, s, step);
-      return adaptive_attempt_fast<1, 1, LOSS_NONE, 1>(p, T, s, step);
+      if (p.loss_mode == LOSS_PHOTO) return adaptive_attempt_fast<1, 1, LOSS_PHOTO, 1, BOUNCE>(NX_ARGS);
+      if (p.loss_mode == LOSS_LIFETIME) return adaptive_attempt_fast<1, 1, LOSS_LIFETIME, 1, BOUNCE>(NX_ARGS);
+      return adaptive_attempt_fast<1, 1, LOSS_NONE, 1, BOUNCE>(NX_ARGS);
     }
-    if (p.loss_mode == LOSS_PHOTO) return adaptive_attempt_fast<1, 0, LOSS_PHOTO, 1>(p, T, s, step);
-    if (p.loss_mode == LOSS_LIFETIME) return adaptive_attempt_fast<1, 0, LOSS_LIFETIME, 1>(p, T, s, step);
-    return adaptive_attempt_fast<1, 0, LOSS_NONE, 1>(p, T, s, step);
+    if (p.loss_mode == LOSS_PHOTO) return adaptive_attempt_fast<1, 0, LOSS_PHOTO, 1, BOUNCE>(NX_ARGS);
+    if (p.loss_mode == LOSS_LIFETIME) return adaptive_attempt_fast<1, 0, LOSS_LIFETIME, 1, BOUNCE>(NX_ARGS);
+    return adaptive_attempt_fast<1, 0, LOSS_NONE, 1, BOUNCE>(NX_ARGS);
   }
   const int key = (p.gravity ? 4 : 0) | (p.radpres ? 2 : 0);
 #define NX_CASE(G, R)                                                                    \
   if (key == ((G) * 4 + (R) * 2)) {                                                      \
-    if (p.loss_mode == LOSS_PHOTO) return adaptive_attempt_fast<G, R, LOSS_PHOTO>(p, T, s, step);       \
-    if (p.loss_mode == LOSS_LIFETIME) return adaptive_attempt_fast<G, R, LOSS_LIFETIME>(p, T, s, step); \
-    return adaptive_attempt_fast<G, R, LOSS_NONE>(p, T, s, step);                     \
+    if (p.loss_mode == LOSS_PHOTO) return adaptive_attempt_fast<G, R, LOSS_PHOTO, 0, BOUNCE>(NX_ARGS);       \
+    if (p.loss_mode == LOSS_LIFETIME) return adaptive_attempt_fast<G, R, LOSS_LIFETIME, 0, BOUNCE>(NX_ARGS); \
+    return adaptive_attempt_fast<G, R, LOSS_NONE, 0, BOUNCE>(NX_ARGS);                     \
   }
   NX_CASE(1, 1) NX_CASE(1, 0) NX_CASE(0, 1) NX_CASE(0, 0)
 #undef NX_CASE
+#undef NX_ARGS
   return 0;
 }
 

@@ -294,14 +294,18 @@ struct PacketFeeder {
 // MODE: -1 = strict (NumPy operation order, runtime force flags);
 //       otherwise fast arithmetic with compile-time forces:
 //       MODE = GR*8 + RP*4 + LOSS.
-template <int MODE>
+// BOUNCE: packets that hit the surface bounce (adaptive_attempt<.., true>), the deviates of
+// packet idx are keyed by (seed, first_id + idx); totals[2] receives the number of bounces.
+// S / seed / first_id are unused otherwise.
+template <int MODE, bool BOUNCE = false>
 __global__ void __launch_bounds__(NX_INT_THREADS, NX_INT_MINBLOCKS)
 k_integrate_adaptive(StateCols In, StateCols P, long long n, RunParams p, InterpTable Tg,
                      FastTable Fg, const unsigned* __restrict__ perm,
                      unsigned long long* __restrict__ queue,
                      unsigned long long* __restrict__ totals,
                      unsigned* __restrict__ att_out, unsigned* __restrict__ acc_out,
-                     int* __restrict__ status, unsigned table_bytes) {
+                     int* __restrict__ status, unsigned table_bytes, Spline2D S, uint64_t seed,
+                     uint64_t first_id) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   InterpTable T;
   FastTable F;
@@ -320,7 +324,7 @@ k_integrate_adaptive(StateCols In, StateCols P, long long n, RunParams p, Interp
   unsigned idx = 0;
   double s[8], step = 0.0;
   unsigned att = 0, acc = 0;
-  unsigned long long tot_att = 0, tot_acc = 0;
+  unsigned long long tot_att = 0, tot_acc = 0, tot_bnc = 0;
   int st = 0;
 #ifdef NX_STREAM_DEBUG
   unsigned long long dbg_iters = 0;
@@ -360,11 +364,15 @@ k_integrate_adaptive(StateCols In, StateCols P, long long n, RunParams p, Interp
     NX_DBG_ITER(__ballot_sync(FULL_MASK, have));
     if (have) {
       int fl;
-      if (MODE < 0) fl = adaptive_attempt<true>(p, T, s, step);
-      else fl = adaptive_attempt_fast<(MODE >> 3) & 1, (MODE >> 2) & 1, MODE & 3, (MODE >> 4) & 1>(p, F, s, step);
+      if (MODE < 0)
+        fl = adaptive_attempt<true, BOUNCE>(p, T, s, step, &S, seed, first_id + idx, acc + 1);
+      else
+        fl = adaptive_attempt_fast<(MODE >> 3) & 1, (MODE >> 2) & 1, MODE & 3, (MODE >> 4) & 1, BOUNCE>(
+            p, F, s, step, &S, seed, first_id + idx, acc + 1);
       ++att;
       if (fl & ATT_ACCEPTED) ++acc;
-      st |= fl & ~(ATT_ACCEPTED | ATT_LIVE);
+      if (BOUNCE && (fl & ATT_BOUNCED)) ++tot_bnc;
+      st |= fl & ~(ATT_ACCEPTED | ATT_LIVE | (BOUNCE ? ATT_BOUNCED : 0));
       if (att >= NX_ATTEMPT_CAP) { st |= NX_ST_NO_PROGRESS; fl &= ~ATT_LIVE; }
       if (!(fl & ATT_LIVE)) {
 #pragma unroll
@@ -381,11 +389,13 @@ k_integrate_adaptive(StateCols In, StateCols P, long long n, RunParams p, Interp
   for (int o = 16; o > 0; o >>= 1) {
     tot_att += __shfl_xor_sync(FULL_MASK, tot_att, o);
     tot_acc += __shfl_xor_sync(FULL_MASK, tot_acc, o);
+    if (BOUNCE) tot_bnc += __shfl_xor_sync(FULL_MASK, tot_bnc, o);
     st |= __shfl_xor_sync(FULL_MASK, st, o);
   }
   if (lane == 0) {
     if (tot_att) atomicAdd(&totals[0], tot_att);
     if (tot_acc) atomicAdd(&totals[1], tot_acc);
+    if (BOUNCE && tot_bnc) atomicAdd(&totals[2], tot_bnc);
     if (st) atomicOr(status, st);
 #ifdef NX_STREAM_DEBUG
     atomicMax(&g_dbg[16], dbg_now());
@@ -406,10 +416,12 @@ k_integrate_adaptive(StateCols In, StateCols P, long long n, RunParams p, Interp
 
 // Predicted attempted steps of a packet, in float (it only orders the queue): Kepler flight
 // time to the surface for bound orbits that dip below it, else the time the packet has left,
-// over the position-error step bound.
+// over the position-error step bound.  to_surface = false (bounce runs: a packet that reaches
+// the surface goes on hopping) always budgets the time left.
 __device__ __forceinline__ float cost_estimate_f(const RunParams& p, int model, float res, float mu,
                                                 float amax, double td, double xd, double yd,
-                                                double zd, double vxd, double vyd, double vzd) {
+                                                double zd, double vxd, double vyd, double vzd,
+                                                bool to_surface = true) {
   const float t = (float)td, x = (float)xd, y = (float)yd, z = (float)zd;
   const float vx = (float)vxd, vy = (float)vyd, vz = (float)vzd;
   const float r2 = x * x + y * y + z * z, r = sqrtf(r2);
@@ -417,7 +429,7 @@ __device__ __forceinline__ float cost_estimate_f(const RunParams& p, int model, 
   const float rv = x * vx + y * vy + z * vz;
   float tfl = t;
   const float en = 0.5f * v2 - mu / r;
-  if (p.gravity && en < 0.0f && mu > 0.0f) {
+  if (to_surface && p.gravity && en < 0.0f && mu > 0.0f) {
     const float a = -mu / (2.0f * en);
     const float l2 = fmaxf(r2 * v2 - rv * rv, 0.0f);
     const float e = sqrtf(fmaxf(1.0f + 2.0f * en * l2 / (mu * mu), 0.0f));
@@ -446,16 +458,17 @@ __device__ __forceinline__ float cost_estimate_f(const RunParams& p, int model, 
   return tfl * v / (40.0f * res * (1.0f + r)) + 4.0f;
 }
 __device__ __forceinline__ int cost_bucket(const RunParams& p, int model, double t, double x, double y,
-                                           double z, double vx, double vy, double vz, double f) {
+                                           double z, double vx, double vy, double vz, double f,
+                                           bool to_surface) {
   if (!(t > p.resolution) || !(f > 0.0)) return 0;
   const float est = cost_estimate_f(p, model, (float)p.resolution, (float)fabs(p.GM),
-                                    (float)p.radpres_amax, t, x, y, z, vx, vy, vz);
+                                    (float)p.radpres_amax, t, x, y, z, vx, vy, vz, to_surface);
   const int b = (int)(2.0f * log2f(est));
   return b < 0 ? 0 : (b > NX_NBUCKET - 1 ? NX_NBUCKET - 1 : b);
 }
 
 __global__ void __launch_bounds__(256)
-k_cost_histogram(StateCols P, long long n, RunParams p, int model,
+k_cost_histogram(StateCols P, long long n, RunParams p, int model, bool to_surface,
                  unsigned char* __restrict__ bucket, unsigned* __restrict__ hist) {
   __shared__ unsigned sh[8][NX_NBUCKET];            // one histogram per warp (most packets
   sh[threadIdx.x >> 5][threadIdx.x & 31] = 0;       // share three or four buckets)
@@ -464,7 +477,7 @@ k_cost_histogram(StateCols P, long long n, RunParams p, int model,
   const long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
     const int b = cost_bucket(p, model, P.c[0][i], P.c[1][i], P.c[2][i], P.c[3][i], P.c[4][i],
-                              P.c[5][i], P.c[6][i], P.c[7][i]);
+                              P.c[5][i], P.c[6][i], P.c[7][i], to_surface);
     bucket[i] = (unsigned char)b;
     atomicAdd(&mine[b], 1u);
   }
@@ -1510,24 +1523,25 @@ static cudaError_t persistent_grid(K kernel, int device, size_t smem, int* block
   return cudaSuccess;
 }
 
-template <int MODE>
+template <int MODE, bool BOUNCE = false>
 static cudaError_t launch_adaptive_mode(cudaStream_t st, int device, StateCols In, StateCols P,
                                         long long n,
                                         const RunParams& p, const InterpTable& T,
                                         const FastTable& F,
                                         const unsigned* perm, unsigned long long* queue,
                                         unsigned long long* totals, unsigned* att, unsigned* acc,
-                                        int* status) {
+                                        int* status, const Spline2D& S, uint64_t seed,
+                                        uint64_t first_id) {
   const size_t tbytes = (MODE < 0) ? table_smem_bytes(T) : fast_table_smem_bytes(F);
   const size_t smem = tbytes + (size_t)(NX_INT_THREADS / 32) * NX_FEED_BYTES_PER_WARP;
   int blocks = 0;
-  cudaError_t e = persistent_grid(k_integrate_adaptive<MODE>, device, smem, &blocks);
+  cudaError_t e = persistent_grid(k_integrate_adaptive<MODE, BOUNCE>, device, smem, &blocks);
   if (e != cudaSuccess) return e;
   const long long need = (n + NX_INT_THREADS - 1) / NX_INT_THREADS;
   if (need < blocks) blocks = (int)(need > 0 ? need : 1);
-  k_integrate_adaptive<MODE><<<blocks, NX_INT_THREADS, smem, st>>>(In, P, n, p, T, F, perm, queue,
-                                                                   totals, att, acc, status,
-                                                                   (unsigned)tbytes);
+  k_integrate_adaptive<MODE, BOUNCE><<<blocks, NX_INT_THREADS, smem, st>>>(
+      In, P, n, p, T, F, perm, queue, totals, att, acc, status, (unsigned)tbytes, S, seed,
+      first_id);
   return cudaGetLastError();
 }
 
@@ -1617,14 +1631,15 @@ cudaError_t launch_integrate_adaptive_stream(cudaStream_t st, int device, const 
 
 cudaError_t launch_cost_order(cudaStream_t st, int device, StateCols P, long long n,
                               const RunParams& p, int model, unsigned char* bucket,
-                              unsigned* hist_cursor, unsigned* perm) {
+                              unsigned* hist_cursor, unsigned* perm, bool to_surface) {
   // hist_cursor: [0..31] histogram, [32..63] cursors
   cudaError_t e = cudaMemsetAsync(hist_cursor, 0, 2 * NX_NBUCKET * sizeof(unsigned), st);
   if (e != cudaSuccess) return e;
   long long blocks = (n + 255) / 256;
   const long long cap = (long long)sm_count(device) * 8;
   if (blocks > cap) blocks = cap;
-  k_cost_histogram<<<(unsigned)blocks, 256, 0, st>>>(P, n, p, model, bucket, hist_cursor);
+  k_cost_histogram<<<(unsigned)blocks, 256, 0, st>>>(P, n, p, model, to_surface, bucket,
+                                                      hist_cursor);
   k_cost_offsets<<<1, 32, 0, st>>>(hist_cursor, hist_cursor + NX_NBUCKET);
   const long long sb = (n + 256 * NX_SCATTER_ITEMS - 1) / (256 * NX_SCATTER_ITEMS);
   k_cost_scatter<<<(unsigned)sb, 256, 0, st>>>(n, bucket, hist_cursor + NX_NBUCKET, perm);
@@ -1635,8 +1650,30 @@ cudaError_t launch_integrate_adaptive(cudaStream_t st, int device, StateCols In,
                                       long long n, const RunParams& p, const InterpTable& T,
                                       const FastTable& F, const unsigned* perm,
                                       unsigned long long* queue, unsigned long long* totals,
-                                      unsigned* att, unsigned* acc, int* status) {
-#define NX_ARGS st, device, In, P, n, p, T, F, perm, queue, totals, att, acc, status
+                                      unsigned* att, unsigned* acc, int* status,
+                                      const Spline2D* S, uint64_t seed, uint64_t first_id) {
+#define NX_ARGS st, device, In, P, n, p, T, F, perm, queue, totals, att, acc, status, \
+                S ? *S : Spline2D{}, seed, first_id
+  if (S) {
+    // bounce builds: the strict kernel, and the fast kernels with gravity (one moon too);
+    // runs without gravity or with more moons take the strict kernel
+    if (p.strict_math || !p.gravity || p.nmoons > 1) return launch_adaptive_mode<-1, true>(NX_ARGS);
+    switch ((p.radpres ? 4 : 0) | (p.loss_mode & 3) | (p.nmoons == 1 ? 16 : 0)) {
+      case 16: return launch_adaptive_mode<24, true>(NX_ARGS);
+      case 17: return launch_adaptive_mode<25, true>(NX_ARGS);
+      case 18: return launch_adaptive_mode<26, true>(NX_ARGS);
+      case 20: return launch_adaptive_mode<28, true>(NX_ARGS);
+      case 21: return launch_adaptive_mode<29, true>(NX_ARGS);
+      case 22: return launch_adaptive_mode<30, true>(NX_ARGS);
+      case 0: return launch_adaptive_mode<8, true>(NX_ARGS);
+      case 1: return launch_adaptive_mode<9, true>(NX_ARGS);
+      case 2: return launch_adaptive_mode<10, true>(NX_ARGS);
+      case 4: return launch_adaptive_mode<12, true>(NX_ARGS);
+      case 5: return launch_adaptive_mode<13, true>(NX_ARGS);
+      case 6: return launch_adaptive_mode<14, true>(NX_ARGS);
+      default: return cudaErrorInvalidValue;
+    }
+  }
   if (p.strict_math || p.nmoons > 1 || (p.nmoons == 1 && !p.gravity))
     return launch_adaptive_mode<-1>(NX_ARGS);
   const int mode = (p.gravity ? 8 : 0) | (p.radpres ? 4 : 0) | (p.loss_mode & 3) |

@@ -397,11 +397,38 @@ enum AttemptFlags {
   ATT_LIVE = 2,           // packet still needs steps: (time > res) & (frac > 0)
   ATT_BAD_ERRMAX = 4,     // non-finite errmax            (reference assert :284)
   ATT_NEG_FRAC = 8,       // accepted negative frac        (reference assert :287)
-  ATT_BAD_STEP = 16       // non-finite / unchanged step   (reference asserts :337-339)
+  ATT_BAD_STEP = 16,      // non-finite / unchanged step   (reference asserts :337-339)
+  ATT_BOUNCED = 256       // accepted step ended in a surface interaction (BOUNCE builds only;
+                          // above the kernels' status bits, never reported as one)
 };
 
-template <bool STRICT>
-NX_HD int adaptive_attempt(const RunParams& p, const InterpTable& T, double* s, double& step) {
+// Surface interaction of an accepted adaptive step that ended inside the planet (r2 < 1),
+// for BOUNCE builds of the attempt functions: K3's bounce (FAST: bounce_fast) with r =
+// sqrt(r2) and the deviates uniform_pair(seed, id, STREAM_BOUNCE, 2k) and (.., 2k + 1), k = the
+// packet's accepted steps counting this one.  s[1..7] is updated in place.  Defined in
+// nx_surface.cuh; on the device it is an out-of-line call, so the rarely taken bounce (spline,
+// trigonometry, Philox) adds neither registers nor instruction-cache footprint to the step loop.
+#if defined(__CUDACC__)
+#define NX_COLD __host__ __device__ __noinline__
+#else
+#define NX_COLD inline
+#endif
+template <bool FAST>
+NX_COLD void adaptive_surface(const RunParams& p, const Spline2D& S, double* s, double r2,
+                              uint64_t seed, uint64_t id, uint32_t k);
+
+// Bounce inputs of the adaptive driver: everything but constant sticking of exactly 1.
+NX_HD bool perfect_sticking(const RunParams& p) {
+  return p.sticktype == STICK_CONSTANT && p.stickcoef == 1.0;
+}
+
+// BOUNCE = false: the reference's driver (a packet that hits the surface sticks, Q6).
+// BOUNCE = true: accepted steps that end inside the planet go through adaptive_surface()
+// unless the sticking is perfect; S / seed / id / k feed it (unused otherwise).
+template <bool STRICT, bool BOUNCE = false>
+NX_HD int adaptive_attempt(const RunParams& p, const InterpTable& T, double* s, double& step,
+                           const Spline2D* S = nullptr, uint64_t seed = 0, uint64_t id = 0,
+                           uint32_t k = 0) {
   const double res = p.resolution;
   const double resv = mul_rn(0.1, res);
   const double h = fmin(s[0], step);
@@ -428,7 +455,15 @@ NX_HD int adaptive_attempt(const RunParams& p, const InterpTable& T, double* s, 
   if (errmax < 1.0) {
     const double r2 = add_rn(add_rn(mul_rn(nx[1], nx[1]), mul_rn(nx[2], nx[2])), mul_rn(nx[3], nx[3]));
     double f = nx[7];
-    if (r2 < 1.0) f = 0.0;                 // impact, stickcoef == 1 (Q6)
+    if (r2 < 1.0) {
+      if (BOUNCE && !perfect_sticking(p)) {  // bounce, then K3's tests on the new state
+        adaptive_surface<false>(p, *S, nx, r2, seed, id, k);
+        f = nx[7];
+        flags |= ATT_BOUNCED;
+      } else {
+        f = 0.0;                           // impact, stickcoef == 1 (Q6)
+      }
+    }
     for (int m = 0; m < p.nmoons; ++m) {   // impact on a moon (same rule, moon surface)
       double mx, my;
       moon_position(p, m, nx[0], mx, my);

@@ -266,6 +266,17 @@ NX_HD void bounce_fast(const RunParams& p, const Spline2D& S, double* s, double 
   }
 }
 
+// Surface interaction of the adaptive driver's BOUNCE builds (declared in nx_physics.cuh).
+template <bool FAST>
+NX_COLD void adaptive_surface(const RunParams& p, const Spline2D& S, double* s, double r2,
+                              uint64_t seed, uint64_t id, uint32_t k) {
+  double u_alt, u_az, u_prob, unused;
+  uniform_pair(seed, id, STREAM_BOUNCE, 2u * k, u_alt, u_az);
+  uniform_pair(seed, id, STREAM_BOUNCE, 2u * k + 1u, u_prob, unused);
+  if (FAST) bounce_fast(p, S, s, sqrt(r2), u_alt, u_az, u_prob);
+  else bounce(p, S, s, sqrt(r2), u_alt, u_az, u_prob);
+}
+
 // post-step handling shared by the strict and the fast constant step
 template <bool FAST>
 NX_HD bool constant_step_finish(const RunParams& p, const Spline2D& S, double* nx, double* s,

@@ -308,6 +308,16 @@ class Engine:
                     'nx_integrate_adaptive')
         return int(att.value), int(acc.value)
 
+    def integrate_adaptive_bounce(self, seed, first_id=0, n=None):
+        """K2 with surface bounce on the resident packets: deviates keyed by (seed, first_id +
+        packet index).  Returns (attempted, accepted, bounces)."""
+        att, acc, bnc = C.c_ulonglong(), C.c_ulonglong(), C.c_ulonglong()
+        n = self.n if n is None else n
+        self._check(self.lib.nx_integrate_adaptive_bounce(self.ctx, int(n), int(seed), int(first_id),
+                                                          C.byref(att), C.byref(acc), C.byref(bnc)),
+                    'nx_integrate_adaptive_bounce')
+        return int(att.value), int(acc.value), int(bnc.value)
+
     def integrate_adaptive_host(self, cols, nchunks=8):
         """import_state + integrate_adaptive with the H2D copy pipelined against
         the integration (host columns should be pinned for real overlap)."""
