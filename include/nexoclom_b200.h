@@ -221,6 +221,50 @@ int nx_integrate_adaptive_bounce(nx_ctx* ctx, long long n, uint64_t seed, uint64
                                  unsigned long long* accepted_steps,
                                  unsigned long long* bounces);
 
+/* ---- K2d: surface deposition maps and the source's loss budget (ModelDeposition) ----------
+ * An extension (the reference records neither).  nx_integrate_adaptive_deposit runs the
+ * adaptive driver on the resident packets exactly as nx_integrate_adaptive (perfect sticking)
+ * or nx_integrate_adaptive_bounce (any other sticking, deviates keyed by seed / first_id)
+ * would, same preconditions, same final state and step totals, and adds to the sink of
+ * nx_deposit_begin where the frac of the packets went:
+ *   SURFACE    per accepted step that ends inside the planet: the frac that stays there
+ *              (all of it for perfect sticking, frac before - frac after a bounce), mapped at
+ *              the post-step point (perfect sticking) or the bounce point, lon =
+ *              fmod(atan2(x, -y) + 2 pi, 2 pi), lat = atan2(z, sqrt(x*x + y*y)), on
+ *              np.histogram2d's axes linspace(0, 2 pi, nlon + 1) x linspace(-pi/2, pi/2,
+ *              nlat + 1), longitude major; one event per such step, whatever its amount
+ *   MOON / ESCAPED (r^2 > outeredge) / VANISHED (frac < 1e-10): the frac the first of these
+ *              tests (in the driver's order) sets to zero
+ *   REMAINING  the frac of packets that retire alive (time <= resolution or the attempt cap)
+ *              or are passed through without integration
+ *   SOURCE     the initial frac > 0 of the packets handed to the kernel
+ * Each bucket and map cell holds an f64 sum and an event count.  The frac lost in flight
+ * (photo-ionisation, lifetime) is SOURCE minus the other buckets.
+ * begin validates nlon, nlat >= 1 (nlon * nlat < 2^31) and allocates and zeroes the sink;
+ * fetch copies map / counts (nlon * nlat) and buckets / bucket_counts (NX_DEP_NBUCKET, in
+ * nx_deposit_bucket order), any of them may be NULL; allreduce sums the sink over the ranks of
+ * `comm` in place, *total riding along (as nx_cube_allreduce_total; NULL: none); end
+ * releases it.  Images, cubes and the line-of-sight buffers are not
+ * touched.                                                                                   */
+typedef enum {
+  NX_DEP_SURFACE = 0,
+  NX_DEP_MOON = 1,
+  NX_DEP_ESCAPED = 2,
+  NX_DEP_VANISHED = 3,
+  NX_DEP_REMAINING = 4,
+  NX_DEP_SOURCE = 5,
+  NX_DEP_NBUCKET = 6
+} nx_deposit_bucket;
+int nx_deposit_begin(nx_ctx* ctx, int nlon, int nlat);
+int nx_integrate_adaptive_deposit(nx_ctx* ctx, long long n, uint64_t seed, uint64_t first_id,
+                                  unsigned long long* attempted_steps,
+                                  unsigned long long* accepted_steps,
+                                  unsigned long long* bounces);
+int nx_deposit_fetch(nx_ctx* ctx, double* map, long long* counts, double* buckets,
+                     long long* bucket_counts);
+int nx_deposit_allreduce(nx_ctx* ctx, nx_comm* comm, double* total);
+int nx_deposit_end(nx_ctx* ctx);
+
 /* ---- K3: constant-step driver with bounce (Output.py:368-455, bouncepackets.py)
  * Optional fused per-step image accumulation (image_dev / counts_dev device
  * pointers, may be NULL) and optional dense trajectory sink traj_host

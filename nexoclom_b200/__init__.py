@@ -11,12 +11,13 @@ from .Output import Output
 from .ModelImage import ModelImage
 from .ModelImageCube import ModelImageCube
 from .ModelDensity import ModelDensity
+from .ModelDeposition import ModelDeposition
 from .LOSResult import LOSResult
 from .LOSSpectrum import LOSSpectrum
 from .LOSResultFitted import LOSResultFitted
 from .solarsystem import SSObject
 from .input_classes import InputError
 
-__all__ = ['Input', 'Output', 'ModelImage', 'ModelImageCube', 'ModelDensity', 'LOSResult',
-           'LOSSpectrum', 'LOSResultFitted', 'SSObject', 'InputError']
+__all__ = ['Input', 'Output', 'ModelImage', 'ModelImageCube', 'ModelDensity', 'ModelDeposition',
+           'LOSResult', 'LOSSpectrum', 'LOSResultFitted', 'SSObject', 'InputError']
 __version__ = '0.1.0'

@@ -169,6 +169,12 @@ def load():
         'nx_cube_fetch': [vp, c_double_p, c_i64_p],
         'nx_cube_allreduce_total': [vp, vp, C.POINTER(C.c_double)],
         'nx_cube_end': [vp],
+        'nx_deposit_begin': [vp, C.c_int, C.c_int],
+        'nx_integrate_adaptive_deposit': [vp, i64, u64, u64, C.POINTER(u64), C.POINTER(u64),
+                                          C.POINTER(u64)],
+        'nx_deposit_fetch': [vp, c_double_p, c_i64_p, c_double_p, c_i64_p],
+        'nx_deposit_allreduce': [vp, vp, C.POINTER(C.c_double)],
+        'nx_deposit_end': [vp],
         'nx_density_accumulate': [vp, i64, i64, c_double_p, c_double_p, c_double_p, c_double_p,
                                   C.POINTER(u64)],
         'nx_source_map': [vp, i64, C.POINTER(SourceMapParams)] + [c_double_p] * 9 +

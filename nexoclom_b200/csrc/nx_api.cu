@@ -124,6 +124,11 @@ struct nx_ctx {
   // slot rides with the all-reduce), then ncell u64 counts, one allocation freed by end
   int cube_nx = 0, cube_nz = 0, cube_nbins = 0;
   double* cube = nullptr;
+  // context-owned deposition sink (nx_deposit_begin .. nx_deposit_end), one allocation: ncell
+  // f64 map sums, NX_DEP_NBUCKET f64 bucket sums, one f64 slot that rides with the all-reduce,
+  // then ncell u64 cell counts, NX_DEP_NBUCKET u64 bucket counts and one unused slot
+  int dep_nlon = 0, dep_nlat = 0;
+  double* dep = nullptr;
   void* pinned = nullptr;      // grow-only pinned staging for small D2H results (image, LOS columns)
   size_t pinned_bytes = 0;
   unsigned* cmp_tiles = nullptr;     // compaction scratch (tile counts)
@@ -417,6 +422,7 @@ int nx_ctx_destroy(nx_ctx* ctx) {
   cudaFree(ctx->scalars); cudaFree(ctx->status); cudaFree(ctx->cmp_tiles);
   for (auto& sc : ctx->scr) cudaFree(sc.p);
   cudaFree(ctx->cube);
+  cudaFree(ctx->dep);
   cudaFree(ctx->squeue); cudaFreeHost(ctx->seq_host);
   if (ctx->pinned) cudaFreeHost(ctx->pinned);
   if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
@@ -824,8 +830,9 @@ static int check_status(nx_ctx* ctx) {
 // [3] bounces), longest first when ordering is on, inside the caller's timed section.
 // S != nullptr: packets bounce (nx_integrate_adaptive_bounce); the cost model then budgets
 // every packet's remaining time, since reaching the surface no longer ends its flight.
+// dep != nullptr: the SINK build of the same kernel (nx_integrate_adaptive_deposit).
 static int adaptive_resident(nx_ctx* ctx, long long n, const Spline2D* S, uint64_t seed,
-                             uint64_t first_id) {
+                             uint64_t first_id, const DepositOut* dep = nullptr) {
   const bool order = ctx->order_packets && n >= 4096;
   const bool to_surface = !S || perfect_sticking(ctx->params);
   if (order)
@@ -835,7 +842,7 @@ static int adaptive_resident(nx_ctx* ctx, long long n, const Spline2D* S, uint64
                                ctx->params,
                                ctx->radpres.view, ctx->radpres.fast,
                                order ? ctx->perm : nullptr, ctx->scalars, ctx->scalars + 1,
-                               ctx->att, ctx->acc, ctx->status, S, seed, first_id));
+                               ctx->att, ctx->acc, ctx->status, S, seed, first_id, dep));
   return end_timed(ctx, order ? 4 : 1);
 }
 
@@ -916,6 +923,121 @@ int nx_integrate_adaptive_bounce(nx_ctx* ctx, long long n, uint64_t seed, uint64
   if (accepted) *accepted = h[2];
   if (bounces) *bounces = h[3];
   return r;
+}
+
+// ---- K2d: deposition maps and the loss budget (ModelDeposition) ----------------------------
+// The sink has its own allocation, released by nx_deposit_end.  nx_integrate_adaptive_deposit
+// runs the SINK build of the kernel nx_integrate_adaptive (perfect sticking) or
+// nx_integrate_adaptive_bounce would run, on the resident packets: the same final state and
+// step totals, plus the events added to the sink.
+static long long deposit_cells(const nx_ctx* ctx) { return (long long)ctx->dep_nlon * ctx->dep_nlat; }
+static long long deposit_half(const nx_ctx* ctx) { return deposit_cells(ctx) + NX_DEP_NBUCKET + 1; }
+static_assert((int)NX_DEP_SURFACE == DEP_SURFACE && (int)NX_DEP_MOON == DEP_MOON &&
+                  (int)NX_DEP_ESCAPED == DEP_ESCAPED && (int)NX_DEP_VANISHED == DEP_VANISHED &&
+                  (int)NX_DEP_REMAINING == DEP_REMAINING && (int)NX_DEP_SOURCE == DEP_SOURCE &&
+                  (int)NX_DEP_NBUCKET == DEP_NBUCKET,
+              "nx_deposit_bucket and DepositBucket disagree");
+
+int nx_deposit_end(nx_ctx* ctx) {
+  CK(cudaSetDevice(ctx->device));
+  if (ctx->dep) {
+    CK(cudaStreamSynchronize(ctx->stream));
+    CK(cudaFree(ctx->dep));
+  }
+  ctx->dep = nullptr;
+  ctx->dep_nlon = ctx->dep_nlat = 0;
+  return 0;
+}
+
+int nx_deposit_begin(nx_ctx* ctx, int nlon, int nlat) {
+  CK(cudaSetDevice(ctx->device));
+  if (nlon < 1 || nlat < 1) { ctx->err = "nx_deposit_begin: nlon and nlat must be >= 1"; return -1; }
+  if ((double)nlon * nlat >= 2147483648.0) {
+    ctx->err = "nx_deposit_begin: nlon * nlat must be < 2^31";
+    return -1;
+  }
+  const long long half = (long long)nlon * nlat + NX_DEP_NBUCKET + 1;
+  if (!ctx->dep || half != deposit_half(ctx)) {
+    int r = nx_deposit_end(ctx);
+    if (r) return r;
+    CK(dev_malloc(&ctx->dep, (size_t)(2 * half) * sizeof(double)));
+  }
+  ctx->dep_nlon = nlon; ctx->dep_nlat = nlat;
+  CK(cudaMemsetAsync(ctx->dep, 0, (size_t)(2 * half) * sizeof(double), ctx->stream));
+  return 0;
+}
+
+int nx_integrate_adaptive_deposit(nx_ctx* ctx, long long n, uint64_t seed, uint64_t first_id,
+                                  unsigned long long* attempted, unsigned long long* accepted,
+                                  unsigned long long* bounces) {
+  ENTER(ctx);
+  if (!ctx->dep) { ctx->err = "nx_deposit_begin not called"; return -1; }
+  if (!ctx->have_params) { ctx->err = "nx_tables_upload not called"; return -1; }
+  ctx->bound = nullptr;            // integrators work on the slab
+  if (n < 0 || n > ctx->cap) { ctx->err = "n exceeds resident packets"; return -1; }
+  const RunParams& p = ctx->params;
+  const bool bounce = !perfect_sticking(p);
+  if (bounce && p.accomfactor != 0.0 && !ctx->spl_c) {
+    ctx->err = "accommodation enabled but no speed spline uploaded";
+    return -1;
+  }
+  CK(cudaMemsetAsync(ctx->scalars, 0, 8 * sizeof(unsigned long long), ctx->stream));
+  int r;
+  if (n > 0) {
+    const long long ncell = deposit_cells(ctx), half = deposit_half(ctx);
+    DepositOut d;
+    d.map = ctx->dep;
+    d.bucket = ctx->dep + ncell;
+    d.cnt = reinterpret_cast<unsigned long long*>(ctx->dep + half);
+    d.bucket_n = d.cnt + ncell;
+    d.nlon = ctx->dep_nlon; d.nlat = ctx->dep_nlat;
+    if ((r = begin_timed(ctx))) return r;
+    if ((r = adaptive_resident(ctx, n, bounce ? &ctx->spline : nullptr, seed, first_id, &d)))
+      return r;
+    ctx->fresh = false;
+  }
+  unsigned long long h[4] = {0, 0, 0, 0};
+  CK(cudaMemcpyAsync(h, ctx->scalars, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
+  r = check_status(ctx);
+  if (r < 0) return r;
+  if (attempted) *attempted = h[1];
+  if (accepted) *accepted = h[2];
+  if (bounces) *bounces = h[3];
+  return r;
+}
+
+int nx_deposit_fetch(nx_ctx* ctx, double* map, long long* counts, double* buckets,
+                     long long* bucket_counts) {
+  CK(cudaSetDevice(ctx->device));
+  if (!ctx->dep) { ctx->err = "nx_deposit_begin not called"; return -1; }
+  const long long ncell = deposit_cells(ctx), half = deposit_half(ctx);
+  const double* d = ctx->dep;
+  if (map) CK(cudaMemcpyAsync(map, d, ncell * 8, cudaMemcpyDeviceToHost, ctx->stream));
+  if (buckets)
+    CK(cudaMemcpyAsync(buckets, d + ncell, NX_DEP_NBUCKET * 8, cudaMemcpyDeviceToHost, ctx->stream));
+  if (counts) CK(cudaMemcpyAsync(counts, d + half, ncell * 8, cudaMemcpyDeviceToHost, ctx->stream));
+  if (bucket_counts)
+    CK(cudaMemcpyAsync(bucket_counts, d + half + ncell, NX_DEP_NBUCKET * 8, cudaMemcpyDeviceToHost,
+                       ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  return 0;
+}
+
+// The one collective of a sharded deposition: map, counts and buckets of every rank of `comm`,
+// in place, with *total (if not NULL) riding in the slot after the bucket sums.
+int nx_deposit_allreduce(nx_ctx* ctx, nx_comm* comm, double* total) {
+  CK(cudaSetDevice(ctx->device));
+  if (!ctx->dep) { ctx->err = "nx_deposit_begin not called"; return -1; }
+  const long long half = deposit_half(ctx);
+  double* slot = ctx->dep + half - 1;
+  CK(cudaMemsetAsync(slot, 0, sizeof(double), ctx->stream));
+  if (total) CK(cudaMemcpyAsync(slot, total, sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+  int r = nx_allreduce(comm, ctx->dep, half, NX_DTYPE_F64, ctx->stream);
+  if (r == 0) r = nx_allreduce(comm, ctx->dep + half, half, NX_DTYPE_I64, ctx->stream);
+  if (r) { ctx->err = std::string("nx_deposit_allreduce: ") + nx_comm_last_error(); return r; }
+  if (total) CK(cudaMemcpyAsync(total, slot, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  return 0;
 }
 
 // Host-buffer variant of K2 for the end-to-end path.  schedule 1 (default): ONE

@@ -306,11 +306,11 @@ NX_HD void fast_stages(const RunParams& p, const FastTable& T, const double* s, 
 
 // One attempted adaptive step, fast arithmetic.  Same contract as
 // adaptive_attempt<>(): s[0..7] = time,x,y,z,vx,vy,vz,frac; returns AttemptFlags.
-// BOUNCE, S, seed, id, k: as in adaptive_attempt<>().
-template <int GR, int RP, int LOSS, int MO = 0, bool BOUNCE = false>
+// BOUNCE, S, seed, id, k, SINK, D: as in adaptive_attempt<>().
+template <int GR, int RP, int LOSS, int MO = 0, bool BOUNCE = false, bool SINK = false>
 NX_HD int adaptive_attempt_fast(const RunParams& p, const FastTable& T, double* s,
                                 double& step, const Spline2D* S = nullptr, uint64_t seed = 0,
-                                uint64_t id = 0, uint32_t k = 0) {
+                                uint64_t id = 0, uint32_t k = 0, DepositSink* D = nullptr) {
   const double res = p.resolution;
   const double resv = 0.1 * res;
   const double h = fmin(s[0], step);
@@ -349,23 +349,37 @@ NX_HD int adaptive_attempt_fast(const RunParams& p, const FastTable& T, double* 
   if (accept) {
     const double r2 = fma(pz, pz, fma(py, py, px * px));
     double f = fn;
+    double dep = 0.0, ff = 0.0;            // SINK: deposited frac, frac of the fate event
+    int fate = -1;
     if (fn < 0.0) flags |= ATT_NEG_FRAC;
     if (r2 < 1.0) {
       if (BOUNCE && !perfect_sticking(p)) {  // bounce, then K3's tests on the new state
         double b[8] = {0.0, px, py, pz, vx, vy, vz, fn};
         adaptive_surface<true>(p, *S, b, r2, seed, id, k);
         px = b[1]; py = b[2]; pz = b[3]; vx = b[4]; vy = b[5]; vz = b[6]; f = b[7];
+        if (SINK) dep = fn - f;
         flags |= ATT_BOUNCED;
       } else {
+        if (SINK) dep = fn;
         f = 0.0;                           // impact, stickcoef == 1 (Q6)
       }
     }
     if (MO) {                              // impact on the moon
       const double dx = px - moon_end[0], dy = py - moon_end[1];
-      if (fma(pz, pz, fma(dy, dy, dx * dx)) < p.moon_r2[0]) f = 0.0;
+      if (fma(pz, pz, fma(dy, dy, dx * dx)) < p.moon_r2[0]) {
+        if (SINK && f != 0.0) { fate = DEP_MOON; ff = f; }
+        f = 0.0;
+      }
     }
-    if (r2 > p.outeredge) f = 0.0;         // escape: r^2 vs outeredge (Q7)
-    if (f < 1e-10) f = 0.0;                // vanish (Q8)
+    if (r2 > p.outeredge) {                // escape: r^2 vs outeredge (Q7)
+      if (SINK && f != 0.0) { fate = DEP_ESCAPED; ff = f; }
+      f = 0.0;
+    }
+    if (f < 1e-10) {                       // vanish (Q8)
+      if (SINK && f != 0.0) { fate = DEP_VANISHED; ff = f; }
+      f = 0.0;
+    }
+    if (SINK && (r2 < 1.0 || fate >= 0)) deposit_record(*D, r2 < 1.0, px, py, pz, dep, fate, ff);
     s[0] = (f == 0.0) ? 0.0 : s[0] - h;
     s[1] = px; s[2] = py; s[3] = pz; s[4] = vx; s[5] = vy; s[6] = vz;
     s[7] = f;
@@ -379,27 +393,28 @@ NX_HD int adaptive_attempt_fast(const RunParams& p, const FastTable& T, double* 
 }
 
 // runtime dispatch over the compile-time force / loss combinations
-template <bool BOUNCE = false>
+template <bool BOUNCE = false, bool SINK = false>
 NX_HD int adaptive_attempt_fast_rt(const RunParams& p, const FastTable& T, double* s,
                                    double& step, const Spline2D* S = nullptr, uint64_t seed = 0,
-                                   uint64_t id = 0, uint32_t k = 0) {
-#define NX_ARGS p, T, s, step, S, seed, id, k
+                                   uint64_t id = 0, uint32_t k = 0,
+                                   DepositSink* D = nullptr) {
+#define NX_ARGS p, T, s, step, S, seed, id, k, D
   if (p.nmoons == 1 && p.gravity) {
     if (p.radpres) {
-      if (p.loss_mode == LOSS_PHOTO) return adaptive_attempt_fast<1, 1, LOSS_PHOTO, 1, BOUNCE>(NX_ARGS);
-      if (p.loss_mode == LOSS_LIFETIME) return adaptive_attempt_fast<1, 1, LOSS_LIFETIME, 1, BOUNCE>(NX_ARGS);
-      return adaptive_attempt_fast<1, 1, LOSS_NONE, 1, BOUNCE>(NX_ARGS);
+      if (p.loss_mode == LOSS_PHOTO) return adaptive_attempt_fast<1, 1, LOSS_PHOTO, 1, BOUNCE, SINK>(NX_ARGS);
+      if (p.loss_mode == LOSS_LIFETIME) return adaptive_attempt_fast<1, 1, LOSS_LIFETIME, 1, BOUNCE, SINK>(NX_ARGS);
+      return adaptive_attempt_fast<1, 1, LOSS_NONE, 1, BOUNCE, SINK>(NX_ARGS);
     }
-    if (p.loss_mode == LOSS_PHOTO) return adaptive_attempt_fast<1, 0, LOSS_PHOTO, 1, BOUNCE>(NX_ARGS);
-    if (p.loss_mode == LOSS_LIFETIME) return adaptive_attempt_fast<1, 0, LOSS_LIFETIME, 1, BOUNCE>(NX_ARGS);
-    return adaptive_attempt_fast<1, 0, LOSS_NONE, 1, BOUNCE>(NX_ARGS);
+    if (p.loss_mode == LOSS_PHOTO) return adaptive_attempt_fast<1, 0, LOSS_PHOTO, 1, BOUNCE, SINK>(NX_ARGS);
+    if (p.loss_mode == LOSS_LIFETIME) return adaptive_attempt_fast<1, 0, LOSS_LIFETIME, 1, BOUNCE, SINK>(NX_ARGS);
+    return adaptive_attempt_fast<1, 0, LOSS_NONE, 1, BOUNCE, SINK>(NX_ARGS);
   }
   const int key = (p.gravity ? 4 : 0) | (p.radpres ? 2 : 0);
 #define NX_CASE(G, R)                                                                    \
   if (key == ((G) * 4 + (R) * 2)) {                                                      \
-    if (p.loss_mode == LOSS_PHOTO) return adaptive_attempt_fast<G, R, LOSS_PHOTO, 0, BOUNCE>(NX_ARGS);       \
-    if (p.loss_mode == LOSS_LIFETIME) return adaptive_attempt_fast<G, R, LOSS_LIFETIME, 0, BOUNCE>(NX_ARGS); \
-    return adaptive_attempt_fast<G, R, LOSS_NONE, 0, BOUNCE>(NX_ARGS);                     \
+    if (p.loss_mode == LOSS_PHOTO) return adaptive_attempt_fast<G, R, LOSS_PHOTO, 0, BOUNCE, SINK>(NX_ARGS);       \
+    if (p.loss_mode == LOSS_LIFETIME) return adaptive_attempt_fast<G, R, LOSS_LIFETIME, 0, BOUNCE, SINK>(NX_ARGS); \
+    return adaptive_attempt_fast<G, R, LOSS_NONE, 0, BOUNCE, SINK>(NX_ARGS);                     \
   }
   NX_CASE(1, 1) NX_CASE(1, 0) NX_CASE(0, 1) NX_CASE(0, 0)
 #undef NX_CASE

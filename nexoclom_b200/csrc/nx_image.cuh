@@ -64,6 +64,23 @@ NX_HD int hist_bin_fast(double v, int n, double lo, double hi, double step, doub
   return k;
 }
 
+// Surface longitude / latitude of a deposition event at (x, y, z): the bounce's convention
+// (nx_surface.cuh::bounce), lon = fmod(atan2(x, -y) + 2 pi, 2 pi), lat = atan2(z, |(x, y)|).
+NX_HD void deposit_lonlat(double x, double y, double z, double& lon, double& lat) {
+  lon = fmod(add_rn(atan2(x, -y), NX_TWO_PI), NX_TWO_PI);
+  lat = atan2(z, sqrt(add_rn(mul_rn(x, x), mul_rn(y, y))));
+}
+
+// Deposition map cell (lon-major: ilon * nlat + ilat) on np.histogram2d's axes
+// linspace(0, 2 pi, nlon + 1) x linspace(-pi/2, pi/2, nlat + 1), the axes of make_source_map;
+// -1 outside.
+NX_HD int deposit_cell(double lon, double lat, int nlon, int nlat) {
+  const double half_pi = NX_PI / 2.0;
+  const int i = hist_bin(lon, nlon, 0.0, NX_TWO_PI, NX_TWO_PI / nlon);
+  const int j = hist_bin(lat, nlat, -half_pi, half_pi, (half_pi - -half_pi) / nlat);
+  return (i < 0 || j < 0) ? -1 : i * nlat + j;
+}
+
 // per-launch constants of the image kernels
 struct ImageSteps {
   double step_x, step_z;          // bin widths, as np.histogram2d's linspace gives them

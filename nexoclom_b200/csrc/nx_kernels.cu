@@ -297,7 +297,11 @@ struct PacketFeeder {
 // BOUNCE: packets that hit the surface bounce (adaptive_attempt<.., true>), the deviates of
 // packet idx are keyed by (seed, first_id + idx); totals[2] receives the number of bounces.
 // S / seed / first_id are unused otherwise.
-template <int MODE, bool BOUNCE = false>
+// SINK: the deposition sink (ModelDeposition): the attempts record every surface, moon, escape
+// and vanish event (deposit_record), the kernel the initial frac (SOURCE) and the frac of the
+// packets that retire alive (REMAINING); Dep is unused otherwise.  The final state and the
+// step totals are the same as without the sink.
+template <int MODE, bool BOUNCE = false, bool SINK = false>
 __global__ void __launch_bounds__(NX_INT_THREADS, NX_INT_MINBLOCKS)
 k_integrate_adaptive(StateCols In, StateCols P, long long n, RunParams p, InterpTable Tg,
                      FastTable Fg, const unsigned* __restrict__ perm,
@@ -305,7 +309,7 @@ k_integrate_adaptive(StateCols In, StateCols P, long long n, RunParams p, Interp
                      unsigned long long* __restrict__ totals,
                      unsigned* __restrict__ att_out, unsigned* __restrict__ acc_out,
                      int* __restrict__ status, unsigned table_bytes, Spline2D S, uint64_t seed,
-                     uint64_t first_id) {
+                     uint64_t first_id, DepositOut Dep) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   InterpTable T;
   FastTable F;
@@ -326,6 +330,12 @@ k_integrate_adaptive(StateCols In, StateCols P, long long n, RunParams p, Interp
   unsigned att = 0, acc = 0;
   unsigned long long tot_att = 0, tot_acc = 0, tot_bnc = 0;
   int st = 0;
+  DepositSink D;                 // SINK: lives in local memory, touched on events only
+  if (SINK) {
+    D.map = Dep.map; D.cnt = Dep.cnt; D.nlon = Dep.nlon; D.nlat = Dep.nlat;
+#pragma unroll
+    for (int b = 0; b < DEP_NBUCKET; ++b) { D.sum[b] = 0.0; D.n[b] = 0; }
+  }
 #ifdef NX_STREAM_DEBUG
   unsigned long long dbg_iters = 0;
 #endif
@@ -345,6 +355,10 @@ k_integrate_adaptive(StateCols In, StateCols P, long long n, RunParams p, Interp
         idx = feed.ids[feed.buf * 32 + slot];
         att = 0; acc = 0;
         have = (s[0] > p.resolution) && (s[7] > 0.0);
+        if (SINK && s[7] > 0.0) {
+          D.sum[DEP_SOURCE] += s[7]; ++D.n[DEP_SOURCE];
+          if (!have) { D.sum[DEP_REMAINING] += s[7]; ++D.n[DEP_REMAINING]; }
+        }
         if (!have) {
           att_out[idx] = 0; acc_out[idx] = 0;
           if (pass_through) {
@@ -365,10 +379,12 @@ k_integrate_adaptive(StateCols In, StateCols P, long long n, RunParams p, Interp
     if (have) {
       int fl;
       if (MODE < 0)
-        fl = adaptive_attempt<true, BOUNCE>(p, T, s, step, &S, seed, first_id + idx, acc + 1);
+        fl = adaptive_attempt<true, BOUNCE, SINK>(p, T, s, step, &S, seed, first_id + idx, acc + 1,
+                                                  SINK ? &D : nullptr);
       else
-        fl = adaptive_attempt_fast<(MODE >> 3) & 1, (MODE >> 2) & 1, MODE & 3, (MODE >> 4) & 1, BOUNCE>(
-            p, F, s, step, &S, seed, first_id + idx, acc + 1);
+        fl = adaptive_attempt_fast<(MODE >> 3) & 1, (MODE >> 2) & 1, MODE & 3, (MODE >> 4) & 1, BOUNCE,
+                                   SINK>(p, F, s, step, &S, seed, first_id + idx, acc + 1,
+                                         SINK ? &D : nullptr);
       ++att;
       if (fl & ATT_ACCEPTED) ++acc;
       if (BOUNCE && (fl & ATT_BOUNCED)) ++tot_bnc;
@@ -380,6 +396,7 @@ k_integrate_adaptive(StateCols In, StateCols P, long long n, RunParams p, Interp
         __stcs(P.c[8] + idx, step);
         att_out[idx] = att; acc_out[idx] = acc;
         tot_att += att; tot_acc += acc;
+        if (SINK && s[7] > 0.0) { D.sum[DEP_REMAINING] += s[7]; ++D.n[DEP_REMAINING]; }
         have = false;
       }
     }
@@ -401,6 +418,22 @@ k_integrate_adaptive(StateCols In, StateCols P, long long n, RunParams p, Interp
     atomicMax(&g_dbg[16], dbg_now());
     atomicAdd(&g_dbg[17], dbg_iters);
 #endif
+  }
+  if (SINK) {
+#pragma unroll
+    for (int b = 0; b < DEP_NBUCKET; ++b) {
+      double v = D.sum[b];
+      unsigned long long c = D.n[b];
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+        v += __shfl_xor_sync(FULL_MASK, v, o);
+        c += __shfl_xor_sync(FULL_MASK, c, o);
+      }
+      if (lane == 0 && c) {
+        atomicAdd(Dep.bucket + b, v);
+        atomicAdd(Dep.bucket_n + b, c);
+      }
+    }
   }
 }
 
@@ -1523,7 +1556,7 @@ static cudaError_t persistent_grid(K kernel, int device, size_t smem, int* block
   return cudaSuccess;
 }
 
-template <int MODE, bool BOUNCE = false>
+template <int MODE, bool BOUNCE = false, bool SINK = false>
 static cudaError_t launch_adaptive_mode(cudaStream_t st, int device, StateCols In, StateCols P,
                                         long long n,
                                         const RunParams& p, const InterpTable& T,
@@ -1531,17 +1564,17 @@ static cudaError_t launch_adaptive_mode(cudaStream_t st, int device, StateCols I
                                         const unsigned* perm, unsigned long long* queue,
                                         unsigned long long* totals, unsigned* att, unsigned* acc,
                                         int* status, const Spline2D& S, uint64_t seed,
-                                        uint64_t first_id) {
+                                        uint64_t first_id, const DepositOut& Dep) {
   const size_t tbytes = (MODE < 0) ? table_smem_bytes(T) : fast_table_smem_bytes(F);
   const size_t smem = tbytes + (size_t)(NX_INT_THREADS / 32) * NX_FEED_BYTES_PER_WARP;
   int blocks = 0;
-  cudaError_t e = persistent_grid(k_integrate_adaptive<MODE, BOUNCE>, device, smem, &blocks);
+  cudaError_t e = persistent_grid(k_integrate_adaptive<MODE, BOUNCE, SINK>, device, smem, &blocks);
   if (e != cudaSuccess) return e;
   const long long need = (n + NX_INT_THREADS - 1) / NX_INT_THREADS;
   if (need < blocks) blocks = (int)(need > 0 ? need : 1);
-  k_integrate_adaptive<MODE, BOUNCE><<<blocks, NX_INT_THREADS, smem, st>>>(
+  k_integrate_adaptive<MODE, BOUNCE, SINK><<<blocks, NX_INT_THREADS, smem, st>>>(
       In, P, n, p, T, F, perm, queue, totals, att, acc, status, (unsigned)tbytes, S, seed,
-      first_id);
+      first_id, Dep);
   return cudaGetLastError();
 }
 
@@ -1646,60 +1679,77 @@ cudaError_t launch_cost_order(cudaStream_t st, int device, StateCols P, long lon
   return cudaGetLastError();
 }
 
+// K2 / K2b kernel selection; SINK builds exist for every kernel it can select.
+template <bool SINK>
+static cudaError_t dispatch_adaptive(cudaStream_t st, int device, StateCols In, StateCols P,
+                                     long long n, const RunParams& p, const InterpTable& T,
+                                     const FastTable& F, const unsigned* perm,
+                                     unsigned long long* queue, unsigned long long* totals,
+                                     unsigned* att, unsigned* acc, int* status,
+                                     const Spline2D* S, uint64_t seed, uint64_t first_id,
+                                     const DepositOut& Dep) {
+#define NX_ARGS st, device, In, P, n, p, T, F, perm, queue, totals, att, acc, status, \
+                S ? *S : Spline2D{}, seed, first_id, Dep
+  if (S) {
+    // bounce builds: the strict kernel, and the fast kernels with gravity (one moon too);
+    // runs without gravity or with more moons take the strict kernel
+    if (p.strict_math || !p.gravity || p.nmoons > 1) return launch_adaptive_mode<-1, true, SINK>(NX_ARGS);
+    switch ((p.radpres ? 4 : 0) | (p.loss_mode & 3) | (p.nmoons == 1 ? 16 : 0)) {
+      case 16: return launch_adaptive_mode<24, true, SINK>(NX_ARGS);
+      case 17: return launch_adaptive_mode<25, true, SINK>(NX_ARGS);
+      case 18: return launch_adaptive_mode<26, true, SINK>(NX_ARGS);
+      case 20: return launch_adaptive_mode<28, true, SINK>(NX_ARGS);
+      case 21: return launch_adaptive_mode<29, true, SINK>(NX_ARGS);
+      case 22: return launch_adaptive_mode<30, true, SINK>(NX_ARGS);
+      case 0: return launch_adaptive_mode<8, true, SINK>(NX_ARGS);
+      case 1: return launch_adaptive_mode<9, true, SINK>(NX_ARGS);
+      case 2: return launch_adaptive_mode<10, true, SINK>(NX_ARGS);
+      case 4: return launch_adaptive_mode<12, true, SINK>(NX_ARGS);
+      case 5: return launch_adaptive_mode<13, true, SINK>(NX_ARGS);
+      case 6: return launch_adaptive_mode<14, true, SINK>(NX_ARGS);
+      default: return cudaErrorInvalidValue;
+    }
+  }
+  if (p.strict_math || p.nmoons > 1 || (p.nmoons == 1 && !p.gravity))
+    return launch_adaptive_mode<-1, false, SINK>(NX_ARGS);
+  const int mode = (p.gravity ? 8 : 0) | (p.radpres ? 4 : 0) | (p.loss_mode & 3) |
+                   (p.nmoons == 1 ? 16 : 0);
+  switch (mode) {
+    case 24: return launch_adaptive_mode<24, false, SINK>(NX_ARGS);
+    case 25: return launch_adaptive_mode<25, false, SINK>(NX_ARGS);
+    case 26: return launch_adaptive_mode<26, false, SINK>(NX_ARGS);
+    case 28: return launch_adaptive_mode<28, false, SINK>(NX_ARGS);
+    case 29: return launch_adaptive_mode<29, false, SINK>(NX_ARGS);
+    case 30: return launch_adaptive_mode<30, false, SINK>(NX_ARGS);
+    case 0: return launch_adaptive_mode<0, false, SINK>(NX_ARGS);
+    case 1: return launch_adaptive_mode<1, false, SINK>(NX_ARGS);
+    case 2: return launch_adaptive_mode<2, false, SINK>(NX_ARGS);
+    case 4: return launch_adaptive_mode<4, false, SINK>(NX_ARGS);
+    case 5: return launch_adaptive_mode<5, false, SINK>(NX_ARGS);
+    case 6: return launch_adaptive_mode<6, false, SINK>(NX_ARGS);
+    case 8: return launch_adaptive_mode<8, false, SINK>(NX_ARGS);
+    case 9: return launch_adaptive_mode<9, false, SINK>(NX_ARGS);
+    case 10: return launch_adaptive_mode<10, false, SINK>(NX_ARGS);
+    case 12: return launch_adaptive_mode<12, false, SINK>(NX_ARGS);
+    case 13: return launch_adaptive_mode<13, false, SINK>(NX_ARGS);
+    case 14: return launch_adaptive_mode<14, false, SINK>(NX_ARGS);
+    default: return cudaErrorInvalidValue;
+  }
+#undef NX_ARGS
+}
+
 cudaError_t launch_integrate_adaptive(cudaStream_t st, int device, StateCols In, StateCols P,
                                       long long n, const RunParams& p, const InterpTable& T,
                                       const FastTable& F, const unsigned* perm,
                                       unsigned long long* queue, unsigned long long* totals,
                                       unsigned* att, unsigned* acc, int* status,
-                                      const Spline2D* S, uint64_t seed, uint64_t first_id) {
-#define NX_ARGS st, device, In, P, n, p, T, F, perm, queue, totals, att, acc, status, \
-                S ? *S : Spline2D{}, seed, first_id
-  if (S) {
-    // bounce builds: the strict kernel, and the fast kernels with gravity (one moon too);
-    // runs without gravity or with more moons take the strict kernel
-    if (p.strict_math || !p.gravity || p.nmoons > 1) return launch_adaptive_mode<-1, true>(NX_ARGS);
-    switch ((p.radpres ? 4 : 0) | (p.loss_mode & 3) | (p.nmoons == 1 ? 16 : 0)) {
-      case 16: return launch_adaptive_mode<24, true>(NX_ARGS);
-      case 17: return launch_adaptive_mode<25, true>(NX_ARGS);
-      case 18: return launch_adaptive_mode<26, true>(NX_ARGS);
-      case 20: return launch_adaptive_mode<28, true>(NX_ARGS);
-      case 21: return launch_adaptive_mode<29, true>(NX_ARGS);
-      case 22: return launch_adaptive_mode<30, true>(NX_ARGS);
-      case 0: return launch_adaptive_mode<8, true>(NX_ARGS);
-      case 1: return launch_adaptive_mode<9, true>(NX_ARGS);
-      case 2: return launch_adaptive_mode<10, true>(NX_ARGS);
-      case 4: return launch_adaptive_mode<12, true>(NX_ARGS);
-      case 5: return launch_adaptive_mode<13, true>(NX_ARGS);
-      case 6: return launch_adaptive_mode<14, true>(NX_ARGS);
-      default: return cudaErrorInvalidValue;
-    }
-  }
-  if (p.strict_math || p.nmoons > 1 || (p.nmoons == 1 && !p.gravity))
-    return launch_adaptive_mode<-1>(NX_ARGS);
-  const int mode = (p.gravity ? 8 : 0) | (p.radpres ? 4 : 0) | (p.loss_mode & 3) |
-                   (p.nmoons == 1 ? 16 : 0);
-  switch (mode) {
-    case 24: return launch_adaptive_mode<24>(NX_ARGS);
-    case 25: return launch_adaptive_mode<25>(NX_ARGS);
-    case 26: return launch_adaptive_mode<26>(NX_ARGS);
-    case 28: return launch_adaptive_mode<28>(NX_ARGS);
-    case 29: return launch_adaptive_mode<29>(NX_ARGS);
-    case 30: return launch_adaptive_mode<30>(NX_ARGS);
-    case 0: return launch_adaptive_mode<0>(NX_ARGS);
-    case 1: return launch_adaptive_mode<1>(NX_ARGS);
-    case 2: return launch_adaptive_mode<2>(NX_ARGS);
-    case 4: return launch_adaptive_mode<4>(NX_ARGS);
-    case 5: return launch_adaptive_mode<5>(NX_ARGS);
-    case 6: return launch_adaptive_mode<6>(NX_ARGS);
-    case 8: return launch_adaptive_mode<8>(NX_ARGS);
-    case 9: return launch_adaptive_mode<9>(NX_ARGS);
-    case 10: return launch_adaptive_mode<10>(NX_ARGS);
-    case 12: return launch_adaptive_mode<12>(NX_ARGS);
-    case 13: return launch_adaptive_mode<13>(NX_ARGS);
-    case 14: return launch_adaptive_mode<14>(NX_ARGS);
-    default: return cudaErrorInvalidValue;
-  }
-#undef NX_ARGS
+                                      const Spline2D* S, uint64_t seed, uint64_t first_id,
+                                      const DepositOut* dep) {
+  if (dep)
+    return dispatch_adaptive<true>(st, device, In, P, n, p, T, F, perm, queue, totals, att, acc,
+                                   status, S, seed, first_id, *dep);
+  return dispatch_adaptive<false>(st, device, In, P, n, p, T, F, perm, queue, totals, att, acc,
+                                  status, S, seed, first_id, DepositOut{});
 }
 
 template <int MODE>

@@ -143,16 +143,27 @@ cudaError_t launch_image_finish(cudaStream_t st, const double* img, const unsign
 cudaError_t launch_cost_order(cudaStream_t st, int device, StateCols P, long long n,
                               const RunParams& p, int model, unsigned char* bucket,
                               unsigned* hist_cursor, unsigned* perm, bool to_surface = true);
+// Deposition sink of K2 (nx_integrate_adaptive_deposit): the nlon x nlat map (f64 sums and
+// u64 counts, longitude major) and the DEP_NBUCKET bucket sums and counts, all device memory
+// the kernel adds to.
+struct DepositOut {
+  double* map;
+  unsigned long long* cnt;
+  double* bucket;
+  unsigned long long* bucket_n;
+  int nlon, nlat;
+};
 // In: columns the initial state is read from (X0 slab right after K1, else == P).
 // S != nullptr: packets bounce (totals[2] counts the bounces), deviates keyed by
 // (seed, first_id + packet index); nullptr: the reference's driver (Q6).
+// dep != nullptr: the same run through the kernel's SINK build, which adds its events to *dep.
 cudaError_t launch_integrate_adaptive(cudaStream_t st, int device, StateCols In, StateCols P,
                                       long long n, const RunParams& p, const InterpTable& T,
                                       const FastTable& F, const unsigned* perm,
                                       unsigned long long* queue, unsigned long long* totals,
                                       unsigned* att, unsigned* acc, int* status,
                                       const Spline2D* S = nullptr, uint64_t seed = 0,
-                                      uint64_t first_id = 0);
+                                      uint64_t first_id = 0, const DepositOut* dep = nullptr);
 #define NX_STREAM_GROUP 128          // == NX_GROUP: segment sizes are multiples of this
 #define NX_STREAM_MAX_SEG 32
 #define NX_STREAM_CURSORS 256        // >= NX_NCLASS x 32 u64 cursors

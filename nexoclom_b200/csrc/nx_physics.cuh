@@ -422,13 +422,45 @@ NX_HD bool perfect_sticking(const RunParams& p) {
   return p.sticktype == STICK_CONSTANT && p.stickcoef == 1.0;
 }
 
+// Where the frac of the packets goes (SINK builds of the adaptive driver, ModelDeposition);
+// the order of nx_deposit_bucket in nexoclom_b200.h.
+enum DepositBucket {
+  DEP_SURFACE = 0,        // deposited on the planet's surface (mapped)
+  DEP_MOON = 1,           // hit a moon
+  DEP_ESCAPED = 2,        // r^2 > outeredge (Q7)
+  DEP_VANISHED = 3,       // frac < 1e-10 (Q8)
+  DEP_REMAINING = 4,      // still in flight when the packet retires
+  DEP_SOURCE = 5,         // initial frac > 0 of the packets handed to the kernel
+  DEP_NBUCKET = 6
+};
+
+// One lane's deposition sink: the device map (nlon x nlat cells, longitude major) and this
+// lane's bucket sums and counts, reduced when the kernel ends.
+struct DepositSink {
+  double* map;
+  unsigned long long* cnt;
+  int nlon, nlat;
+  double sum[DEP_NBUCKET];
+  unsigned long long n[DEP_NBUCKET];
+};
+
+// Records the events of one accepted step (SINK builds): surf = the step ended inside the
+// planet, `dep` of frac deposited at the surface point (x, y, z) into the map and SURFACE;
+// fate >= 0: the bucket that took the remaining frac ff (MOON, ESCAPED, VANISHED).  Defined in
+// nx_surface.cuh, an out-of-line call like adaptive_surface().
+template <class Sink>
+NX_COLD void deposit_record(Sink& D, bool surf, double x, double y, double z, double dep,
+                            int fate, double ff);
+
 // BOUNCE = false: the reference's driver (a packet that hits the surface sticks, Q6).
 // BOUNCE = true: accepted steps that end inside the planet go through adaptive_surface()
 // unless the sticking is perfect; S / seed / id / k feed it (unused otherwise).
-template <bool STRICT, bool BOUNCE = false>
+// SINK = true: every surface, moon, escape and vanish event goes to deposit_record(*D); the
+// state the attempt computes is the same as without the sink.
+template <bool STRICT, bool BOUNCE = false, bool SINK = false>
 NX_HD int adaptive_attempt(const RunParams& p, const InterpTable& T, double* s, double& step,
                            const Spline2D* S = nullptr, uint64_t seed = 0, uint64_t id = 0,
-                           uint32_t k = 0) {
+                           uint32_t k = 0, DepositSink* D = nullptr) {
   const double res = p.resolution;
   const double resv = mul_rn(0.1, res);
   const double h = fmin(s[0], step);
@@ -455,12 +487,16 @@ NX_HD int adaptive_attempt(const RunParams& p, const InterpTable& T, double* s, 
   if (errmax < 1.0) {
     const double r2 = add_rn(add_rn(mul_rn(nx[1], nx[1]), mul_rn(nx[2], nx[2])), mul_rn(nx[3], nx[3]));
     double f = nx[7];
+    double dep = 0.0, ff = 0.0;            // SINK: deposited frac, frac of the fate event
+    int fate = -1;
     if (r2 < 1.0) {
       if (BOUNCE && !perfect_sticking(p)) {  // bounce, then K3's tests on the new state
         adaptive_surface<false>(p, *S, nx, r2, seed, id, k);
+        if (SINK) dep = f - nx[7];
         f = nx[7];
         flags |= ATT_BOUNCED;
       } else {
+        if (SINK) dep = f;
         f = 0.0;                           // impact, stickcoef == 1 (Q6)
       }
     }
@@ -468,10 +504,20 @@ NX_HD int adaptive_attempt(const RunParams& p, const InterpTable& T, double* s, 
       double mx, my;
       moon_position(p, m, nx[0], mx, my);
       const double dx = nx[1] - mx, dy = nx[2] - my;
-      if (dx * dx + dy * dy + nx[3] * nx[3] < p.moon_r2[m]) f = 0.0;
+      if (dx * dx + dy * dy + nx[3] * nx[3] < p.moon_r2[m]) {
+        if (SINK && f != 0.0) { fate = DEP_MOON; ff = f; }
+        f = 0.0;
+      }
     }
-    if (r2 > p.outeredge) f = 0.0;         // escape: r^2 vs outeredge (Q7)
-    if (f < 1e-10) f = 0.0;                // vanish (Q8)
+    if (r2 > p.outeredge) {                // escape: r^2 vs outeredge (Q7)
+      if (SINK && f != 0.0) { fate = DEP_ESCAPED; ff = f; }
+      f = 0.0;
+    }
+    if (f < 1e-10) {                       // vanish (Q8)
+      if (SINK && f != 0.0) { fate = DEP_VANISHED; ff = f; }
+      f = 0.0;
+    }
+    if (SINK && (r2 < 1.0 || fate >= 0)) deposit_record(*D, r2 < 1.0, nx[1], nx[2], nx[3], dep, fate, ff);
     s[0] = (f == 0.0) ? 0.0 : nx[0];
 #pragma unroll
     for (int k = 1; k < 7; ++k) s[k] = nx[k];

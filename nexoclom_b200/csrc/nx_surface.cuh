@@ -4,6 +4,7 @@
 // tests/_hostcheck.
 #pragma once
 #include "nx_fast.cuh"
+#include "nx_image.cuh"
 #include "nx_physics.cuh"
 
 namespace nx {
@@ -275,6 +276,32 @@ NX_COLD void adaptive_surface(const RunParams& p, const Spline2D& S, double* s, 
   uniform_pair(seed, id, STREAM_BOUNCE, 2u * k + 1u, u_prob, unused);
   if (FAST) bounce_fast(p, S, s, sqrt(r2), u_alt, u_az, u_prob);
   else bounce(p, S, s, sqrt(r2), u_alt, u_az, u_prob);
+}
+
+// Deposition events of one accepted adaptive step (declared in nx_physics.cuh).
+template <class Sink>
+NX_COLD void deposit_record(Sink& D, bool surf, double x, double y, double z, double dep,
+                            int fate, double ff) {
+  if (surf) {
+    D.sum[DEP_SURFACE] += dep;
+    D.n[DEP_SURFACE] += 1;
+    double lon, lat;
+    deposit_lonlat(x, y, z, lon, lat);
+    const int c = deposit_cell(lon, lat, D.nlon, D.nlat);
+    if (c >= 0) {
+#if defined(__CUDA_ARCH__)
+      atomicAdd(D.map + c, dep);
+      atomicAdd(D.cnt + c, 1ull);
+#else
+      D.map[c] += dep;
+      D.cnt[c] += 1;
+#endif
+    }
+  }
+  if (fate >= 0) {
+    D.sum[fate] += ff;
+    D.n[fate] += 1;
+  }
 }
 
 // post-step handling shared by the strict and the fast constant step

@@ -560,6 +560,51 @@ class Engine:
         """Release the cube's device memory."""
         self._check(self.lib.nx_cube_end(self.ctx), 'nx_cube_end')
 
+    # bucket order of nx_deposit_fetch (nx_deposit_bucket)
+    DEPOSIT_BUCKETS = ('surface', 'moon', 'escaped', 'vanished', 'remaining', 'source')
+
+    def deposit_begin(self, nlon, nlat):
+        """Allocate and zero the context-owned deposition sink: an (nlon, nlat) map of f64
+        sums and int64 counts plus the bucket sums and counts, until ``deposit_end``."""
+        self._check(self.lib.nx_deposit_begin(self.ctx, int(nlon), int(nlat)), 'nx_deposit_begin')
+
+    def integrate_adaptive_deposit(self, seed, first_id=0, n=None):
+        """K2 on the resident packets through its deposition sink: the run
+        ``integrate_adaptive`` (perfect sticking) or ``integrate_adaptive_bounce`` (deviates
+        keyed by (seed, first_id + packet index)) would make, its events added to the sink.
+        Returns (attempted, accepted, bounces)."""
+        att, acc, bnc = C.c_ulonglong(), C.c_ulonglong(), C.c_ulonglong()
+        n = self.n if n is None else n
+        self._check(self.lib.nx_integrate_adaptive_deposit(self.ctx, int(n), int(seed),
+                                                           int(first_id), C.byref(att),
+                                                           C.byref(acc), C.byref(bnc)),
+                    'nx_integrate_adaptive_deposit')
+        return int(att.value), int(acc.value), int(bnc.value)
+
+    def deposit_fetch(self, nlon, nlat):
+        """(map, counts, buckets, bucket_counts): (nlon, nlat) float64 and int64, then the
+        six buckets in ``DEPOSIT_BUCKETS`` order, float64 and int64."""
+        shape = (int(nlon), int(nlat))
+        dmap = np.zeros(shape)
+        cnt = np.zeros(shape, dtype=np.int64)
+        buckets = np.zeros(len(self.DEPOSIT_BUCKETS))
+        bcnt = np.zeros(len(self.DEPOSIT_BUCKETS), dtype=np.int64)
+        self._check(self.lib.nx_deposit_fetch(self.ctx, dptr(dmap), cnt.ctypes.data_as(_lib.c_i64_p),
+                                              dptr(buckets), bcnt.ctypes.data_as(_lib.c_i64_p)),
+                    'nx_deposit_fetch')
+        return dmap, cnt, buckets, bcnt
+
+    def deposit_allreduce(self, comm, total):
+        """Sum the deposition sink over the ranks of ``comm`` in place, with one scalar riding
+        along; returns the summed scalar."""
+        v = C.c_double(float(total))
+        self._check(self.lib.nx_deposit_allreduce(self.ctx, comm, C.byref(v)), 'nx_deposit_allreduce')
+        return v.value
+
+    def deposit_end(self):
+        """Release the deposition sink's device memory."""
+        self._check(self.lib.nx_deposit_end(self.ctx), 'nx_deposit_end')
+
     def density_accumulate(self, points, radius, s1, s2, count, n=None):
         """K7 of the bound packet table (or the slab): ADDS to ``s1`` (sum of frac), ``s2``
         (sum of frac**2) and ``count`` (member rows) of every ball.  ``points``: (npts, 3) in
