@@ -221,6 +221,25 @@ int nx_integrate_adaptive_bounce(nx_ctx* ctx, long long n, uint64_t seed, uint64
                                  unsigned long long* accepted_steps,
                                  unsigned long long* bounces);
 
+/* ---- context-owned accumulators (image, cube, deposition) ----------------------------------
+ * Each product below sums on the device into its own accumulator of `nsum` f64 sums and
+ * `ncount` i64 counts (the product states the shape), so one product's calls leave the others
+ * alone.  Its begin validates the shape and zeroes the accumulator (the device block is reused
+ * when large enough); its add sums into it, any number of times.  nx_product_fetch copies sums
+ * and counts to the host (either may be NULL; page-locked destinations from nx_host_alloc get
+ * the DMA directly, the driver stages pageable ones) and waits.  nx_product_device_ptrs returns
+ * the device buffers (fused K3 image, NCCL).  nx_product_allreduce sums them over the ranks of
+ * `comm` in place on the context's stream, the one collective of a sharded product; a non-NULL
+ * *total (e.g. ModelImage's totalsource) rides along: this rank's share on entry, the sum on
+ * return (the call then waits).  nx_product_end waits for the stream and frees the block.
+ * Before begin, or after end, each returns -1 with "<product> begin not called".  None of them
+ * drops the candidate pairs nx_los_used_fill reads.                                          */
+typedef enum { NX_PRODUCT_IMAGE = 0, NX_PRODUCT_CUBE = 1, NX_PRODUCT_DEPOSIT = 2 } nx_product;
+int nx_product_fetch(nx_ctx* ctx, nx_product which, double* sums, long long* counts);
+int nx_product_device_ptrs(nx_ctx* ctx, nx_product which, void** sums, void** counts);
+int nx_product_allreduce(nx_ctx* ctx, nx_product which, nx_comm* comm, double* total);
+int nx_product_end(nx_ctx* ctx, nx_product which);
+
 /* ---- K2d: surface deposition maps and the source's loss budget (ModelDeposition) ----------
  * An extension (the reference records neither).  nx_integrate_adaptive_deposit runs the
  * adaptive driver on the resident packets exactly as nx_integrate_adaptive (perfect sticking)
@@ -238,14 +257,10 @@ int nx_integrate_adaptive_bounce(nx_ctx* ctx, long long n, uint64_t seed, uint64
  *   REMAINING  the frac of packets that retire alive (time <= resolution or the attempt cap)
  *              or are passed through without integration
  *   SOURCE     the initial frac > 0 of the packets handed to the kernel
- * Each bucket and map cell holds an f64 sum and an event count.  The frac lost in flight
- * (photo-ionisation, lifetime) is SOURCE minus the other buckets.
- * begin validates nlon, nlat >= 1 (nlon * nlat < 2^31) and allocates and zeroes the sink;
- * fetch copies map / counts (nlon * nlat) and buckets / bucket_counts (NX_DEP_NBUCKET, in
- * nx_deposit_bucket order), any of them may be NULL; allreduce sums the sink over the ranks of
- * `comm` in place, *total riding along (as nx_cube_allreduce_total; NULL: none); end
- * releases it.  Images, cubes and the line-of-sight buffers are not
- * touched.                                                                                   */
+ * The frac lost in flight (photo-ionisation, lifetime) is SOURCE minus the other buckets.
+ * The sink is the NX_PRODUCT_DEPOSIT accumulator, nsum = ncount = nlon * nlat + NX_DEP_NBUCKET:
+ * the map cells, then the buckets in nx_deposit_bucket order, each an f64 sum and an event
+ * count.  begin validates nlon, nlat >= 1 (nlon * nlat < 2^31).                              */
 typedef enum {
   NX_DEP_SURFACE = 0,
   NX_DEP_MOON = 1,
@@ -260,10 +275,6 @@ int nx_integrate_adaptive_deposit(nx_ctx* ctx, long long n, uint64_t seed, uint6
                                   unsigned long long* attempted_steps,
                                   unsigned long long* accepted_steps,
                                   unsigned long long* bounces);
-int nx_deposit_fetch(nx_ctx* ctx, double* map, long long* counts, double* buckets,
-                     long long* bucket_counts);
-int nx_deposit_allreduce(nx_ctx* ctx, nx_comm* comm, double* total);
-int nx_deposit_end(nx_ctx* ctx);
 
 /* ---- K3: constant-step driver with bounce (Output.py:368-455, bouncepackets.py)
  * Optional fused per-step image accumulation (image_dev / counts_dev device
@@ -288,14 +299,11 @@ int nx_image_accumulate(nx_ctx* ctx, long long n, const nx_image_params* ip,
                         double* image /* nx*nz */, long long* counts /* nx*nz */);
 int nx_image_accumulate_dev(nx_ctx* ctx, long long n, const nx_image_params* ip,
                             void* image_dev, void* counts_dev);
-/* The same through an image the CONTEXT owns: begin allocates / zeroes nx * nz pixels, every
- * add bins the bound packet table (or the slab) into it -- ModelImage sums its output files
- * this way (ModelImage.py:92-99) --, fetch copies image f64 / counts i64 to the host (either
- * may be NULL).  nx_image_device_ptrs exposes the buffers (fused K3 image, NCCL).          */
+/* The same into the NX_PRODUCT_IMAGE accumulator, nsum = ncount = nx * nz (row-major (nx, nz)):
+ * every add bins the bound packet table (or the slab) into it -- ModelImage sums its output
+ * files this way (ModelImage.py:92-99).  ModelImage never ends it, so its block only grows. */
 int nx_image_begin(nx_ctx* ctx, int nx, int nz);
 int nx_image_add(nx_ctx* ctx, long long n, const nx_image_params* ip);
-int nx_image_fetch(nx_ctx* ctx, double* image, long long* counts);
-int nx_image_device_ptrs(nx_ctx* ctx, void** image_dev, void** counts_dev);
 /* What ModelImage keeps (ModelImage.py:92-105): image * scale (scale = atoms_per_packet) and the
  * packet image as float64, converted on the device, one copy.  Destinations obtained from
  * nx_host_alloc (page-locked) receive the DMA directly, pageable ones are staged.            */
@@ -304,13 +312,6 @@ int nx_image_fetch_scaled(nx_ctx* ctx, double scale, double* image, double* coun
  * are NumPy arrays; these let the device write them without a staging copy).                  */
 int nx_host_alloc(long long bytes, void** out);
 int nx_host_free(void* p);
-/* Sharded runs: sum the context-owned image + counts over the ranks of `comm` (see nx_comm_create
- * below), in place, on the context's stream -- the single all-reduce of an image product.    */
-int nx_image_allreduce(nx_ctx* ctx, nx_comm* comm);
-/* The same with one scalar riding along (ModelImage's totalsource, ModelImage.py:92-99 sums it
- * over the output files; here also over the ranks): *total is this rank's
- * contribution on entry, the sum over the ranks on return.                                  */
-int nx_image_allreduce_total(nx_ctx* ctx, nx_comm* comm, double* total);
 
 /* ---- K5: lines of sight (compute_iteration.py:151-222) ------------------------
  * los[6*nlos] SoA: x,y,z,xbore,ybore,zbore; dist_from_plan[nlos] as computed at
@@ -371,19 +372,13 @@ int nx_los_spectrum(nx_ctx* ctx, long long n, long long nlos, const double* los,
  * ip->round_f32.  Columns as nx_los_spectrum: 0 = v < vmin, 1..nbins = np.histogram on
  * linspace(vmin, vmax, nbins + 1), nbins + 1 = v > vmax (NaN included).  Layout row-major
  * (nx, nz, nbins + 2), so the sum over the last axis is K4's image and counts.
- * begin allocates and zeroes the context-owned cube (f64 sums + i64 counts, 16 B per cell;
- * nx * nz * (nbins + 2) < 2^31), add bins the bound packet table (or the slab) into it (any
- * number of tables; checks dims, the velocity axis, g-tables for radiance and n before any
- * launch), fetch copies the raw sums and counts to the host (either may be NULL; page-locked
- * destinations receive the DMA directly), allreduce_total is the one collective of a sharded
- * cube (*total rides along, as nx_image_allreduce_total), end releases the device buffers.
- * None of these touch the image scratch or the candidate pairs nx_los_used_fill reads.      */
+ * The cube is the NX_PRODUCT_CUBE accumulator, nsum = ncount = nx * nz * (nbins + 2) < 2^31
+ * (16 B per cell; nx_product_end releases it).  add bins the bound packet table (or the slab)
+ * into it (any number of tables; checks dims, the velocity axis, g-tables for radiance and n
+ * before any launch).                                                                      */
 int nx_cube_begin(nx_ctx* ctx, int nx, int nz, int nbins);
 int nx_cube_add(nx_ctx* ctx, long long n, const nx_image_params* ip,
                 const nx_spectrum_params* sp);
-int nx_cube_fetch(nx_ctx* ctx, double* cube, long long* counts);
-int nx_cube_allreduce_total(nx_ctx* ctx, nx_comm* comm, double* total);
-int nx_cube_end(nx_ctx* ctx);
 
 /* ---- K7: number density at sample points (ModelDensity) ------------------------
  * Over the rows of the bound packet table (or the slab), float32-rounded, frac == 0 rows

@@ -37,6 +37,7 @@ from .engine import get_engine
 from .LOSResult import dist_from_planet_cut
 from .ModelResult import ModelResult
 from .runsetup import get_setup
+from .sharding import combine_ranks, local_device
 from ._lib import LosParams
 from .units import Quantity, value_of
 
@@ -66,15 +67,6 @@ def velocity_bins(velocity, nspec):
     return vmin, vmax, nbins
 
 
-def combine_ranks(spectrum, counts, totalsource, npackets):
-    """Sum the per-rank sums of a sharded run: ONE all-reduce (no-op for a single process).
-    Updates the arrays in place; returns (totalsource, npackets)."""
-    from .sharding import allreduce_sum
-    tot = np.array([float(totalsource), float(npackets)])
-    allreduce_sum(spectrum, counts, tot)
-    return float(tot[0]), int(round(tot[1]))
-
-
 class LOSSpectrum(ModelResult):
     def __init__(self, scdata, inputs, velocity, params=None, dphi=Quantity(1., 'deg'),
                  device=None):
@@ -86,7 +78,6 @@ class LOSSpectrum(ModelResult):
         vmin, vmax, nbins = velocity_bins(velocity, nspec)
         scdata.set_frame('Model')
         super().__init__(inputs, params)
-        from .sharding import local_device
         self.type = 'LineOfSightSpectrum'
         self.species = scdata.species
         self.query = scdata.query
@@ -133,7 +124,8 @@ class LOSSpectrum(ModelResult):
                     cnt += c_
             totalsource += output.totalsource
             npackets += output.npackets
-        self.totalsource, npackets = combine_ranks(spec, cnt, totalsource, npackets)
+        self.totalsource, npackets = combine_ranks((spec, cnt), totalsource, npackets)
+        npackets = int(round(npackets))
 
         endtime = float(value_of(self.inputs.options.endtime))
         self.atoms_per_packet = (1e23 / (self.totalsource / endtime) if self.totalsource > 0

@@ -23,6 +23,7 @@ import pandas as pd
 from . import catalogue
 from .engine import get_engine
 from .ModelResult import ModelResult
+from .sharding import combine_ranks, local_device
 from .units import Quantity, value_of
 
 
@@ -68,15 +69,6 @@ def sample_points(points, radius):
     return pts, np.ascontiguousarray(rad), index
 
 
-def combine_ranks(s1, s2, count, totalsource):
-    """Sum the per-rank sums of a sharded run: ONE all-reduce (no-op for a single process).
-    Updates the arrays in place; returns the total source."""
-    from .sharding import allreduce_sum
-    tot = np.array([float(totalsource)])
-    allreduce_sum(s1, s2, count, tot)
-    return float(tot[0])
-
-
 class ModelDensity(ModelResult):
     def __init__(self, inputs, points, radius, params=None, device=None):
         pts, rad, index = sample_points(points, radius)
@@ -86,7 +78,6 @@ class ModelDensity(ModelResult):
             raise ValueError("ModelDensity computes quantity = 'density'")
         params = dict(params, quantity='density')
         super().__init__(inputs, params)
-        from .sharding import local_device
         self.type = 'density'
         self._device = local_device() if device is None else device
         self.points = pd.DataFrame(pts, columns=['x', 'y', 'z'], index=index)
@@ -113,7 +104,7 @@ class ModelDensity(ModelResult):
                         eng.bind_packets(None)
             totalsource += output.totalsource
             npackets += output.npackets
-        self.totalsource = combine_ranks(s1, s2, count, totalsource)
+        self.totalsource, = combine_ranks((s1, s2, count), totalsource)
         self.npackets_total = npackets
 
         endtime = float(value_of(self.inputs.options.endtime))

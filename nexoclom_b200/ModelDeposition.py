@@ -40,6 +40,7 @@ import pandas as pd
 from . import catalogue
 from .engine import Engine, get_engine
 from .runsetup import get_setup
+from .sharding import combine_ranks, local_device, nccl_comm
 from .units import Quantity, value_of
 
 BUCKETS = Engine.DEPOSIT_BUCKETS                    # nx_deposit_bucket order
@@ -86,19 +87,8 @@ def regeneration(output):
     return 'seed', seed
 
 
-def combine_ranks(dmap, cnt, sums, counts, totalsource):
-    """Sum the per-rank sinks of a sharded run held on the host (torch.distributed's gloo
-    backend): ONE all-reduce, a no-op for a single process.  Updates the arrays in place;
-    returns the summed totalsource."""
-    from .sharding import allreduce_sum
-    tot = np.array([float(totalsource)])
-    allreduce_sum(dmap, cnt, sums, counts, tot)
-    return float(tot[0])
-
-
 class ModelDeposition:
     def __init__(self, inputs, params=None, device=None):
-        from .sharding import local_device, nccl_comm
         params = {} if params is None else params
         if not isinstance(params, dict):
             raise ValueError('params must be a dict')
@@ -148,7 +138,7 @@ class ModelDeposition:
             finally:
                 eng.deposit_end()
         if comm is None:
-            totalsource = combine_ranks(dmap, cnt, sums, counts, totalsource)
+            totalsource, = combine_ranks((dmap, cnt, sums, counts), totalsource)
         self._finish(dmap, cnt, sums, counts, totalsource)
 
     def _run(self, eng, output, kind, what):

@@ -58,7 +58,7 @@ class _Hist2d:
 
 class ModelImage(ModelResult):
     def __init__(self, inputs, params, overwrite=False, distribute=None, device=None):
-        from .sharding import allreduce_sum, nccl_comm
+        from .sharding import allreduce_sum, combine_ranks, nccl_comm
         super().__init__(inputs, params)
         self.type = 'image'
         self._image_geometry(inputs, device)
@@ -82,9 +82,7 @@ class ModelImage(ModelResult):
         if comm is not None:                       # (totalsource rides with the image)
             self.totalsource = eng.image_allreduce_total(comm[1], float(self.totalsource))
         else:
-            tot = np.array([float(self.totalsource)])
-            allreduce_sum(tot)
-            self.totalsource = float(tot[0])
+            self.totalsource, = combine_ranks((), self.totalsource)
 
         mod_rate = self.totalsource / self.inputs.options.endtime.value
         self.atoms_per_packet = 1e23 / mod_rate

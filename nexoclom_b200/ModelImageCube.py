@@ -33,6 +33,7 @@ from .LOSSpectrum import velocity_bins
 from .ModelImage import ModelImage
 from .ModelResult import ModelResult
 from .runsetup import get_setup
+from .sharding import combine_ranks, nccl_comm
 from .units import Quantity
 
 MAX_CELLS = 2**31          # nx * nz * (nbins + 2) must stay below (32-bit cell index)
@@ -51,19 +52,8 @@ def cube_bins(velocity, dims):
     return vmin, vmax, nbins
 
 
-def combine_ranks(sums, counts, totalsource):
-    """Sum the per-rank cubes of a sharded run held on the host (torch.distributed's gloo
-    backend): ONE all-reduce, a no-op for a single process.  Updates the arrays in place;
-    returns the summed totalsource."""
-    from .sharding import allreduce_sum
-    tot = np.array([float(totalsource)])
-    allreduce_sum(sums, counts, tot)
-    return float(tot[0])
-
-
 class ModelImageCube(ModelImage):
     def __init__(self, inputs, params, velocity, device=None):
-        from .sharding import nccl_comm
         if not isinstance(params, dict):
             raise ValueError('params must be a dict')
         if params.get('quantity', None) not in ('column', 'radiance'):
@@ -96,7 +86,7 @@ class ModelImageCube(ModelImage):
             finally:
                 eng.cube_end()
         if comm is None:
-            totalsource = combine_ranks(sums, counts, totalsource)
+            totalsource, = combine_ranks((sums, counts), totalsource)
         self.totalsource = totalsource
 
         endtime = float(self.inputs.options.endtime.value)

@@ -17,6 +17,9 @@ c_i64_p = C.POINTER(C.c_longlong)
 c_u32_p = C.POINTER(C.c_uint32)
 c_u8_p = C.POINTER(C.c_uint8)
 
+# nx_product: the context-owned accumulators
+NX_PRODUCT_IMAGE, NX_PRODUCT_CUBE, NX_PRODUCT_DEPOSIT = 0, 1, 2
+
 
 class RunParams(C.Structure):
     """Mirror of ``nx_run_params`` (include/nexoclom_b200.h)."""
@@ -146,13 +149,9 @@ def load():
         'nx_image_accumulate_dev': [vp, i64, C.POINTER(ImageParams), vp, vp],
         'nx_image_begin': [vp, C.c_int, C.c_int],
         'nx_image_add': [vp, i64, C.POINTER(ImageParams)],
-        'nx_image_fetch': [vp, c_double_p, c_i64_p],
-        'nx_image_device_ptrs': [vp, C.POINTER(vp), C.POINTER(vp)],
         'nx_image_fetch_scaled': [vp, C.c_double, c_double_p, c_double_p],
         'nx_host_alloc': [i64, C.POINTER(vp)],
         'nx_host_free': [vp],
-        'nx_image_allreduce': [vp, vp],
-        'nx_image_allreduce_total': [vp, vp, C.POINTER(C.c_double)],
         'nx_los_accumulate': [vp, i64, i64, c_double_p, c_double_p, C.POINTER(LosParams),
                               c_double_p, c_i64_p, c_u8_p],
         'nx_los_accumulate_dev': [vp, i64, i64, vp, vp, C.POINTER(LosParams), vp, vp, vp],
@@ -166,15 +165,13 @@ def load():
                             C.POINTER(SpectrumParams), c_double_p, c_i64_p],
         'nx_cube_begin': [vp, C.c_int, C.c_int, C.c_int],
         'nx_cube_add': [vp, i64, C.POINTER(ImageParams), C.POINTER(SpectrumParams)],
-        'nx_cube_fetch': [vp, c_double_p, c_i64_p],
-        'nx_cube_allreduce_total': [vp, vp, C.POINTER(C.c_double)],
-        'nx_cube_end': [vp],
         'nx_deposit_begin': [vp, C.c_int, C.c_int],
         'nx_integrate_adaptive_deposit': [vp, i64, u64, u64, C.POINTER(u64), C.POINTER(u64),
                                           C.POINTER(u64)],
-        'nx_deposit_fetch': [vp, c_double_p, c_i64_p, c_double_p, c_i64_p],
-        'nx_deposit_allreduce': [vp, vp, C.POINTER(C.c_double)],
-        'nx_deposit_end': [vp],
+        'nx_product_fetch': [vp, C.c_int, c_double_p, c_i64_p],
+        'nx_product_device_ptrs': [vp, C.c_int, C.POINTER(vp), C.POINTER(vp)],
+        'nx_product_allreduce': [vp, C.c_int, vp, C.POINTER(C.c_double)],
+        'nx_product_end': [vp, C.c_int],
         'nx_density_accumulate': [vp, i64, i64, c_double_p, c_double_p, c_double_p, c_double_p,
                                   C.POINTER(u64)],
         'nx_source_map': [vp, i64, C.POINTER(SourceMapParams)] + [c_double_p] * 9 +

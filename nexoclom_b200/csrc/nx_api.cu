@@ -85,6 +85,22 @@ static void free_packets(nx_packets* h, cudaStream_t st) {
   delete h;
 }
 
+// The context-owned accumulator of one product (nx_product): one device block of `nsum` f64
+// sums, one f64 slot after them that carries a scalar through nx_product_allreduce, then, from
+// the next 256-byte boundary, `ncount` u64 counts.  begin reuses a block that is large enough;
+// nx_product_end frees it.  nsum == 0: begin has not been called since the last end.
+struct Accum {
+  void* block = nullptr;
+  size_t cap = 0;                    // bytes of `block`
+  long long nsum = 0, ncount = 0;
+  int dims[3] = {};                  // begin's shape: image nx, nz; cube nx, nz, nbins; nlon, nlat
+  static size_t count_offset(long long nsum) { return ((size_t)(nsum + 1) * 8 + 255) / 256 * 256; }
+  double* sums() const { return static_cast<double*>(block); }
+  unsigned long long* counts() const {
+    return reinterpret_cast<unsigned long long*>(static_cast<char*>(block) + count_offset(nsum));
+  }
+};
+
 struct nx_ctx {
   int device = 0;
   cudaStream_t stream = nullptr;
@@ -119,16 +135,7 @@ struct nx_ctx {
   // cudaFree (an implicit device synchronisation each) on the calls LOSResult / ModelImage
   // make once per output file, and nothing to leak on an error path
   struct Scratch { void* p = nullptr; size_t bytes = 0; } scr[32];
-  int img_nx = 0, img_nz = 0;  // shape of the context-owned image scratch (nx_image_begin)
-  // context-owned image cube (nx_cube_begin .. nx_cube_end): ncell + 1 f64 sums (the last
-  // slot rides with the all-reduce), then ncell u64 counts, one allocation freed by end
-  int cube_nx = 0, cube_nz = 0, cube_nbins = 0;
-  double* cube = nullptr;
-  // context-owned deposition sink (nx_deposit_begin .. nx_deposit_end), one allocation: ncell
-  // f64 map sums, NX_DEP_NBUCKET f64 bucket sums, one f64 slot that rides with the all-reduce,
-  // then ncell u64 cell counts, NX_DEP_NBUCKET u64 bucket counts and one unused slot
-  int dep_nlon = 0, dep_nlat = 0;
-  double* dep = nullptr;
+  Accum accum[NX_PRODUCT_DEPOSIT + 1];   // one per nx_product
   void* pinned = nullptr;      // grow-only pinned staging for small D2H results (image, LOS columns)
   size_t pinned_bytes = 0;
   unsigned* cmp_tiles = nullptr;     // compaction scratch (tile counts)
@@ -275,7 +282,7 @@ static int alloc_los_work(nx_ctx* ctx, long long n) {
   return 0;
 }
 
-enum { SCR_IMG, SCR_CNT, SCR_LOS, SCR_DIST, SCR_RAD, SCR_NP, SCR_INC, SCR_NBALL, SCR_LADDER,
+enum { SCR_LOS, SCR_DIST, SCR_RAD, SCR_NP, SCR_INC, SCR_NBALL, SCR_LADDER,
        SCR_WID2, SCR_ORDER, SCR_NUSED, SCR_CURSOR, SCR_OFF, SCR_IDX, SCR_SM_IN, SCR_SM_PTS,
        SCR_SM_OUT, SCR_SM_CNT, SCR_TMP, SCR_IMG_OUT, SCR_DD, SCR_KEY, SCR_DENS_IN, SCR_DENS_OUT,
        SCR_DENS_IDX, SCR_SPEC, SCR_NSLOTS };
@@ -307,6 +314,96 @@ static int pinned_staging(nx_ctx* ctx, size_t bytes) {
   ctx->pinned = nullptr; ctx->pinned_bytes = 0;
   CK(cudaHostAlloc(&ctx->pinned, bytes, cudaHostAllocDefault));
   ctx->pinned_bytes = bytes;
+  return 0;
+}
+
+// ---- context-owned accumulators (image, cube, deposition) -----------------------------------
+// None of these calls ENTER: nothing here changes what the line-of-sight kernels read, so the
+// candidate pairs nx_los_accumulate_counted keeps stay valid.
+static const char* const accum_begin_name[] = {"nx_image_begin", "nx_cube_begin",
+                                               "nx_deposit_begin"};
+
+// The accumulator of `which` when its begin has run; else NULL with the error set.
+static Accum* accum_of(nx_ctx* ctx, int which) {
+  if (which < NX_PRODUCT_IMAGE || which > NX_PRODUCT_DEPOSIT) {
+    ctx->err = "unknown nx_product";
+    return nullptr;
+  }
+  Accum& a = ctx->accum[which];
+  if (!a.nsum) {
+    ctx->err = std::string(accum_begin_name[which]) + " not called";
+    return nullptr;
+  }
+  return &a;
+}
+
+// The common half of a begin, after the product has validated its shape: a zeroed block of
+// nsum sums, the slot and ncount counts.
+static int accum_begin(nx_ctx* ctx, nx_product which, long long nsum, long long ncount, int d0,
+                       int d1, int d2) {
+  Accum& a = ctx->accum[which];
+  const size_t bytes = Accum::count_offset(nsum) + (size_t)ncount * 8;
+  if (bytes > a.cap) {
+    void* old = a.block;
+    a = Accum{};
+    CK(cudaFree(old));
+    CK(dev_malloc(&a.block, bytes));
+    a.cap = bytes;
+  }
+  a.nsum = nsum; a.ncount = ncount;
+  a.dims[0] = d0; a.dims[1] = d1; a.dims[2] = d2;
+  CK(cudaMemsetAsync(a.block, 0, bytes, ctx->stream));
+  return 0;
+}
+
+int nx_product_fetch(nx_ctx* ctx, nx_product which, double* sums, long long* counts) {
+  CK(cudaSetDevice(ctx->device));
+  const Accum* a = accum_of(ctx, which);
+  if (!a) return -1;
+  // page-locked destinations (nx_host_alloc) get the DMA directly; pageable ones are staged by
+  // the driver (a pinned staging buffer of the context, grow-only, would outlive a cube)
+  if (sums) CK(cudaMemcpyAsync(sums, a->sums(), a->nsum * 8, cudaMemcpyDeviceToHost, ctx->stream));
+  if (counts)
+    CK(cudaMemcpyAsync(counts, a->counts(), a->ncount * 8, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  return 0;
+}
+
+int nx_product_device_ptrs(nx_ctx* ctx, nx_product which, void** sums, void** counts) {
+  const Accum* a = accum_of(ctx, which);
+  if (!a) return -1;
+  if (sums) *sums = a->sums();
+  if (counts) *counts = a->counts();
+  return 0;
+}
+
+// The one collective of a product (SURVEY section 8e), in place on the context's stream.  With
+// a total it rides in the slot after the sums and is read back (the call then waits for the
+// stream); without one nothing waits.
+int nx_product_allreduce(nx_ctx* ctx, nx_product which, nx_comm* comm, double* total) {
+  CK(cudaSetDevice(ctx->device));
+  Accum* a = accum_of(ctx, which);
+  if (!a) return -1;
+  double* slot = a->sums() + a->nsum;
+  if (total) CK(cudaMemcpyAsync(slot, total, sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+  int r = nx_allreduce(comm, a->sums(), a->nsum + (total ? 1 : 0), NX_DTYPE_F64, ctx->stream);
+  if (r == 0) r = nx_allreduce(comm, a->counts(), a->ncount, NX_DTYPE_I64, ctx->stream);
+  if (r) { ctx->err = std::string("nx_product_allreduce: ") + nx_comm_last_error(); return r; }
+  if (total) {
+    CK(cudaMemcpyAsync(total, slot, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+  }
+  return 0;
+}
+
+int nx_product_end(nx_ctx* ctx, nx_product which) {
+  CK(cudaSetDevice(ctx->device));
+  Accum* a = accum_of(ctx, which);
+  if (!a) return -1;
+  CK(cudaStreamSynchronize(ctx->stream));
+  void* block = a->block;
+  *a = Accum{};
+  CK(cudaFree(block));
   return 0;
 }
 
@@ -421,8 +518,7 @@ int nx_ctx_destroy(nx_ctx* ctx) {
   cudaFree(ctx->pipe_scalars); cudaFree(ctx->pipe_hist);
   cudaFree(ctx->scalars); cudaFree(ctx->status); cudaFree(ctx->cmp_tiles);
   for (auto& sc : ctx->scr) cudaFree(sc.p);
-  cudaFree(ctx->cube);
-  cudaFree(ctx->dep);
+  for (auto& a : ctx->accum) cudaFree(a.block);
   cudaFree(ctx->squeue); cudaFreeHost(ctx->seq_host);
   if (ctx->pinned) cudaFreeHost(ctx->pinned);
   if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
@@ -926,28 +1022,16 @@ int nx_integrate_adaptive_bounce(nx_ctx* ctx, long long n, uint64_t seed, uint64
 }
 
 // ---- K2d: deposition maps and the loss budget (ModelDeposition) ----------------------------
-// The sink has its own allocation, released by nx_deposit_end.  nx_integrate_adaptive_deposit
-// runs the SINK build of the kernel nx_integrate_adaptive (perfect sticking) or
-// nx_integrate_adaptive_bounce would run, on the resident packets: the same final state and
-// step totals, plus the events added to the sink.
-static long long deposit_cells(const nx_ctx* ctx) { return (long long)ctx->dep_nlon * ctx->dep_nlat; }
-static long long deposit_half(const nx_ctx* ctx) { return deposit_cells(ctx) + NX_DEP_NBUCKET + 1; }
+// The sink is the NX_PRODUCT_DEPOSIT accumulator: the map cells, then the buckets, in the sums
+// and in the counts.
+// nx_integrate_adaptive_deposit runs the SINK build of the kernel nx_integrate_adaptive (perfect
+// sticking) or nx_integrate_adaptive_bounce would run, on the resident packets: the same final
+// state and step totals, plus the events added to the sink.
 static_assert((int)NX_DEP_SURFACE == DEP_SURFACE && (int)NX_DEP_MOON == DEP_MOON &&
                   (int)NX_DEP_ESCAPED == DEP_ESCAPED && (int)NX_DEP_VANISHED == DEP_VANISHED &&
                   (int)NX_DEP_REMAINING == DEP_REMAINING && (int)NX_DEP_SOURCE == DEP_SOURCE &&
                   (int)NX_DEP_NBUCKET == DEP_NBUCKET,
               "nx_deposit_bucket and DepositBucket disagree");
-
-int nx_deposit_end(nx_ctx* ctx) {
-  CK(cudaSetDevice(ctx->device));
-  if (ctx->dep) {
-    CK(cudaStreamSynchronize(ctx->stream));
-    CK(cudaFree(ctx->dep));
-  }
-  ctx->dep = nullptr;
-  ctx->dep_nlon = ctx->dep_nlat = 0;
-  return 0;
-}
 
 int nx_deposit_begin(nx_ctx* ctx, int nlon, int nlat) {
   CK(cudaSetDevice(ctx->device));
@@ -956,22 +1040,16 @@ int nx_deposit_begin(nx_ctx* ctx, int nlon, int nlat) {
     ctx->err = "nx_deposit_begin: nlon * nlat must be < 2^31";
     return -1;
   }
-  const long long half = (long long)nlon * nlat + NX_DEP_NBUCKET + 1;
-  if (!ctx->dep || half != deposit_half(ctx)) {
-    int r = nx_deposit_end(ctx);
-    if (r) return r;
-    CK(dev_malloc(&ctx->dep, (size_t)(2 * half) * sizeof(double)));
-  }
-  ctx->dep_nlon = nlon; ctx->dep_nlat = nlat;
-  CK(cudaMemsetAsync(ctx->dep, 0, (size_t)(2 * half) * sizeof(double), ctx->stream));
-  return 0;
+  const long long n = (long long)nlon * nlat + NX_DEP_NBUCKET;
+  return accum_begin(ctx, NX_PRODUCT_DEPOSIT, n, n, nlon, nlat, 0);
 }
 
 int nx_integrate_adaptive_deposit(nx_ctx* ctx, long long n, uint64_t seed, uint64_t first_id,
                                   unsigned long long* attempted, unsigned long long* accepted,
                                   unsigned long long* bounces) {
   ENTER(ctx);
-  if (!ctx->dep) { ctx->err = "nx_deposit_begin not called"; return -1; }
+  const Accum* sink = accum_of(ctx, NX_PRODUCT_DEPOSIT);
+  if (!sink) return -1;
   if (!ctx->have_params) { ctx->err = "nx_tables_upload not called"; return -1; }
   ctx->bound = nullptr;            // integrators work on the slab
   if (n < 0 || n > ctx->cap) { ctx->err = "n exceeds resident packets"; return -1; }
@@ -984,13 +1062,13 @@ int nx_integrate_adaptive_deposit(nx_ctx* ctx, long long n, uint64_t seed, uint6
   CK(cudaMemsetAsync(ctx->scalars, 0, 8 * sizeof(unsigned long long), ctx->stream));
   int r;
   if (n > 0) {
-    const long long ncell = deposit_cells(ctx), half = deposit_half(ctx);
+    const long long ncell = (long long)sink->dims[0] * sink->dims[1];
     DepositOut d;
-    d.map = ctx->dep;
-    d.bucket = ctx->dep + ncell;
-    d.cnt = reinterpret_cast<unsigned long long*>(ctx->dep + half);
+    d.map = sink->sums();
+    d.bucket = d.map + ncell;
+    d.cnt = sink->counts();
     d.bucket_n = d.cnt + ncell;
-    d.nlon = ctx->dep_nlon; d.nlat = ctx->dep_nlat;
+    d.nlon = sink->dims[0]; d.nlat = sink->dims[1];
     if ((r = begin_timed(ctx))) return r;
     if ((r = adaptive_resident(ctx, n, bounce ? &ctx->spline : nullptr, seed, first_id, &d)))
       return r;
@@ -1004,40 +1082,6 @@ int nx_integrate_adaptive_deposit(nx_ctx* ctx, long long n, uint64_t seed, uint6
   if (accepted) *accepted = h[2];
   if (bounces) *bounces = h[3];
   return r;
-}
-
-int nx_deposit_fetch(nx_ctx* ctx, double* map, long long* counts, double* buckets,
-                     long long* bucket_counts) {
-  CK(cudaSetDevice(ctx->device));
-  if (!ctx->dep) { ctx->err = "nx_deposit_begin not called"; return -1; }
-  const long long ncell = deposit_cells(ctx), half = deposit_half(ctx);
-  const double* d = ctx->dep;
-  if (map) CK(cudaMemcpyAsync(map, d, ncell * 8, cudaMemcpyDeviceToHost, ctx->stream));
-  if (buckets)
-    CK(cudaMemcpyAsync(buckets, d + ncell, NX_DEP_NBUCKET * 8, cudaMemcpyDeviceToHost, ctx->stream));
-  if (counts) CK(cudaMemcpyAsync(counts, d + half, ncell * 8, cudaMemcpyDeviceToHost, ctx->stream));
-  if (bucket_counts)
-    CK(cudaMemcpyAsync(bucket_counts, d + half + ncell, NX_DEP_NBUCKET * 8, cudaMemcpyDeviceToHost,
-                       ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
-  return 0;
-}
-
-// The one collective of a sharded deposition: map, counts and buckets of every rank of `comm`,
-// in place, with *total (if not NULL) riding in the slot after the bucket sums.
-int nx_deposit_allreduce(nx_ctx* ctx, nx_comm* comm, double* total) {
-  CK(cudaSetDevice(ctx->device));
-  if (!ctx->dep) { ctx->err = "nx_deposit_begin not called"; return -1; }
-  const long long half = deposit_half(ctx);
-  double* slot = ctx->dep + half - 1;
-  CK(cudaMemsetAsync(slot, 0, sizeof(double), ctx->stream));
-  if (total) CK(cudaMemcpyAsync(slot, total, sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-  int r = nx_allreduce(comm, ctx->dep, half, NX_DTYPE_F64, ctx->stream);
-  if (r == 0) r = nx_allreduce(comm, ctx->dep + half, half, NX_DTYPE_I64, ctx->stream);
-  if (r) { ctx->err = std::string("nx_deposit_allreduce: ") + nx_comm_last_error(); return r; }
-  if (total) CK(cudaMemcpyAsync(total, slot, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
-  return 0;
 }
 
 // Host-buffer variant of K2 for the end-to-end path.  schedule 1 (default): ONE
@@ -1310,52 +1354,23 @@ int nx_image_accumulate_dev(nx_ctx* ctx, long long n, const nx_image_params* ip_
   return end_timed(ctx, 1);
 }
 
-// Context-owned image scratch: begin (allocate + zero), add (K4 into it, any number of packet
-// tables), fetch (D2H).  ModelImage sums its output files on the device this way.
+// The NX_PRODUCT_IMAGE accumulator: begin (allocate + zero), add (K4 into it, any number of
+// packet tables).  ModelImage sums its output files on the device this way and never ends it,
+// so its block only grows.
 int nx_image_begin(nx_ctx* ctx, int nx_, int nz_) {
   CK(cudaSetDevice(ctx->device));
   if (nx_ < 1 || nz_ < 1) { ctx->err = "nx_image_begin: bad dims"; return -1; }
-  const size_t npix = (size_t)nx_ * nz_;
-  double* d_img = nullptr;
-  unsigned long long* d_cnt = nullptr;
-  SCR(SCR_IMG, d_img, npix + 1);                // [npix]: a scalar that rides with the all-reduce
-  SCR(SCR_CNT, d_cnt, npix);
-  CK(cudaMemsetAsync(d_img, 0, (npix + 1) * sizeof(double), ctx->stream));
-  CK(cudaMemsetAsync(d_cnt, 0, npix * sizeof(unsigned long long), ctx->stream));
-  ctx->img_nx = nx_; ctx->img_nz = nz_;
-  return 0;
-}
-
-int nx_image_device_ptrs(nx_ctx* ctx, void** image_dev, void** counts_dev) {
-  if (!ctx->img_nx) { ctx->err = "nx_image_begin not called"; return -1; }
-  if (image_dev) *image_dev = ctx->scr[SCR_IMG].p;
-  if (counts_dev) *counts_dev = ctx->scr[SCR_CNT].p;
-  return 0;
+  const long long npix = (long long)nx_ * nz_;
+  return accum_begin(ctx, NX_PRODUCT_IMAGE, npix, npix, nx_, nz_, 0);
 }
 
 int nx_image_add(nx_ctx* ctx, long long n, const nx_image_params* ip) {
-  if (!ctx->img_nx || ip->nx != ctx->img_nx || ip->nz != ctx->img_nz) {
+  const Accum& a = ctx->accum[NX_PRODUCT_IMAGE];
+  if (!a.nsum || ip->nx != a.dims[0] || ip->nz != a.dims[1]) {
     ctx->err = "nx_image_add: dims differ from nx_image_begin";
     return -1;
   }
-  return nx_image_accumulate_dev(ctx, n, ip, ctx->scr[SCR_IMG].p, ctx->scr[SCR_CNT].p);
-}
-
-int nx_image_fetch(nx_ctx* ctx, double* image, long long* counts) {
-  CK(cudaSetDevice(ctx->device));
-  if (!ctx->img_nx) { ctx->err = "nx_image_begin not called"; return -1; }
-  const size_t npix = (size_t)ctx->img_nx * ctx->img_nz;
-  // D2H into pinned staging (full PCIe rate), then a host memcpy into the caller's pageable
-  // arrays: about 3x faster than letting the driver stage a pageable copy
-  int r = pinned_staging(ctx, 2 * npix * 8);
-  if (r) return r;
-  char* st = static_cast<char*>(ctx->pinned);
-  if (image) CK(cudaMemcpyAsync(st, ctx->scr[SCR_IMG].p, npix * 8, cudaMemcpyDeviceToHost, ctx->stream));
-  if (counts) CK(cudaMemcpyAsync(st + npix * 8, ctx->scr[SCR_CNT].p, npix * 8, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
-  if (image) std::memcpy(image, st, npix * 8);
-  if (counts) std::memcpy(counts, st + npix * 8, npix * 8);
-  return 0;
+  return nx_image_accumulate_dev(ctx, n, ip, a.sums(), a.counts());
 }
 
 // Page-locked host memory for results the caller wants at full PCIe rate and without a
@@ -1377,14 +1392,14 @@ int nx_host_free(void* p) {
 // receive the DMA directly; pageable ones go through the context's pinned staging buffer.
 int nx_image_fetch_scaled(nx_ctx* ctx, double scale, double* image, double* counts) {
   CK(cudaSetDevice(ctx->device));
-  if (!ctx->img_nx) { ctx->err = "nx_image_begin not called"; return -1; }
+  const Accum* img = accum_of(ctx, NX_PRODUCT_IMAGE);
+  if (!img) return -1;
   if (!image || !counts) { ctx->err = "nx_image_fetch_scaled: null destination"; return -1; }
-  const size_t npix = (size_t)ctx->img_nx * ctx->img_nz;
+  const size_t npix = (size_t)img->nsum;
   double* d_out = nullptr;
   SCR(SCR_IMG_OUT, d_out, 2 * npix);
-  CK(launch_image_finish(ctx->stream, static_cast<const double*>(ctx->scr[SCR_IMG].p),
-                         static_cast<const unsigned long long*>(ctx->scr[SCR_CNT].p), scale,
-                         d_out, d_out + npix, (long long)npix));
+  CK(launch_image_finish(ctx->stream, img->sums(), img->counts(), scale, d_out, d_out + npix,
+                         (long long)npix));
   ctx->launches += 1;
   auto pinned = [](const void* p) {
     cudaPointerAttributes a;
@@ -1407,36 +1422,6 @@ int nx_image_fetch_scaled(nx_ctx* ctx, double scale, double* image, double* coun
   return 0;
 }
 
-// The ONE collective of an image product (SURVEY section 8e): the context-owned image and
-// counts of every rank of `comm` are summed in place, on the context's stream.
-int nx_image_allreduce(nx_ctx* ctx, nx_comm* comm) {
-  CK(cudaSetDevice(ctx->device));
-  if (!ctx->img_nx) { ctx->err = "nx_image_begin not called"; return -1; }
-  const long long npix = (long long)ctx->img_nx * ctx->img_nz;
-  int r = nx_allreduce(comm, ctx->scr[SCR_IMG].p, npix, NX_DTYPE_F64, ctx->stream);
-  if (r == 0) r = nx_allreduce(comm, ctx->scr[SCR_CNT].p, npix, NX_DTYPE_I64, ctx->stream);
-  if (r) ctx->err = std::string("nx_image_allreduce: ") + nx_comm_last_error();
-  return r;
-}
-
-// The same with one scalar riding along (ModelImage's totalsource, ModelImage.py:92-99): *total
-// is this rank's contribution on entry and the sum over the ranks on return -- no second
-// collective for 8 bytes.
-int nx_image_allreduce_total(nx_ctx* ctx, nx_comm* comm, double* total) {
-  CK(cudaSetDevice(ctx->device));
-  if (!ctx->img_nx) { ctx->err = "nx_image_begin not called"; return -1; }
-  if (!total) return nx_image_allreduce(ctx, comm);
-  const long long npix = (long long)ctx->img_nx * ctx->img_nz;
-  double* d_img = static_cast<double*>(ctx->scr[SCR_IMG].p);
-  CK(cudaMemcpyAsync(d_img + npix, total, sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-  int r = nx_allreduce(comm, d_img, npix + 1, NX_DTYPE_F64, ctx->stream);
-  if (r == 0) r = nx_allreduce(comm, ctx->scr[SCR_CNT].p, npix, NX_DTYPE_I64, ctx->stream);
-  if (r) { ctx->err = std::string("nx_image_allreduce_total: ") + nx_comm_last_error(); return r; }
-  CK(cudaMemcpyAsync(total, d_img + npix, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
-  return 0;
-}
-
 int nx_ctx_stream(nx_ctx* ctx, void** cuda_stream) {
   if (!cuda_stream) return -1;
   *cuda_stream = ctx->stream;
@@ -1447,7 +1432,7 @@ int nx_image_accumulate(nx_ctx* ctx, long long n, const nx_image_params* ip, dou
                         long long* counts) {
   int r = nx_image_begin(ctx, ip->nx, ip->nz);
   if (r == 0) r = nx_image_add(ctx, n, ip);
-  if (r == 0) r = nx_image_fetch(ctx, image, counts);
+  if (r == 0) r = nx_product_fetch(ctx, NX_PRODUCT_IMAGE, image, counts);
   return r;
 }
 
@@ -1858,25 +1843,8 @@ int nx_los_spectrum(nx_ctx* ctx, long long n, long long nlos, const double* los,
 }
 
 // ---- Doppler-resolved image cubes (ModelImageCube) -----------------------------------------
-// The cube has its own allocation, released by nx_cube_end: an 800 x 800 x 100 cube is 0.5 GB per
-// plane, too much to keep in grow-only scratch after the product is fetched.  No ENTER: like
-// nx_image_add, nothing here changes what the line-of-sight kernels read, so the candidate
-// pairs nx_los_accumulate_counted keeps stay valid.
-static long long cube_cells(const nx_ctx* ctx) {
-  return (long long)ctx->cube_nx * ctx->cube_nz * (ctx->cube_nbins + 2);
-}
-
-int nx_cube_end(nx_ctx* ctx) {
-  CK(cudaSetDevice(ctx->device));
-  if (ctx->cube) {
-    CK(cudaStreamSynchronize(ctx->stream));
-    CK(cudaFree(ctx->cube));
-  }
-  ctx->cube = nullptr;
-  ctx->cube_nx = ctx->cube_nz = ctx->cube_nbins = 0;
-  return 0;
-}
-
+// The cube is the NX_PRODUCT_CUBE accumulator, released by nx_product_end: an 800 x 800 x 100
+// cube is 0.5 GB per plane, too much to keep after the product is fetched.
 int nx_cube_begin(nx_ctx* ctx, int nx_, int nz_, int nbins) {
   CK(cudaSetDevice(ctx->device));
   if (nx_ < 1 || nz_ < 1 || nbins < 1) { ctx->err = "nx_cube_begin: bad dims"; return -1; }
@@ -1885,25 +1853,19 @@ int nx_cube_begin(nx_ctx* ctx, int nx_, int nz_, int nbins) {
     return -1;
   }
   const long long ncell = (long long)nx_ * nz_ * (nbins + 2);
-  if (!ctx->cube || ncell != cube_cells(ctx)) {
-    int r = nx_cube_end(ctx);
-    if (r) return r;
-    CK(dev_malloc(&ctx->cube, (size_t)(2 * ncell + 1) * sizeof(double)));
-  }
-  ctx->cube_nx = nx_; ctx->cube_nz = nz_; ctx->cube_nbins = nbins;
-  CK(cudaMemsetAsync(ctx->cube, 0, (size_t)(2 * ncell + 1) * sizeof(double), ctx->stream));
-  return 0;
+  return accum_begin(ctx, NX_PRODUCT_CUBE, ncell, ncell, nx_, nz_, nbins);
 }
 
 int nx_cube_add(nx_ctx* ctx, long long n, const nx_image_params* ip_,
                 const nx_spectrum_params* sp_) {
   CK(cudaSetDevice(ctx->device));
-  if (!ctx->cube) { ctx->err = "nx_cube_begin not called"; return -1; }
+  const Accum* cube = accum_of(ctx, NX_PRODUCT_CUBE);
+  if (!cube) return -1;
   if (!ip_ || !sp_) { ctx->err = "nx_cube_add: null argument"; return -1; }
   ImageParams ip;
   std::memcpy(&ip, ip_, sizeof(ip));
   const nx_spectrum_params sp = *sp_;
-  if (ip.nx != ctx->cube_nx || ip.nz != ctx->cube_nz || sp.nbins != ctx->cube_nbins) {
+  if (ip.nx != cube->dims[0] || ip.nz != cube->dims[1] || sp.nbins != cube->dims[2]) {
     ctx->err = "nx_cube_add: dims or nbins differ from nx_cube_begin";
     return -1;
   }
@@ -1924,43 +1886,12 @@ int nx_cube_add(nx_ctx* ctx, long long n, const nx_image_params* ip_,
   ax.step = (sp.vmax - sp.vmin) / sp.nbins;         // np.linspace's step
   ax.vscale = sp.vscale;
   ax.nbins = sp.nbins;
-  const long long ncell = cube_cells(ctx);
   int r;
   if ((r = materialize(ctx))) return r;
   if ((r = begin_timed(ctx))) return r;
   CK(launch_image_cube(ctx->stream, ctx->device, state_cols(ctx), n, ip, ctx->gtables, ax,
-                       ctx->cube, reinterpret_cast<unsigned long long*>(ctx->cube + ncell + 1)));
+                       cube->sums(), cube->counts()));
   return end_timed(ctx, 1);
-}
-
-int nx_cube_fetch(nx_ctx* ctx, double* cube, long long* counts) {
-  CK(cudaSetDevice(ctx->device));
-  if (!ctx->cube) { ctx->err = "nx_cube_begin not called"; return -1; }
-  const size_t bytes = (size_t)cube_cells(ctx) * 8;
-  // page-locked destinations (nx_host_alloc) get the DMA directly; pageable ones are staged by
-  // the driver (a pinned staging buffer of the context, grow-only, would outlive the cube)
-  if (cube) CK(cudaMemcpyAsync(cube, ctx->cube, bytes, cudaMemcpyDeviceToHost, ctx->stream));
-  if (counts)
-    CK(cudaMemcpyAsync(counts, ctx->cube + cube_cells(ctx) + 1, bytes, cudaMemcpyDeviceToHost,
-                       ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
-  return 0;
-}
-
-// The one collective of a sharded cube: sums and counts of every rank of `comm`, in place, with
-// *total riding in the slot after the sums (as nx_image_allreduce_total).
-int nx_cube_allreduce_total(nx_ctx* ctx, nx_comm* comm, double* total) {
-  CK(cudaSetDevice(ctx->device));
-  if (!ctx->cube) { ctx->err = "nx_cube_begin not called"; return -1; }
-  if (!total) { ctx->err = "nx_cube_allreduce_total: null total"; return -1; }
-  const long long ncell = cube_cells(ctx);
-  CK(cudaMemcpyAsync(ctx->cube + ncell, total, sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-  int r = nx_allreduce(comm, ctx->cube, ncell + 1, NX_DTYPE_F64, ctx->stream);
-  if (r == 0) r = nx_allreduce(comm, ctx->cube + ncell + 1, ncell, NX_DTYPE_I64, ctx->stream);
-  if (r) { ctx->err = std::string("nx_cube_allreduce_total: ") + nx_comm_last_error(); return r; }
-  CK(cudaMemcpyAsync(total, ctx->cube + ncell, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
-  return 0;
 }
 
 // ---- K7: number density at sample points (ModelDensity) ------------------------------------

@@ -11,7 +11,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import (RunParams, SourceParams, ImageParams, LosParams, SpectrumParams, as_f64,
-                   dptr, c_double_p)
+                   dptr, c_double_p, NX_PRODUCT_IMAGE, NX_PRODUCT_CUBE, NX_PRODUCT_DEPOSIT)
 
 STATE_COLS = ('time', 'x', 'y', 'z', 'vx', 'vy', 'vz', 'frac')
 X0_COLS = ('time', 'x', 'y', 'z', 'vx', 'vy', 'vz', 'frac', 'v', 'longitude', 'latitude',
@@ -379,11 +379,7 @@ class Engine:
                     'nx_image_add')
 
     def image_fetch(self, nx, nz):
-        img = np.empty((nx, nz))
-        cnt = np.empty((nx, nz), dtype=np.int64)
-        self._check(self.lib.nx_image_fetch(self.ctx, dptr(img),
-                                            cnt.ctypes.data_as(_lib.c_i64_p)), 'nx_image_fetch')
-        return img, cnt
+        return self._product_fetch(NX_PRODUCT_IMAGE, (nx, nz))
 
     def image_fetch_scaled(self, nx, nz, scale):
         """(image * scale, packet counts as float64): what ``ModelImage`` keeps
@@ -398,14 +394,11 @@ class Engine:
     def image_allreduce(self, comm):
         """Sum the context-owned image + counts over the ranks of ``comm`` (an ``nx_comm``
         handle), in place on the device: the one collective of an image product."""
-        self._check(self.lib.nx_image_allreduce(self.ctx, comm), 'nx_image_allreduce')
+        self._product_allreduce(NX_PRODUCT_IMAGE, comm)
 
     def image_allreduce_total(self, comm, total):
         """``image_allreduce`` with one scalar riding along; returns the summed scalar."""
-        v = C.c_double(float(total))
-        self._check(self.lib.nx_image_allreduce_total(self.ctx, comm, C.byref(v)),
-                    'nx_image_allreduce_total')
-        return v.value
+        return self._product_allreduce(NX_PRODUCT_IMAGE, comm, total)
 
     def stream_ptr(self):
         p = C.c_void_p()
@@ -414,8 +407,8 @@ class Engine:
 
     def image_device_ptrs(self):
         a, b = C.c_void_p(), C.c_void_p()
-        self._check(self.lib.nx_image_device_ptrs(self.ctx, C.byref(a), C.byref(b)),
-                    'nx_image_device_ptrs')
+        self._check(self.lib.nx_product_device_ptrs(self.ctx, NX_PRODUCT_IMAGE, C.byref(a),
+                                                    C.byref(b)), 'nx_product_device_ptrs')
         return a.value, b.value
 
     def image_accumulate_dev(self, image_params, image_dev, counts_dev, n=None):
@@ -540,27 +533,18 @@ class Engine:
 
     def cube_fetch(self, nx, nz, nbins):
         """(sums, counts), both (nx, nz, nbins + 2), float64 and int64, in page-locked arrays."""
-        pool = _pinned_pool(self.lib)
-        shape = (int(nx), int(nz), int(nbins) + 2)
-        cube = pool.array(shape)
-        cnt = pool.array(shape, dtype=np.int64)
-        self._check(self.lib.nx_cube_fetch(self.ctx, dptr(cube), cnt.ctypes.data_as(_lib.c_i64_p)),
-                    'nx_cube_fetch')
-        return cube, cnt
+        return self._product_fetch(NX_PRODUCT_CUBE, (int(nx), int(nz), int(nbins) + 2))
 
     def cube_allreduce_total(self, comm, total):
         """Sum the cube's sums and counts over the ranks of ``comm`` in place, with one scalar
         riding along; returns the summed scalar."""
-        v = C.c_double(float(total))
-        self._check(self.lib.nx_cube_allreduce_total(self.ctx, comm, C.byref(v)),
-                    'nx_cube_allreduce_total')
-        return v.value
+        return self._product_allreduce(NX_PRODUCT_CUBE, comm, total)
 
     def cube_end(self):
         """Release the cube's device memory."""
-        self._check(self.lib.nx_cube_end(self.ctx), 'nx_cube_end')
+        self._product_end(NX_PRODUCT_CUBE)
 
-    # bucket order of nx_deposit_fetch (nx_deposit_bucket)
+    # bucket order of the deposition sink (nx_deposit_bucket)
     DEPOSIT_BUCKETS = ('surface', 'moon', 'escaped', 'vanished', 'remaining', 'source')
 
     def deposit_begin(self, nlon, nlat):
@@ -584,26 +568,41 @@ class Engine:
     def deposit_fetch(self, nlon, nlat):
         """(map, counts, buckets, bucket_counts): (nlon, nlat) float64 and int64, then the
         six buckets in ``DEPOSIT_BUCKETS`` order, float64 and int64."""
+        ncell = int(nlon) * int(nlat)
+        sums, cnt = self._product_fetch(NX_PRODUCT_DEPOSIT, (ncell + len(self.DEPOSIT_BUCKETS),))
         shape = (int(nlon), int(nlat))
-        dmap = np.zeros(shape)
-        cnt = np.zeros(shape, dtype=np.int64)
-        buckets = np.zeros(len(self.DEPOSIT_BUCKETS))
-        bcnt = np.zeros(len(self.DEPOSIT_BUCKETS), dtype=np.int64)
-        self._check(self.lib.nx_deposit_fetch(self.ctx, dptr(dmap), cnt.ctypes.data_as(_lib.c_i64_p),
-                                              dptr(buckets), bcnt.ctypes.data_as(_lib.c_i64_p)),
-                    'nx_deposit_fetch')
-        return dmap, cnt, buckets, bcnt
+        return sums[:ncell].reshape(shape), cnt[:ncell].reshape(shape), sums[ncell:], cnt[ncell:]
 
     def deposit_allreduce(self, comm, total):
         """Sum the deposition sink over the ranks of ``comm`` in place, with one scalar riding
         along; returns the summed scalar."""
-        v = C.c_double(float(total))
-        self._check(self.lib.nx_deposit_allreduce(self.ctx, comm, C.byref(v)), 'nx_deposit_allreduce')
-        return v.value
+        return self._product_allreduce(NX_PRODUCT_DEPOSIT, comm, total)
 
     def deposit_end(self):
         """Release the deposition sink's device memory."""
-        self._check(self.lib.nx_deposit_end(self.ctx), 'nx_deposit_end')
+        self._product_end(NX_PRODUCT_DEPOSIT)
+
+    # -- context-owned accumulators (nx_product) --------------------------------
+    def _product_fetch(self, which, shape):
+        """(sums, counts) of an accumulator, both ``shape``, float64 and int64, in page-locked
+        arrays (a direct DMA)."""
+        pool = _pinned_pool(self.lib)
+        sums, cnt = pool.array(shape), pool.array(shape, dtype=np.int64)
+        self._check(self.lib.nx_product_fetch(self.ctx, which, dptr(sums),
+                                              cnt.ctypes.data_as(_lib.c_i64_p)), 'nx_product_fetch')
+        return sums, cnt
+
+    def _product_allreduce(self, which, comm, total=None):
+        """The accumulator summed over the ranks of ``comm`` in place; with ``total``, that
+        scalar rides along and the sum over the ranks is returned."""
+        v = None if total is None else C.c_double(float(total))
+        self._check(self.lib.nx_product_allreduce(self.ctx, which, comm,
+                                                  None if v is None else C.byref(v)),
+                    'nx_product_allreduce')
+        return None if v is None else v.value
+
+    def _product_end(self, which):
+        self._check(self.lib.nx_product_end(self.ctx, which), 'nx_product_end')
 
     def density_accumulate(self, points, radius, s1, s2, count, n=None):
         """K7 of the bound packet table (or the slab): ADDS to ``s1`` (sum of frac), ``s2``

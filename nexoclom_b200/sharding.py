@@ -128,6 +128,15 @@ def allreduce_sum(*arrays):
     return arrays
 
 
+def combine_ranks(arrays, *scalars):
+    """Sum a product's host ``arrays`` over the ranks in place, with ``scalars`` (totalsource,
+    ...) riding along in one float64 array: ONE all-reduce, a no-op for a single process.
+    Returns the summed scalars as a tuple of floats."""
+    tot = np.array(scalars, dtype=np.float64)
+    allreduce_sum(*arrays, tot)
+    return tuple(float(v) for v in tot)
+
+
 def nccl_comm():
     """``(lib, nx_comm handle)`` when this process group runs over NCCL, else ``None`` (single
     process, or the gloo backend of the CPU tests)."""

@@ -15,7 +15,8 @@ import torch.distributed as dist
 import torch.multiprocessing as mp
 
 from common import REPO, workload
-from nexoclom_b200.ModelDensity import lens_volume, sample_points, combine_ranks
+from nexoclom_b200.ModelDensity import lens_volume, sample_points
+from nexoclom_b200.sharding import combine_ranks
 from oracle import density as odens
 
 
@@ -155,14 +156,14 @@ def _gloo_worker(rank, world, port, q):
     sys.path.insert(0, os.path.join(REPO, 'tests'))
     os.environ.update(MASTER_ADDR='127.0.0.1', MASTER_PORT=str(port))
     dist.init_process_group('gloo', rank=rank, world_size=world)
-    from nexoclom_b200.ModelDensity import combine_ranks
+    from nexoclom_b200.sharding import combine_ranks
     from nexoclom_b200.sharding import shard_range
     from oracle import density as od
     X, frac = _cloud(30000, 3)
     pts, rad = _gloo_points()
     first, n = shard_range(len(X), rank, world)
     s1, s2, cnt = od.ball_sums_kdtree(X[first:first + n], frac[first:first + n], pts, rad)
-    tot = combine_ranks(s1, s2, cnt, float(n))          # what ModelDensity does per product
+    tot, = combine_ranks((s1, s2, cnt), float(n))       # what ModelDensity does per product
     if rank == 0:
         q.put((s1, s2, cnt, tot))
     dist.barrier()
@@ -193,7 +194,7 @@ def test_two_rank_allreduce_equals_single_rank():
     assert np.allclose(s1, o1, rtol=1e-12, atol=0) and np.allclose(s2, o2, rtol=1e-12, atol=0)
     # a single process: the reduction leaves the sums alone
     a, b, c = o1.copy(), o2.copy(), oc.copy()
-    assert combine_ranks(a, b, c, 5.0) == 5.0 and np.array_equal(a, o1) and np.array_equal(c, oc)
+    assert combine_ranks((a, b, c), 5.0) == (5.0,) and np.array_equal(a, o1) and np.array_equal(c, oc)
 
 
 # ---------------------------------------------------------------------------------------

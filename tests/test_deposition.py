@@ -245,12 +245,12 @@ def _gloo_worker(rank, world, port, q):
                       WORLD_SIZE=str(world))
     dist.init_process_group('gloo', rank=rank, world_size=world)
     try:
-        from nexoclom_b200.ModelDeposition import combine_ranks
+        from nexoclom_b200.sharding import combine_ranks
         dmap = np.full((3, 2), rank + 1.0)
         cnt = np.full((3, 2), rank + 1, np.int64)
         sums = np.arange(6.0) * (rank + 1)
         counts = np.arange(6, dtype=np.int64) * (rank + 1)
-        tot = combine_ranks(dmap, cnt, sums, counts, 10.0 * (rank + 1))
+        tot, = combine_ranks((dmap, cnt, sums, counts), 10.0 * (rank + 1))
         q.put((rank, dmap.tolist(), cnt.tolist(), sums.tolist(), counts.tolist(), tot))
     finally:
         dist.destroy_process_group()

@@ -15,7 +15,8 @@ import torch.distributed as dist
 import torch.multiprocessing as mp
 
 from common import REPO, workload
-from nexoclom_b200.ModelImageCube import cube_bins, combine_ranks
+from nexoclom_b200.ModelImageCube import cube_bins
+from nexoclom_b200.sharding import combine_ranks
 from oracle import cube as ocube
 from oracle import imaging
 from oracle import spectrum as ospec
@@ -151,12 +152,12 @@ def _gloo_worker(rank, world, port, q):
     sys.path.insert(0, os.path.join(REPO, 'tests'))
     os.environ.update(MASTER_ADDR='127.0.0.1', MASTER_PORT=str(port))
     dist.init_process_group('gloo', rank=rank, world_size=world)
-    from nexoclom_b200.ModelImageCube import combine_ranks
+    from nexoclom_b200.sharding import combine_ranks
     from nexoclom_b200.sharding import shard_range
     X = _gloo_cloud()
     first, n = shard_range(len(X), rank, world)
     cube, cnt = _gloo_oracle(X[first:first + n])
-    tot = combine_ranks(cube, cnt, float(n))             # what ModelImageCube does off NCCL
+    tot, = combine_ranks((cube, cnt), float(n))          # what ModelImageCube does off NCCL
     if rank == 0:
         q.put((cube, cnt, tot))
     dist.barrier()
@@ -181,7 +182,7 @@ def test_two_rank_allreduce_equals_single_rank():
     assert np.array_equal(cube > 0, nz)
     assert np.max(np.abs(cube[nz] - ocube_[nz]) / ocube_[nz]) < 1e-12
     a, c = ocube_.copy(), ocnt.copy()                    # a single process: left alone
-    assert combine_ranks(a, c, 5.0) == 5.0 and np.array_equal(a, ocube_)
+    assert combine_ranks((a, c), 5.0) == (5.0,) and np.array_equal(a, ocube_)
 
 
 # ---------------------------------------------------------------------------------------

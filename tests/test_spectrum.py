@@ -16,7 +16,8 @@ import torch.distributed as dist
 import torch.multiprocessing as mp
 
 from common import REPO, workload
-from nexoclom_b200.LOSSpectrum import velocity_bins, combine_ranks
+from nexoclom_b200.LOSSpectrum import velocity_bins
+from nexoclom_b200.sharding import combine_ranks
 from oracle import imaging
 from oracle import spectrum as ospec
 
@@ -219,13 +220,13 @@ def _gloo_worker(rank, world, port, q):
     sys.path.insert(0, os.path.join(REPO, 'tests'))
     os.environ.update(MASTER_ADDR='127.0.0.1', MASTER_PORT=str(port))
     dist.init_process_group('gloo', rank=rank, world_size=world)
-    from nexoclom_b200.LOSSpectrum import combine_ranks
+    from nexoclom_b200.sharding import combine_ranks
     from nexoclom_b200.sharding import shard_range
     X = _gloo_cloud()
     first, n = shard_range(len(X), rank, world)
     spec, cnt = _oracle_spectrum(X[first:first + n], _gloo_lines(), _na_setup(),
                                  np.radians(3.0), -6.0, 6.0, 24)
-    tot = combine_ranks(spec, cnt, float(n), n)          # what LOSSpectrum does per product
+    tot = combine_ranks((spec, cnt), float(n), n)        # what LOSSpectrum does per product
     if rank == 0:
         q.put((spec, cnt, tot))
     dist.barrier()
@@ -251,7 +252,7 @@ def test_two_rank_allreduce_equals_single_rank():
     assert np.array_equal(spec > 0, nz)
     assert np.max(np.abs(spec[nz] - ospec_[nz]) / ospec_[nz]) < 1e-12
     a, c = ospec_.copy(), ocnt.copy()                    # a single process: left alone
-    assert combine_ranks(a, c, 5.0, 5) == (5.0, 5) and np.array_equal(a, ospec_)
+    assert combine_ranks((a, c), 5.0, 5) == (5.0, 5) and np.array_equal(a, ospec_)
 
 
 # ---------------------------------------------------------------------------------------
