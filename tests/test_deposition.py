@@ -8,7 +8,7 @@ import os
 import numpy as np
 import pytest
 
-from common import REPO, workload, oracle_constants
+from common import REPO, KERNEL_CELLS, Cell, workload, oracle_constants
 from nexoclom_b200._lib import dptr
 from nexoclom_b200.runsetup import RunSetup
 from oracle import adaptive_bounce, deposition, initial_state, tracking
@@ -151,14 +151,22 @@ def test_oracle_events_classify_final_state(wl):
     assert (want == deposition.SURFACE).sum() > 0
 
 
-@pytest.mark.parametrize('wl', WORKLOADS)
+# the workloads, and every force x loss x moon cell of the adaptive driver
+@pytest.mark.parametrize('wl', WORKLOADS + [c for c in KERNEL_CELLS if c.driver == 'adaptive'],
+                         ids=str)
 @pytest.mark.parametrize('strict', [1, 0])
 def test_host_build_matches_oracle(hcd, wl, strict):
-    setup = setup_of(wl, strict_math=bool(strict))
-    X0 = initial_state.draw_x0(setup, 300, 21)[:, :8]
+    from test_hostcheck import host_strict
+    if isinstance(wl, Cell):
+        setup = wl.setup(strict_math=bool(strict))
+        X0 = wl.x0(setup, 300, 21)
+    else:
+        setup = setup_of(wl, strict_math=bool(strict))
+        X0 = initial_state.draw_x0(setup, 300, 21)[:, :8]
     seed, first = 5, 1000
     Xo, a_o, c_o, b_o, ev, _ = run_oracle(setup, X0, seed, first)
-    Xh, a_h, c_h, got = run_host(hcd, setup, X0, seed, first, strict)
+    Xh, a_h, c_h, got = run_host(hcd, setup, X0, seed, first,
+                                 host_strict(setup, strict, is_bounce(setup)))
     assert np.array_equal(a_h, a_o) and np.array_equal(c_h, c_o)
     compare_sink(got, ev, NLON, NLAT, exact_cells=False)
     # Sigma map == SURFACE, and the host's own sums add up to its source

@@ -8,7 +8,8 @@ import os
 import numpy as np
 import pytest
 
-from common import REPO, GOLDEN, workload, oracle_constants, state_parity
+from common import (REPO, GOLDEN, KERNEL_CELLS, Cell, adaptive_mode, workload, oracle_constants,
+                    state_parity)
 from nexoclom_b200._lib import RunParams, SourceParams, ImageParams, dptr
 from nexoclom_b200.runsetup import RunSetup
 from nexoclom_b200.units import Quantity
@@ -45,13 +46,27 @@ def run_adaptive(hc, setup, X0, strict):
     return X, att, acc, step
 
 
-@pytest.mark.parametrize('wl', ['Na.maxwellian.radpres.input', 'Ca.isotropic.flat.input'])
+def host_strict(setup, strict, bounce=False):
+    """The host build's flag for the build the device runs: adaptive_attempt_fast_rt has fast
+    builds the dispatchers never select (a moon or bounce without gravity), those runs take the
+    strict build on the device."""
+    return int(bool(strict) or adaptive_mode(setup.params, bounce) < 0)
+
+
+# the workloads, and every force x loss x moon cell of the perfect-sticking adaptive driver
+@pytest.mark.parametrize('wl', ['Na.maxwellian.radpres.input', 'Ca.isotropic.flat.input'] +
+                         [c for c in KERNEL_CELLS if c.driver == 'adaptive' and not c.bounce],
+                         ids=str)
 @pytest.mark.parametrize('strict', [1, 0])
 def test_adaptive_attempt_matches_oracle(hc, wl, strict):
-    setup = RunSetup(workload(wl))
-    X0 = initial_state.draw_x0(setup, 600, 3)[:, :8]
+    if isinstance(wl, Cell):
+        setup = wl.setup()
+        X0 = wl.x0(setup, 600, 3)
+    else:
+        setup = RunSetup(workload(wl))
+        X0 = initial_state.draw_x0(setup, 600, 3)[:, :8]
     Xo, a_o, c_o = tracking.integrate_adaptive(X0, oracle_constants(setup))
-    Xh, a_h, c_h, _ = run_adaptive(hc, setup, X0, strict)
+    Xh, a_h, c_h, _ = run_adaptive(hc, setup, X0, host_strict(setup, strict))
     par = state_parity(Xh, Xo)
     assert par['alive_mismatch'] == 0
     assert np.array_equal(a_h, a_o) and np.array_equal(c_h, c_o)      # same step sequence
@@ -141,18 +156,31 @@ def test_surface_spot_sampling(hc):
     assert abs(np.median(out[:, 10]) + 0.2) < 0.1
 
 
+# the bounce workloads, and every force x loss cell of the constant-step driver with bounce
 @pytest.mark.parametrize('tag, wl', [('tdep', 'Na.bounce.input'),
-                                     ('c05', 'Na.bounce.stick05.input')])
+                                     ('c05', 'Na.bounce.stick05.input')] +
+                         [pytest.param(c.id, c, id=c.id) for c in KERNEL_CELLS
+                          if c.driver == 'constant'])
 def test_constant_step_bounce_matches_oracle(hc, tag, wl):
-    inputs = workload(wl)
-    inputs.options.endtime = Quantity(1500., 's')
-    setup = RunSetup(inputs)
+    n, seed, first = 400, 99, 7
+    if isinstance(wl, Cell):
+        setup = wl.setup()
+        X0 = wl.x0(setup, n, 9)
+    else:
+        inputs = workload(wl)
+        inputs.options.endtime = Quantity(1500., 's')
+        setup = RunSetup(inputs)
+        X0 = initial_state.draw_x0(setup, n, 9)[:, :8]
     rc = oracle_constants(setup)
     p = setup.params
-    n, seed, first = 400, 99, 7
-    X0 = initial_state.draw_x0(setup, n, 9)[:, :8]
-    ref, nsteps, _ = tracking.integrate_constant(
-        X0, rc, uniforms=initial_state.bounce_uniforms(seed, first))
+    hits = []
+    uniforms = initial_state.bounce_uniforms(seed, first)
+
+    def counted(ct, idx):
+        hits.append(len(idx))
+        return uniforms(ct, idx)
+
+    ref, nsteps, _ = tracking.integrate_constant(X0, rc, uniforms=counted)
     tx, ty, c = setup.spline_tck
     prv, pra, nrp, _rv, _ra = _rp(setup)
     for strict in (1, 0):
@@ -164,8 +192,11 @@ def test_constant_step_bounce_matches_oracle(hc, tag, wl):
                                  C.c_int(len(ty)), dptr(c), C.c_int(strict))
         assert np.array_equal(traj[:, 7, :] > 0, ref[:, 7, :] > 0)
         assert np.max(np.abs(traj - ref)) < 1e-10
-    # packets did bounce: some frac values strictly between 0 and 1 without photo-loss alone
-    assert (ref[:, 7, -1] < 0.9).any()
+    # packets did bounce (a force brings them back to the surface)
+    if p.gravity or p.radpres:
+        assert sum(hits) > 0
+    if not isinstance(wl, Cell):
+        assert (ref[:, 7, -1] < 0.9).any()
 
 
 def test_spline_matches_scipy(hc):
