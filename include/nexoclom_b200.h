@@ -221,7 +221,7 @@ int nx_integrate_adaptive_bounce(nx_ctx* ctx, long long n, uint64_t seed, uint64
                                  unsigned long long* accepted_steps,
                                  unsigned long long* bounces);
 
-/* ---- context-owned accumulators (image, cube, deposition) ----------------------------------
+/* ---- context-owned accumulators (image, cube, deposition, ion production) ------------------
  * Each product below sums on the device into its own accumulator of `nsum` f64 sums and
  * `ncount` i64 counts (the product states the shape), so one product's calls leave the others
  * alone.  Its begin validates the shape and zeroes the accumulator (the device block is reused
@@ -234,7 +234,12 @@ int nx_integrate_adaptive_bounce(nx_ctx* ctx, long long n, uint64_t seed, uint64
  * return (the call then waits).  nx_product_end waits for the stream and frees the block.
  * Before begin, or after end, each returns -1 with "<product> begin not called".  None of them
  * drops the candidate pairs nx_los_used_fill reads.                                          */
-typedef enum { NX_PRODUCT_IMAGE = 0, NX_PRODUCT_CUBE = 1, NX_PRODUCT_DEPOSIT = 2 } nx_product;
+typedef enum {
+  NX_PRODUCT_IMAGE = 0,
+  NX_PRODUCT_CUBE = 1,
+  NX_PRODUCT_DEPOSIT = 2,
+  NX_PRODUCT_IONIZE = 3
+} nx_product;
 int nx_product_fetch(nx_ctx* ctx, nx_product which, double* sums, long long* counts);
 int nx_product_device_ptrs(nx_ctx* ctx, nx_product which, void** sums, void** counts);
 int nx_product_allreduce(nx_ctx* ctx, nx_product which, nx_comm* comm, double* total);
@@ -275,6 +280,38 @@ int nx_integrate_adaptive_deposit(nx_ctx* ctx, long long n, uint64_t seed, uint6
                                   unsigned long long* attempted_steps,
                                   unsigned long long* accepted_steps,
                                   unsigned long long* bounces);
+
+/* ---- K2i: 3-D ion production maps (ModelIonization) ----------------------------------------
+ * An extension (the reference has no such product).  nx_integrate_adaptive_ionize runs the
+ * adaptive driver on the resident packets exactly as nx_integrate_adaptive_deposit would (the
+ * same preconditions, the same kernel choice: perfect sticking or bounce, deviates keyed by
+ * seed / first_id, the same final state and step totals), and adds to the grid of
+ * nx_ionize_begin where the frac was lost in flight.  For every accepted step, before any
+ * surface, moon, escape or vanish handling:
+ *   loss       frac before the step - frac of the Runge-Kutta step (one f64 subtraction); a
+ *              step with loss == 0 is not recorded, a negative loss (a step across the shadow
+ *              edge) is recorded as it is
+ *   where      the midpoint of the step's chord, (x + x_rk) * 0.5 per axis, x_rk taken before
+ *              a bounce moves the packet; planet frame (R_p, Sun toward -y)
+ *   binning    np.histogramdd's rule on linspace(lo[k], hi[k], n[k] + 1) per axis, the last
+ *              right edge in the last cell; a midpoint outside the box, or NaN, goes to OUTSIDE
+ * Summed over the grid and OUTSIDE, the loss is ModelDeposition's LOST (SOURCE minus the other
+ * buckets), up to rounding.  The run needs a loss process (loss_mode 1 or 2): -1 otherwise.
+ * The sink is the NX_PRODUCT_IONIZE accumulator, nsum = ncount = nx * ny * nz + 1: the cells,
+ * row-major (nx, ny, nz), then OUTSIDE, each an f64 loss sum and a count of recorded steps.
+ * begin validates n[k] >= 1, lo[k] < hi[k] (finite) and nx * ny * nz + 1 < 2^31.  Every
+ * recorded step is one f64 and one u64 atomic add; a 100^3 grid (16 MB) stays in the B200's
+ * 126 MB L2, a 200^3 grid (128 MB) does not.                                                 */
+typedef struct nx_ion_grid {
+  double lo[3], hi[3];        /* box edges per axis (x, y, z), R_p                           */
+  int32_t n[3];               /* cells per axis                                              */
+  int32_t reserved;
+} nx_ion_grid;
+int nx_ionize_begin(nx_ctx* ctx, const nx_ion_grid* grid);
+int nx_integrate_adaptive_ionize(nx_ctx* ctx, long long n, uint64_t seed, uint64_t first_id,
+                                 unsigned long long* attempted_steps,
+                                 unsigned long long* accepted_steps,
+                                 unsigned long long* bounces);
 
 /* ---- K3: constant-step driver with bounce (Output.py:368-455, bouncepackets.py)
  * Optional fused per-step image accumulation (image_dev / counts_dev device

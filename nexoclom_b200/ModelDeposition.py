@@ -87,6 +87,46 @@ def regeneration(output):
     return 'seed', seed
 
 
+def regeneration_plan(inputs):
+    """(outid, outputfiles, outputs, recipes) of every output file of ``inputs``, with the
+    ``regeneration`` recipe of each; ValueError before any device work when one cannot be
+    regenerated (a bounce run needs the seed of its deviates)."""
+    outid, outputfiles, _, _ = inputs.search()
+    outputs = [catalogue.fetch(f) for f in outputfiles]
+    si = inputs.surfaceinteraction
+    bounce = not (si.sticktype == 'constant' and si.stickcoef == 1.0)
+    recipes = []
+    for output in outputs:
+        how = regeneration(output)
+        if bounce and getattr(output, 'seed', None) is None:
+            raise ValueError('a bounce run needs the seed of its deviates, and an output file '
+                             'has none (written by the reference?)')
+        recipes.append(how)
+    return outid, outputfiles, outputs, recipes
+
+
+def regenerate(model, eng, outputs, recipes, integrate):
+    """Re-run every Output on ``eng`` from its recipe through ``integrate(eng, seed, first_id,
+    n)``, a sink entry of the adaptive driver returning (attempted, accepted, bounces).  Adds
+    the step totals and the kernel time to ``model``; returns the summed totalsource."""
+    totalsource = 0.
+    for output, (kind, what) in zip(outputs, recipes):
+        setup = get_setup(model.inputs, strict_math=getattr(output, 'strict_math', False))
+        setup.upload(eng)
+        n = int(output.npackets)
+        if kind == 'x0':
+            eng.import_state(what)
+        else:
+            eng.init_state(setup.source_params(eng), what, output.first_id, n)
+        att, acc, bnc = integrate(eng, getattr(output, 'seed', None) or 0, output.first_id, n)
+        model.kernel_ms += eng.last_kernel_ms()
+        model.attempted_steps += att
+        model.accepted_steps += acc
+        model.bounces += bnc
+        totalsource += float(output.totalsource)
+    return totalsource
+
+
 class ModelDeposition:
     def __init__(self, inputs, params=None, device=None):
         params = {} if params is None else params
@@ -106,17 +146,7 @@ class ModelDeposition:
         self.longitude = 0.5 * (self.lon_edges[:-1] + self.lon_edges[1:])
         self.latitude = 0.5 * (self.lat_edges[:-1] + self.lat_edges[1:])
 
-        self.outid, self.outputfiles, _, _ = self.inputs.search()
-        outputs = [catalogue.fetch(f) for f in self.outputfiles]
-        si = self.inputs.surfaceinteraction
-        bounce = not (si.sticktype == 'constant' and si.stickcoef == 1.0)
-        recipes = []
-        for output in outputs:
-            how = regeneration(output)
-            if bounce and getattr(output, 'seed', None) is None:
-                raise ValueError('a bounce run needs the seed of its deviates, and an output file '
-                                 'has none (written by the reference?)')
-            recipes.append(how)
+        self.outid, self.outputfiles, outputs, recipes = regeneration_plan(self.inputs)
 
         comm = nccl_comm()
         dmap = np.zeros((nlon, nlat))
@@ -130,8 +160,8 @@ class ModelDeposition:
             eng = get_engine(self._device)
             eng.deposit_begin(nlon, nlat)
             try:
-                for output, (kind, what) in zip(outputs, recipes):
-                    totalsource += self._run(eng, output, kind, what)
+                totalsource = regenerate(self, eng, outputs, recipes,
+                                         Engine.integrate_adaptive_deposit)
                 if comm is not None:          # one collective; totalsource rides with the sink
                     totalsource = eng.deposit_allreduce(comm[1], totalsource)
                 dmap, cnt, sums, counts = eng.deposit_fetch(nlon, nlat)
@@ -140,23 +170,6 @@ class ModelDeposition:
         if comm is None:
             totalsource, = combine_ranks((dmap, cnt, sums, counts), totalsource)
         self._finish(dmap, cnt, sums, counts, totalsource)
-
-    def _run(self, eng, output, kind, what):
-        """One Output regenerated through the sink; returns its totalsource."""
-        setup = get_setup(self.inputs, strict_math=getattr(output, 'strict_math', False))
-        setup.upload(eng)
-        n = int(output.npackets)
-        if kind == 'x0':
-            eng.import_state(what)
-        else:
-            eng.init_state(setup.source_params(eng), what, output.first_id, n)
-        att, acc, bnc = eng.integrate_adaptive_deposit(getattr(output, 'seed', None) or 0,
-                                                       output.first_id, n)
-        self.kernel_ms += eng.last_kernel_ms()
-        self.attempted_steps += att
-        self.accepted_steps += acc
-        self.bounces += bnc
-        return float(output.totalsource)
 
     def _finish(self, dmap, cnt, sums, counts, totalsource):
         self.totalsource = totalsource

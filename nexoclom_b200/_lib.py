@@ -18,7 +18,7 @@ c_u32_p = C.POINTER(C.c_uint32)
 c_u8_p = C.POINTER(C.c_uint8)
 
 # nx_product: the context-owned accumulators
-NX_PRODUCT_IMAGE, NX_PRODUCT_CUBE, NX_PRODUCT_DEPOSIT = 0, 1, 2
+NX_PRODUCT_IMAGE, NX_PRODUCT_CUBE, NX_PRODUCT_DEPOSIT, NX_PRODUCT_IONIZE = 0, 1, 2, 3
 
 
 class RunParams(C.Structure):
@@ -34,6 +34,12 @@ class RunParams(C.Structure):
         ('moon_GM', C.c_double * 4), ('moon_a', C.c_double * 4), ('moon_omega', C.c_double * 4),
         ('moon_phi', C.c_double * 4), ('moon_r2', C.c_double * 4),
     ]
+
+
+class IonGrid(C.Structure):
+    """Mirror of ``nx_ion_grid``: the ion-production grid's box and cells per axis."""
+    _fields_ = [('lo', C.c_double * 3), ('hi', C.c_double * 3), ('n', C.c_int32 * 3),
+                ('reserved', C.c_int32)]
 
 
 class SourceParams(C.Structure):
@@ -168,6 +174,9 @@ def load():
         'nx_deposit_begin': [vp, C.c_int, C.c_int],
         'nx_integrate_adaptive_deposit': [vp, i64, u64, u64, C.POINTER(u64), C.POINTER(u64),
                                           C.POINTER(u64)],
+        'nx_ionize_begin': [vp, C.POINTER(IonGrid)],
+        'nx_integrate_adaptive_ionize': [vp, i64, u64, u64, C.POINTER(u64), C.POINTER(u64),
+                                         C.POINTER(u64)],
         'nx_product_fetch': [vp, C.c_int, c_double_p, c_i64_p],
         'nx_product_device_ptrs': [vp, C.c_int, C.POINTER(vp), C.POINTER(vp)],
         'nx_product_allreduce': [vp, C.c_int, vp, C.POINTER(C.c_double)],

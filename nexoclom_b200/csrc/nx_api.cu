@@ -135,7 +135,8 @@ struct nx_ctx {
   // cudaFree (an implicit device synchronisation each) on the calls LOSResult / ModelImage
   // make once per output file, and nothing to leak on an error path
   struct Scratch { void* p = nullptr; size_t bytes = 0; } scr[32];
-  Accum accum[NX_PRODUCT_DEPOSIT + 1];   // one per nx_product
+  Accum accum[NX_PRODUCT_IONIZE + 1];    // one per nx_product
+  IonOut ion_axes{};                     // the grid of nx_ionize_begin (axes only)
   void* pinned = nullptr;      // grow-only pinned staging for small D2H results (image, LOS columns)
   size_t pinned_bytes = 0;
   unsigned* cmp_tiles = nullptr;     // compaction scratch (tile counts)
@@ -317,15 +318,15 @@ static int pinned_staging(nx_ctx* ctx, size_t bytes) {
   return 0;
 }
 
-// ---- context-owned accumulators (image, cube, deposition) -----------------------------------
+// ---- context-owned accumulators (image, cube, deposition, ion production) -------------------
 // None of these calls ENTER: nothing here changes what the line-of-sight kernels read, so the
 // candidate pairs nx_los_accumulate_counted keeps stay valid.
 static const char* const accum_begin_name[] = {"nx_image_begin", "nx_cube_begin",
-                                               "nx_deposit_begin"};
+                                               "nx_deposit_begin", "nx_ionize_begin"};
 
 // The accumulator of `which` when its begin has run; else NULL with the error set.
 static Accum* accum_of(nx_ctx* ctx, int which) {
-  if (which < NX_PRODUCT_IMAGE || which > NX_PRODUCT_DEPOSIT) {
+  if (which < NX_PRODUCT_IMAGE || which > NX_PRODUCT_IONIZE) {
     ctx->err = "unknown nx_product";
     return nullptr;
   }
@@ -926,9 +927,11 @@ static int check_status(nx_ctx* ctx) {
 // [3] bounces), longest first when ordering is on, inside the caller's timed section.
 // S != nullptr: packets bounce (nx_integrate_adaptive_bounce); the cost model then budgets
 // every packet's remaining time, since reaching the surface no longer ends its flight.
-// dep != nullptr: the SINK build of the same kernel (nx_integrate_adaptive_deposit).
+// dep != nullptr: the SINK build of the same kernel (nx_integrate_adaptive_deposit);
+// ion != nullptr: its ion build (nx_integrate_adaptive_ionize).
 static int adaptive_resident(nx_ctx* ctx, long long n, const Spline2D* S, uint64_t seed,
-                             uint64_t first_id, const DepositOut* dep = nullptr) {
+                             uint64_t first_id, const DepositOut* dep = nullptr,
+                             const IonOut* ion = nullptr) {
   const bool order = ctx->order_packets && n >= 4096;
   const bool to_surface = !S || perfect_sticking(ctx->params);
   if (order)
@@ -938,7 +941,7 @@ static int adaptive_resident(nx_ctx* ctx, long long n, const Spline2D* S, uint64
                                ctx->params,
                                ctx->radpres.view, ctx->radpres.fast,
                                order ? ctx->perm : nullptr, ctx->scalars, ctx->scalars + 1,
-                               ctx->att, ctx->acc, ctx->status, S, seed, first_id, dep));
+                               ctx->att, ctx->acc, ctx->status, S, seed, first_id, dep, ion));
   return end_timed(ctx, order ? 4 : 1);
 }
 
@@ -1071,6 +1074,80 @@ int nx_integrate_adaptive_deposit(nx_ctx* ctx, long long n, uint64_t seed, uint6
     d.nlon = sink->dims[0]; d.nlat = sink->dims[1];
     if ((r = begin_timed(ctx))) return r;
     if ((r = adaptive_resident(ctx, n, bounce ? &ctx->spline : nullptr, seed, first_id, &d)))
+      return r;
+    ctx->fresh = false;
+  }
+  unsigned long long h[4] = {0, 0, 0, 0};
+  CK(cudaMemcpyAsync(h, ctx->scalars, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
+  r = check_status(ctx);
+  if (r < 0) return r;
+  if (attempted) *attempted = h[1];
+  if (accepted) *accepted = h[2];
+  if (bounces) *bounces = h[3];
+  return r;
+}
+
+// ---- K2i: ion production maps (ModelIonization) ---------------------------------------------
+// The sink is the NX_PRODUCT_IONIZE accumulator: the grid's cells, row-major (nx, ny, nz), then
+// OUTSIDE, in the sums and in the counts.
+// nx_integrate_adaptive_ionize runs k_ionize_adaptive, the build of the kernel
+// nx_integrate_adaptive (perfect sticking) or nx_integrate_adaptive_bounce would run, on the
+// resident packets: the same final state and step totals, plus the loss added to the grid.
+static_assert(sizeof(nx_ion_grid) == 64, "nx_ion_grid layout");
+
+int nx_ionize_begin(nx_ctx* ctx, const nx_ion_grid* grid) {
+  CK(cudaSetDevice(ctx->device));
+  if (!grid) { ctx->err = "nx_ionize_begin: grid is NULL"; return -1; }
+  double ncell = 1.0;
+  for (int a = 0; a < 3; ++a) {
+    if (grid->n[a] < 1) { ctx->err = "nx_ionize_begin: n must be >= 1 on every axis"; return -1; }
+    if (!(std::isfinite(grid->lo[a]) && std::isfinite(grid->hi[a]) && grid->lo[a] < grid->hi[a])) {
+      ctx->err = "nx_ionize_begin: lo < hi, both finite, on every axis";
+      return -1;
+    }
+    ncell *= grid->n[a];
+  }
+  if (ncell + 1.0 >= 2147483648.0) {
+    ctx->err = "nx_ionize_begin: nx * ny * nz + 1 must be < 2^31";
+    return -1;
+  }
+  IonOut g{};
+  for (int a = 0; a < 3; ++a) { g.lo[a] = grid->lo[a]; g.hi[a] = grid->hi[a]; g.n[a] = grid->n[a]; }
+  ion_steps(g);
+  const long long n = (long long)ncell + 1;
+  int r = accum_begin(ctx, NX_PRODUCT_IONIZE, n, n, g.n[0], g.n[1], g.n[2]);
+  if (r == 0) ctx->ion_axes = g;
+  return r;
+}
+
+int nx_integrate_adaptive_ionize(nx_ctx* ctx, long long n, uint64_t seed, uint64_t first_id,
+                                 unsigned long long* attempted, unsigned long long* accepted,
+                                 unsigned long long* bounces) {
+  ENTER(ctx);
+  const Accum* sink = accum_of(ctx, NX_PRODUCT_IONIZE);
+  if (!sink) return -1;
+  if (!ctx->have_params) { ctx->err = "nx_tables_upload not called"; return -1; }
+  ctx->bound = nullptr;            // integrators work on the slab
+  if (n < 0 || n > ctx->cap) { ctx->err = "n exceeds resident packets"; return -1; }
+  const RunParams& p = ctx->params;
+  if (p.loss_mode != LOSS_LIFETIME && p.loss_mode != LOSS_PHOTO) {
+    ctx->err = "nx_integrate_adaptive_ionize: the run has no loss process (loss_mode 0)";
+    return -1;
+  }
+  const bool bounce = !perfect_sticking(p);
+  if (bounce && p.accomfactor != 0.0 && !ctx->spl_c) {
+    ctx->err = "accommodation enabled but no speed spline uploaded";
+    return -1;
+  }
+  CK(cudaMemsetAsync(ctx->scalars, 0, 8 * sizeof(unsigned long long), ctx->stream));
+  int r;
+  if (n > 0) {
+    IonOut g = ctx->ion_axes;
+    g.sum = sink->sums();
+    g.cnt = sink->counts();
+    if ((r = begin_timed(ctx))) return r;
+    if ((r = adaptive_resident(ctx, n, bounce ? &ctx->spline : nullptr, seed, first_id, nullptr,
+                               &g)))
       return r;
     ctx->fresh = false;
   }

@@ -306,11 +306,13 @@ NX_HD void fast_stages(const RunParams& p, const FastTable& T, const double* s, 
 
 // One attempted adaptive step, fast arithmetic.  Same contract as
 // adaptive_attempt<>(): s[0..7] = time,x,y,z,vx,vy,vz,frac; returns AttemptFlags.
-// BOUNCE, S, seed, id, k, SINK, D: as in adaptive_attempt<>().
-template <int GR, int RP, int LOSS, int MO = 0, bool BOUNCE = false, bool SINK = false>
+// BOUNCE, S, seed, id, k, SINK, D, ION, I: as in adaptive_attempt<>().
+template <int GR, int RP, int LOSS, int MO = 0, bool BOUNCE = false, bool SINK = false,
+          bool ION = false>
 NX_HD int adaptive_attempt_fast(const RunParams& p, const FastTable& T, double* s,
                                 double& step, const Spline2D* S = nullptr, uint64_t seed = 0,
-                                uint64_t id = 0, uint32_t k = 0, DepositSink* D = nullptr) {
+                                uint64_t id = 0, uint32_t k = 0, DepositSink* D = nullptr,
+                                IonSink* I = nullptr) {
   const double res = p.resolution;
   const double resv = 0.1 * res;
   const double h = fmin(s[0], step);
@@ -347,6 +349,10 @@ NX_HD int adaptive_attempt_fast(const RunParams& p, const FastTable& T, double* 
   int flags = 0;
   if (!(dsum <= 1.7976931348623157e308)) flags |= ATT_BAD_ERRMAX;    // NaN / inf deltas
   if (accept) {
+    if (ION) {                             // before a bounce moves the packet
+      const double loss = s[7] - fn;
+      if (loss != 0.0) ion_record(*I, loss, (s[1] + px) * 0.5, (s[2] + py) * 0.5, (s[3] + pz) * 0.5);
+    }
     const double r2 = fma(pz, pz, fma(py, py, px * px));
     double f = fn;
     double dep = 0.0, ff = 0.0;            // SINK: deposited frac, frac of the fate event
@@ -393,28 +399,28 @@ NX_HD int adaptive_attempt_fast(const RunParams& p, const FastTable& T, double* 
 }
 
 // runtime dispatch over the compile-time force / loss combinations
-template <bool BOUNCE = false, bool SINK = false>
+template <bool BOUNCE = false, bool SINK = false, bool ION = false>
 NX_HD int adaptive_attempt_fast_rt(const RunParams& p, const FastTable& T, double* s,
                                    double& step, const Spline2D* S = nullptr, uint64_t seed = 0,
                                    uint64_t id = 0, uint32_t k = 0,
-                                   DepositSink* D = nullptr) {
-#define NX_ARGS p, T, s, step, S, seed, id, k, D
+                                   DepositSink* D = nullptr, IonSink* I = nullptr) {
+#define NX_ARGS p, T, s, step, S, seed, id, k, D, I
   if (p.nmoons == 1 && p.gravity) {
     if (p.radpres) {
-      if (p.loss_mode == LOSS_PHOTO) return adaptive_attempt_fast<1, 1, LOSS_PHOTO, 1, BOUNCE, SINK>(NX_ARGS);
-      if (p.loss_mode == LOSS_LIFETIME) return adaptive_attempt_fast<1, 1, LOSS_LIFETIME, 1, BOUNCE, SINK>(NX_ARGS);
-      return adaptive_attempt_fast<1, 1, LOSS_NONE, 1, BOUNCE, SINK>(NX_ARGS);
+      if (p.loss_mode == LOSS_PHOTO) return adaptive_attempt_fast<1, 1, LOSS_PHOTO, 1, BOUNCE, SINK, ION>(NX_ARGS);
+      if (p.loss_mode == LOSS_LIFETIME) return adaptive_attempt_fast<1, 1, LOSS_LIFETIME, 1, BOUNCE, SINK, ION>(NX_ARGS);
+      return adaptive_attempt_fast<1, 1, LOSS_NONE, 1, BOUNCE, SINK, ION>(NX_ARGS);
     }
-    if (p.loss_mode == LOSS_PHOTO) return adaptive_attempt_fast<1, 0, LOSS_PHOTO, 1, BOUNCE, SINK>(NX_ARGS);
-    if (p.loss_mode == LOSS_LIFETIME) return adaptive_attempt_fast<1, 0, LOSS_LIFETIME, 1, BOUNCE, SINK>(NX_ARGS);
-    return adaptive_attempt_fast<1, 0, LOSS_NONE, 1, BOUNCE, SINK>(NX_ARGS);
+    if (p.loss_mode == LOSS_PHOTO) return adaptive_attempt_fast<1, 0, LOSS_PHOTO, 1, BOUNCE, SINK, ION>(NX_ARGS);
+    if (p.loss_mode == LOSS_LIFETIME) return adaptive_attempt_fast<1, 0, LOSS_LIFETIME, 1, BOUNCE, SINK, ION>(NX_ARGS);
+    return adaptive_attempt_fast<1, 0, LOSS_NONE, 1, BOUNCE, SINK, ION>(NX_ARGS);
   }
   const int key = (p.gravity ? 4 : 0) | (p.radpres ? 2 : 0);
 #define NX_CASE(G, R)                                                                    \
   if (key == ((G) * 4 + (R) * 2)) {                                                      \
-    if (p.loss_mode == LOSS_PHOTO) return adaptive_attempt_fast<G, R, LOSS_PHOTO, 0, BOUNCE, SINK>(NX_ARGS);       \
-    if (p.loss_mode == LOSS_LIFETIME) return adaptive_attempt_fast<G, R, LOSS_LIFETIME, 0, BOUNCE, SINK>(NX_ARGS); \
-    return adaptive_attempt_fast<G, R, LOSS_NONE, 0, BOUNCE, SINK>(NX_ARGS);                     \
+    if (p.loss_mode == LOSS_PHOTO) return adaptive_attempt_fast<G, R, LOSS_PHOTO, 0, BOUNCE, SINK, ION>(NX_ARGS);       \
+    if (p.loss_mode == LOSS_LIFETIME) return adaptive_attempt_fast<G, R, LOSS_LIFETIME, 0, BOUNCE, SINK, ION>(NX_ARGS); \
+    return adaptive_attempt_fast<G, R, LOSS_NONE, 0, BOUNCE, SINK, ION>(NX_ARGS);                     \
   }
   NX_CASE(1, 1) NX_CASE(1, 0) NX_CASE(0, 1) NX_CASE(0, 0)
 #undef NX_CASE

@@ -81,6 +81,42 @@ NX_HD int deposit_cell(double lon, double lat, int nlon, int nlat) {
   return (i < 0 || j < 0) ? -1 : i * nlat + j;
 }
 
+// Ion-production grid cell of (x, y, z), row-major (ix * ny + iy) * nz + iz, by
+// np.histogramdd's rule per axis (hist_bin_fast); -1 outside the box or NaN.
+NX_HD long long ion_cell(const IonOut& g, double x, double y, double z) {
+  const int i = hist_bin_fast(x, g.n[0], g.lo[0], g.hi[0], g.step[0], g.inv_step[0]);
+  const int j = hist_bin_fast(y, g.n[1], g.lo[1], g.hi[1], g.step[1], g.inv_step[1]);
+  const int k = hist_bin_fast(z, g.n[2], g.lo[2], g.hi[2], g.step[2], g.inv_step[2]);
+  if (i < 0 || j < 0 || k < 0) return -1;
+  return ((long long)i * g.n[1] + j) * g.n[2] + k;
+}
+
+// The steps and reciprocals of the grid's axes, as ImageSteps forms them.
+NX_HD void ion_steps(IonOut& g) {
+  for (int a = 0; a < 3; ++a) {
+    g.step[a] = (g.hi[a] - g.lo[a]) / g.n[a];
+    g.inv_step[a] = 1.0 / g.step[a];
+  }
+}
+
+// Ion production of one accepted adaptive step (declared in nx_physics.cuh).
+template <class Sink>
+NX_COLD void ion_record(Sink& I, double loss, double x, double y, double z) {
+  const long long c = ion_cell(I.g, x, y, z);
+  if (c < 0) {
+    I.out_sum += loss;
+    I.out_n += 1;
+    return;
+  }
+#if defined(__CUDA_ARCH__)
+  atomicAdd(I.g.sum + c, loss);
+  atomicAdd(I.g.cnt + c, 1ull);
+#else
+  I.g.sum[c] += loss;
+  I.g.cnt[c] += 1;
+#endif
+}
+
 // per-launch constants of the image kernels
 struct ImageSteps {
   double step_x, step_z;          // bin widths, as np.histogram2d's linspace gives them

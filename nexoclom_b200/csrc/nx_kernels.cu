@@ -301,15 +301,18 @@ struct PacketFeeder {
 // and vanish event (deposit_record), the kernel the initial frac (SOURCE) and the frac of the
 // packets that retire alive (REMAINING); Dep is unused otherwise.  The final state and the
 // step totals are the same as without the sink.
-template <int MODE, bool BOUNCE = false, bool SINK = false>
-__global__ void __launch_bounds__(NX_INT_THREADS, NX_INT_MINBLOCKS)
-k_integrate_adaptive(StateCols In, StateCols P, long long n, RunParams p, InterpTable Tg,
-                     FastTable Fg, const unsigned* __restrict__ perm,
-                     unsigned long long* __restrict__ queue,
-                     unsigned long long* __restrict__ totals,
-                     unsigned* __restrict__ att_out, unsigned* __restrict__ acc_out,
-                     int* __restrict__ status, unsigned table_bytes, Spline2D S, uint64_t seed,
-                     uint64_t first_id, DepositOut Dep) {
+// ION: the ion-production sink (ModelIonization, k_ionize_adaptive): the attempts record the
+// frac every accepted step loses in flight (ion_record), each lane its OUTSIDE share, reduced
+// here; Ion is unused otherwise.  The final state and the step totals are again unchanged.
+// The persistent lane loop of both kernels (feeder, refill, step totals), inlined into each.
+template <int MODE, bool BOUNCE, bool SINK, bool ION>
+__device__ __forceinline__ void
+adaptive_lanes(const StateCols& In, const StateCols& P, long long n, const RunParams& p,
+               const InterpTable& Tg, const FastTable& Fg, const unsigned* __restrict__ perm,
+               unsigned long long* __restrict__ queue, unsigned long long* __restrict__ totals,
+               unsigned* __restrict__ att_out, unsigned* __restrict__ acc_out,
+               int* __restrict__ status, unsigned table_bytes, const Spline2D& S, uint64_t seed,
+               uint64_t first_id, const DepositOut& Dep, const IonOut& Ion) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   InterpTable T;
   FastTable F;
@@ -336,6 +339,8 @@ k_integrate_adaptive(StateCols In, StateCols P, long long n, RunParams p, Interp
 #pragma unroll
     for (int b = 0; b < DEP_NBUCKET; ++b) { D.sum[b] = 0.0; D.n[b] = 0; }
   }
+  IonSink I;                     // ION: lives in local memory, the grid read by ion_record
+  if (ION) { I.g = Ion; I.out_sum = 0.0; I.out_n = 0; }
 #ifdef NX_STREAM_DEBUG
   unsigned long long dbg_iters = 0;
 #endif
@@ -379,12 +384,13 @@ k_integrate_adaptive(StateCols In, StateCols P, long long n, RunParams p, Interp
     if (have) {
       int fl;
       if (MODE < 0)
-        fl = adaptive_attempt<true, BOUNCE, SINK>(p, T, s, step, &S, seed, first_id + idx, acc + 1,
-                                                  SINK ? &D : nullptr);
+        fl = adaptive_attempt<true, BOUNCE, SINK, ION>(p, T, s, step, &S, seed, first_id + idx,
+                                                       acc + 1, SINK ? &D : nullptr,
+                                                       ION ? &I : nullptr);
       else
         fl = adaptive_attempt_fast<(MODE >> 3) & 1, (MODE >> 2) & 1, MODE & 3, (MODE >> 4) & 1, BOUNCE,
-                                   SINK>(p, F, s, step, &S, seed, first_id + idx, acc + 1,
-                                         SINK ? &D : nullptr);
+                                   SINK, ION>(p, F, s, step, &S, seed, first_id + idx, acc + 1,
+                                              SINK ? &D : nullptr, ION ? &I : nullptr);
       ++att;
       if (fl & ATT_ACCEPTED) ++acc;
       if (BOUNCE && (fl & ATT_BOUNCED)) ++tot_bnc;
@@ -435,6 +441,50 @@ k_integrate_adaptive(StateCols In, StateCols P, long long n, RunParams p, Interp
       }
     }
   }
+  if (ION) {
+    double v = I.out_sum;
+    unsigned long long c = I.out_n;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      v += __shfl_xor_sync(FULL_MASK, v, o);
+      c += __shfl_xor_sync(FULL_MASK, c, o);
+    }
+    if (lane == 0 && c) {
+      const long long out = (long long)Ion.n[0] * Ion.n[1] * Ion.n[2];
+      atomicAdd(Ion.sum + out, v);
+      atomicAdd(Ion.cnt + out, c);
+    }
+  }
+}
+
+template <int MODE, bool BOUNCE = false, bool SINK = false>
+__global__ void __launch_bounds__(NX_INT_THREADS, NX_INT_MINBLOCKS)
+k_integrate_adaptive(StateCols In, StateCols P, long long n, RunParams p, InterpTable Tg,
+                     FastTable Fg, const unsigned* __restrict__ perm,
+                     unsigned long long* __restrict__ queue,
+                     unsigned long long* __restrict__ totals,
+                     unsigned* __restrict__ att_out, unsigned* __restrict__ acc_out,
+                     int* __restrict__ status, unsigned table_bytes, Spline2D S, uint64_t seed,
+                     uint64_t first_id, DepositOut Dep) {
+  adaptive_lanes<MODE, BOUNCE, SINK, false>(In, P, n, p, Tg, Fg, perm, queue, totals, att_out,
+                                            acc_out, status, table_bytes, S, seed, first_id, Dep,
+                                            IonOut{});
+}
+
+// K2i: the adaptive driver with the ion-production sink (ModelIonization).  Built only where
+// the run has a loss term: the strict kernel and MODE & 3 = LOSS_LIFETIME or LOSS_PHOTO.
+template <int MODE, bool BOUNCE>
+__global__ void __launch_bounds__(NX_INT_THREADS, NX_INT_MINBLOCKS)
+k_ionize_adaptive(StateCols In, StateCols P, long long n, RunParams p, InterpTable Tg,
+                  FastTable Fg, const unsigned* __restrict__ perm,
+                  unsigned long long* __restrict__ queue,
+                  unsigned long long* __restrict__ totals,
+                  unsigned* __restrict__ att_out, unsigned* __restrict__ acc_out,
+                  int* __restrict__ status, unsigned table_bytes, Spline2D S, uint64_t seed,
+                  uint64_t first_id, IonOut Ion) {
+  adaptive_lanes<MODE, BOUNCE, false, true>(In, P, n, p, Tg, Fg, perm, queue, totals, att_out,
+                                            acc_out, status, table_bytes, S, seed, first_id,
+                                            DepositOut{}, Ion);
 }
 
 // ---------------------------------------------------------------------------
@@ -1556,6 +1606,26 @@ static cudaError_t persistent_grid(K kernel, int device, size_t smem, int* block
   return cudaSuccess;
 }
 
+// the ion builds: the kernels with a loss term (MODE & 3 = LOSS_LIFETIME or LOSS_PHOTO) and
+// the strict kernels
+constexpr bool ion_build(int mode) {
+  return mode < 0 || (mode & 3) == LOSS_LIFETIME || (mode & 3) == LOSS_PHOTO;
+}
+
+template <typename K, typename... Args>
+static cudaError_t launch_lanes(K kernel, cudaStream_t st, int device, size_t smem, long long n,
+                                Args... args) {
+  int blocks = 0;
+  cudaError_t e = persistent_grid(kernel, device, smem, &blocks);
+  if (e != cudaSuccess) return e;
+  const long long need = (n + NX_INT_THREADS - 1) / NX_INT_THREADS;
+  if (need < blocks) blocks = (int)(need > 0 ? need : 1);
+  kernel<<<blocks, NX_INT_THREADS, smem, st>>>(args...);
+  return cudaGetLastError();
+}
+
+// Ion != nullptr: the same run through k_ionize_adaptive<MODE, BOUNCE> (SINK false, MODE with
+// a loss term), so the ion run selects its build by the dispatch of the plain run.
 template <int MODE, bool BOUNCE = false, bool SINK = false>
 static cudaError_t launch_adaptive_mode(cudaStream_t st, int device, StateCols In, StateCols P,
                                         long long n,
@@ -1564,18 +1634,20 @@ static cudaError_t launch_adaptive_mode(cudaStream_t st, int device, StateCols I
                                         const unsigned* perm, unsigned long long* queue,
                                         unsigned long long* totals, unsigned* att, unsigned* acc,
                                         int* status, const Spline2D& S, uint64_t seed,
-                                        uint64_t first_id, const DepositOut& Dep) {
+                                        uint64_t first_id, const DepositOut& Dep,
+                                        const IonOut* Ion) {
   const size_t tbytes = (MODE < 0) ? table_smem_bytes(T) : fast_table_smem_bytes(F);
   const size_t smem = tbytes + (size_t)(NX_INT_THREADS / 32) * NX_FEED_BYTES_PER_WARP;
-  int blocks = 0;
-  cudaError_t e = persistent_grid(k_integrate_adaptive<MODE, BOUNCE, SINK>, device, smem, &blocks);
-  if (e != cudaSuccess) return e;
-  const long long need = (n + NX_INT_THREADS - 1) / NX_INT_THREADS;
-  if (need < blocks) blocks = (int)(need > 0 ? need : 1);
-  k_integrate_adaptive<MODE, BOUNCE, SINK><<<blocks, NX_INT_THREADS, smem, st>>>(
-      In, P, n, p, T, F, perm, queue, totals, att, acc, status, (unsigned)tbytes, S, seed,
-      first_id, Dep);
-  return cudaGetLastError();
+  if constexpr (!SINK && ion_build(MODE)) {
+    if (Ion)
+      return launch_lanes(k_ionize_adaptive<MODE, BOUNCE>, st, device, smem, n, In, P, n, p, T, F,
+                          perm, queue, totals, att, acc, status, (unsigned)tbytes, S, seed,
+                          first_id, *Ion);
+  }
+  if (Ion) return cudaErrorInvalidValue;         // no ion build: a run without loss
+  return launch_lanes(k_integrate_adaptive<MODE, BOUNCE, SINK>, st, device, smem, n, In, P, n, p,
+                      T, F, perm, queue, totals, att, acc, status, (unsigned)tbytes, S, seed,
+                      first_id, Dep);
 }
 
 #ifdef NX_STREAM_DEBUG
@@ -1679,7 +1751,8 @@ cudaError_t launch_cost_order(cudaStream_t st, int device, StateCols P, long lon
   return cudaGetLastError();
 }
 
-// K2 / K2b kernel selection; SINK builds exist for every kernel it can select.
+// K2 / K2b kernel selection; SINK builds exist for every kernel it can select, ion builds
+// (Ion != nullptr, SINK false) for those of them with a loss term.
 template <bool SINK>
 static cudaError_t dispatch_adaptive(cudaStream_t st, int device, StateCols In, StateCols P,
                                      long long n, const RunParams& p, const InterpTable& T,
@@ -1687,9 +1760,9 @@ static cudaError_t dispatch_adaptive(cudaStream_t st, int device, StateCols In, 
                                      unsigned long long* queue, unsigned long long* totals,
                                      unsigned* att, unsigned* acc, int* status,
                                      const Spline2D* S, uint64_t seed, uint64_t first_id,
-                                     const DepositOut& Dep) {
+                                     const DepositOut& Dep, const IonOut* Ion) {
 #define NX_ARGS st, device, In, P, n, p, T, F, perm, queue, totals, att, acc, status, \
-                S ? *S : Spline2D{}, seed, first_id, Dep
+                S ? *S : Spline2D{}, seed, first_id, Dep, Ion
   if (S) {
     // bounce builds: the strict kernel, and the fast kernels with gravity (one moon too);
     // runs without gravity or with more moons take the strict kernel
@@ -1744,12 +1817,13 @@ cudaError_t launch_integrate_adaptive(cudaStream_t st, int device, StateCols In,
                                       unsigned long long* queue, unsigned long long* totals,
                                       unsigned* att, unsigned* acc, int* status,
                                       const Spline2D* S, uint64_t seed, uint64_t first_id,
-                                      const DepositOut* dep) {
+                                      const DepositOut* dep, const IonOut* ion) {
+  if (dep && ion) return cudaErrorInvalidValue;
   if (dep)
     return dispatch_adaptive<true>(st, device, In, P, n, p, T, F, perm, queue, totals, att, acc,
-                                   status, S, seed, first_id, *dep);
+                                   status, S, seed, first_id, *dep, nullptr);
   return dispatch_adaptive<false>(st, device, In, P, n, p, T, F, perm, queue, totals, att, acc,
-                                  status, S, seed, first_id, DepositOut{});
+                                  status, S, seed, first_id, DepositOut{}, ion);
 }
 
 template <int MODE>

@@ -157,13 +157,16 @@ struct DepositOut {
 // S != nullptr: packets bounce (totals[2] counts the bounces), deviates keyed by
 // (seed, first_id + packet index); nullptr: the reference's driver (Q6).
 // dep != nullptr: the same run through the kernel's SINK build, which adds its events to *dep.
+// ion != nullptr (dep == nullptr, a run with a loss term): the same run through
+// k_ionize_adaptive, which adds the frac lost in flight to the grid *ion.
 cudaError_t launch_integrate_adaptive(cudaStream_t st, int device, StateCols In, StateCols P,
                                       long long n, const RunParams& p, const InterpTable& T,
                                       const FastTable& F, const unsigned* perm,
                                       unsigned long long* queue, unsigned long long* totals,
                                       unsigned* att, unsigned* acc, int* status,
                                       const Spline2D* S = nullptr, uint64_t seed = 0,
-                                      uint64_t first_id = 0, const DepositOut* dep = nullptr);
+                                      uint64_t first_id = 0, const DepositOut* dep = nullptr,
+                                      const IonOut* ion = nullptr);
 #define NX_STREAM_GROUP 128          // == NX_GROUP: segment sizes are multiples of this
 #define NX_STREAM_MAX_SEG 32
 #define NX_STREAM_CURSORS 256        // >= NX_NCLASS x 32 u64 cursors

@@ -452,15 +452,43 @@ template <class Sink>
 NX_COLD void deposit_record(Sink& D, bool surf, double x, double y, double z, double dep,
                             int fate, double ff);
 
+// The ion-production grid (ION builds of the adaptive driver, ModelIonization): n[0] x n[1] x
+// n[2] cells, row-major, of f64 frac sums and u64 step counts, then one OUTSIDE slot (index
+// n[0] * n[1] * n[2]) in each; per axis np.histogramdd's edges linspace(lo, hi, n + 1), with
+// the bin widths and their reciprocals formed once per launch as ImageSteps does.
+struct IonOut {
+  double* sum;
+  unsigned long long* cnt;
+  double lo[3], hi[3], step[3], inv_step[3];
+  int n[3];
+};
+
+// One lane's ion sink: the grid, and this lane's OUTSIDE sum and count, reduced when the
+// kernel ends.
+struct IonSink {
+  IonOut g;
+  double out_sum;
+  unsigned long long out_n;
+};
+
+// Records the frac `loss` one accepted step lost in flight at its chord midpoint (x, y, z):
+// one f64 and one u64 atomic add to its cell, or the lane's OUTSIDE slot (outside the box, or
+// NaN).  Defined in nx_image.cuh, an out-of-line call like deposit_record().
+template <class Sink>
+NX_COLD void ion_record(Sink& I, double loss, double x, double y, double z);
+
 // BOUNCE = false: the reference's driver (a packet that hits the surface sticks, Q6).
 // BOUNCE = true: accepted steps that end inside the planet go through adaptive_surface()
 // unless the sticking is perfect; S / seed / id / k feed it (unused otherwise).
 // SINK = true: every surface, moon, escape and vanish event goes to deposit_record(*D); the
 // state the attempt computes is the same as without the sink.
-template <bool STRICT, bool BOUNCE = false, bool SINK = false>
+// ION = true: every accepted step that changes the frac goes to ion_record(*I) with
+// frac before - frac of the Runge-Kutta step, at the midpoint of the step's chord (before a
+// bounce moves the packet); the state is again the same as without it.
+template <bool STRICT, bool BOUNCE = false, bool SINK = false, bool ION = false>
 NX_HD int adaptive_attempt(const RunParams& p, const InterpTable& T, double* s, double& step,
                            const Spline2D* S = nullptr, uint64_t seed = 0, uint64_t id = 0,
-                           uint32_t k = 0, DepositSink* D = nullptr) {
+                           uint32_t k = 0, DepositSink* D = nullptr, IonSink* I = nullptr) {
   const double res = p.resolution;
   const double resv = mul_rn(0.1, res);
   const double h = fmin(s[0], step);
@@ -485,6 +513,12 @@ NX_HD int adaptive_attempt(const RunParams& p, const InterpTable& T, double* s, 
   double htried = h;
   if (errmax < 1e-7) { errmax = 1.0; htried = mul_rn(h, 10.0); }       // quirk Q4
   if (errmax < 1.0) {
+    if (ION) {
+      const double loss = sub_rn(s[7], nx[7]);
+      if (loss != 0.0)
+        ion_record(*I, loss, mul_rn(add_rn(s[1], nx[1]), 0.5), mul_rn(add_rn(s[2], nx[2]), 0.5),
+                   mul_rn(add_rn(s[3], nx[3]), 0.5));
+    }
     const double r2 = add_rn(add_rn(mul_rn(nx[1], nx[1]), mul_rn(nx[2], nx[2])), mul_rn(nx[3], nx[3]));
     double f = nx[7];
     double dep = 0.0, ff = 0.0;            // SINK: deposited frac, frac of the fate event

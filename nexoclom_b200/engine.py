@@ -11,7 +11,8 @@ import numpy as np
 
 from . import _lib
 from ._lib import (RunParams, SourceParams, ImageParams, LosParams, SpectrumParams, as_f64,
-                   dptr, c_double_p, NX_PRODUCT_IMAGE, NX_PRODUCT_CUBE, NX_PRODUCT_DEPOSIT)
+                   dptr, c_double_p, NX_PRODUCT_IMAGE, NX_PRODUCT_CUBE, NX_PRODUCT_DEPOSIT,
+                   NX_PRODUCT_IONIZE)
 
 STATE_COLS = ('time', 'x', 'y', 'z', 'vx', 'vy', 'vz', 'frac')
 X0_COLS = ('time', 'x', 'y', 'z', 'vx', 'vy', 'vz', 'frac', 'v', 'longitude', 'latitude',
@@ -581,6 +582,46 @@ class Engine:
     def deposit_end(self):
         """Release the deposition sink's device memory."""
         self._product_end(NX_PRODUCT_DEPOSIT)
+
+    def ionize_begin(self, lo, hi, dims):
+        """Allocate and zero the context-owned ion-production grid: the box ``lo``..``hi``
+        (x, y, z in R_p) in ``dims`` = (nx, ny, nz) cells of f64 loss sums and int64 step
+        counts, plus OUTSIDE, until ``ionize_end``."""
+        g = _lib.IonGrid()
+        for k in range(3):
+            g.lo[k], g.hi[k], g.n[k] = float(lo[k]), float(hi[k]), int(dims[k])
+        self._check(self.lib.nx_ionize_begin(self.ctx, C.byref(g)), 'nx_ionize_begin')
+
+    def integrate_adaptive_ionize(self, seed, first_id=0, n=None):
+        """K2 on the resident packets through its ion-production sink: the run
+        ``integrate_adaptive_deposit`` would make, the frac each accepted step loses in flight
+        added to the grid at the step's chord midpoint.  Returns (attempted, accepted,
+        bounces)."""
+        att, acc, bnc = C.c_ulonglong(), C.c_ulonglong(), C.c_ulonglong()
+        n = self.n if n is None else n
+        self._check(self.lib.nx_integrate_adaptive_ionize(self.ctx, int(n), int(seed),
+                                                          int(first_id), C.byref(att),
+                                                          C.byref(acc), C.byref(bnc)),
+                    'nx_integrate_adaptive_ionize')
+        return int(att.value), int(acc.value), int(bnc.value)
+
+    def ionize_fetch(self, dims):
+        """(sums, counts, outside, outside_count): the (nx, ny, nz) grid's loss sums (float64)
+        and recorded steps (int64), then OUTSIDE's sum and count."""
+        shape = tuple(int(d) for d in dims)
+        ncell = shape[0] * shape[1] * shape[2]
+        sums, cnt = self._product_fetch(NX_PRODUCT_IONIZE, (ncell + 1,))
+        return (sums[:ncell].reshape(shape), cnt[:ncell].reshape(shape), float(sums[ncell]),
+                int(cnt[ncell]))
+
+    def ionize_allreduce(self, comm, total):
+        """Sum the ion-production grid over the ranks of ``comm`` in place, with one scalar
+        riding along; returns the summed scalar."""
+        return self._product_allreduce(NX_PRODUCT_IONIZE, comm, total)
+
+    def ionize_end(self):
+        """Release the ion-production grid's device memory."""
+        self._product_end(NX_PRODUCT_IONIZE)
 
     # -- context-owned accumulators (nx_product) --------------------------------
     def _product_fetch(self, which, shape):
