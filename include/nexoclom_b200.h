@@ -116,7 +116,7 @@ typedef struct nx_image_params {
 
 /* Line-of-sight accumulation (compute_iteration.py:90-240). */
 typedef struct nx_los_params {
-  double dphi;               /* cone half-angle [rad]                               */
+  double dphi;               /* cone half-angle [rad], finite, > 0 and < pi/2       */
   double outeredge;          /* R_p                                                 */
   double vrplanet;           /* R_p/s                                               */
   double rp_cm;              /* planet radius [cm]                                  */

@@ -72,6 +72,17 @@ def dist_from_planet_cut(data):
     return dist_from_plan
 
 
+def cone_half_angle(dphi):
+    """The lines of sight's cone half-angle in radians, from a Quantity or a number of
+    degrees.  ValueError unless it is finite, > 0 and < 90 degrees (the same rule the C ABI
+    applies), so a bad angle fails before any device work."""
+    rad = (float(dphi.to('rad').value) if isinstance(dphi, Quantity)
+           else float(np.radians(dphi)))
+    if not 0.0 < rad < np.pi / 2:
+        raise ValueError(f'dphi = {dphi}: the cone half-angle must be finite, > 0 and < 90 deg')
+    return rad
+
+
 def compute_iteration(self, outputfile, scdata, delay=False):
     """One output file against all spectra (reference compute_iteration.py:90-240).  The
     packets are the Output's resident table (the rows the reference reads back from its
@@ -148,6 +159,7 @@ def compute_iteration(self, outputfile, scdata, delay=False):
 class LOSResult(ModelResult):
     def __init__(self, scdata, inputs, params=None, dphi=Quantity(1., 'deg'), device=None,
                  **kwargs):
+        dphi = cone_half_angle(dphi)
         if params is None:
             params = {'quantity': 'radiance'}
         scdata.set_frame('Model')
@@ -155,8 +167,7 @@ class LOSResult(ModelResult):
         self.species = scdata.species
         self.query = scdata.query
         self.type = 'LineOfSight'
-        self.dphi = (float(dphi.to('rad').value) if isinstance(dphi, Quantity)
-                     else float(np.radians(dphi)))
+        self.dphi = dphi
         self._oedge = np.min([self.inputs.options.outeredge * 2, 100])
         self.fitted = self.inputs.options.fitted
         nspec = len(scdata)

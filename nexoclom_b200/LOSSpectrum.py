@@ -34,7 +34,7 @@ import pandas as pd
 
 from . import catalogue
 from .engine import get_engine
-from .LOSResult import dist_from_planet_cut
+from .LOSResult import cone_half_angle, dist_from_planet_cut
 from .ModelResult import ModelResult
 from .runsetup import get_setup
 from .sharding import combine_ranks, local_device
@@ -76,13 +76,13 @@ class LOSSpectrum(ModelResult):
             raise ValueError("LOSSpectrum computes quantity = 'radiance' only")
         nspec = len(scdata)
         vmin, vmax, nbins = velocity_bins(velocity, nspec)
+        dphi = cone_half_angle(dphi)
         scdata.set_frame('Model')
         super().__init__(inputs, params)
         self.type = 'LineOfSightSpectrum'
         self.species = scdata.species
         self.query = scdata.query
-        self.dphi = (float(dphi.to('rad').value) if isinstance(dphi, Quantity)
-                     else float(np.radians(dphi)))
+        self.dphi = dphi
         self._device = local_device() if device is None else device
         self.edges = np.linspace(vmin, vmax, nbins + 1)
         self.velocity = 0.5 * (self.edges[:-1] + self.edges[1:])

@@ -1513,66 +1513,32 @@ int nx_image_accumulate(nx_ctx* ctx, long long n, const nx_image_params* ip, dou
   return r;
 }
 
-// Per-LOS ladder length and the shared geometric ladder (compute_iteration.py:158-171).
-// Constants of a line-of-sight call and the ladder of KD-ball centres (compute_iteration.py:
-// 151-170), given the longest boresight distance `ddmax` to the outer edge.
-static void los_constants(const LosParams& lp, double ddmax, std::vector<double>& ladder,
-                          std::vector<double>& wid2, LosConsts& lc) {
-  const double s = std::sin(lp.dphi);
-  const double s2 = std::sin(lp.dphi * 2);
-  ladder.clear();
-  ladder.push_back(s);
-  while (ladder.back() < ddmax && ladder.size() < (1u << 20)) {
-    const double t = ladder.back();
-    ladder.push_back(t + t * s);
-  }
-  wid2.resize(ladder.size());
-  for (size_t k = 0; k < ladder.size(); ++k) { const double w = ladder[k] * s2; wid2[k] = w * w; }
-  lc.sin_dphi = s;
-  const double cd = std::cos(lp.dphi);
-  lc.cos_margin2 = (cd * (1 - 1e-9)) * (cd * (1 - 1e-9));
-  lc.cos_loose2 = (cd * (1 - 1e-6)) * (cd * (1 - 1e-6));
-  lc.cos_accept2 = (cd * (1 + 1e-9)) * (cd * (1 + 1e-9));
-  // nearest ball centre is <= t_k s/2 away along the axis, the cone is <= t_k (1+s) tan(dphi)
-  // wide there, the ball radius is t_k sin(2 dphi): covered if the sum of squares fits with
-  // 10 % to spare
-  const double td = std::tan(lp.dphi);
-  lc.cover = (0.25 * s * s + (1 + s) * (1 + s) * td * td <= 0.9 * s2 * s2) ? 1 : 0;
-  lc.inv_log_ratio = 1.0 / std::log1p(s);
-  lc.log_t0 = std::log(s);
-  const double w1 = std::log1p(s2) * lc.inv_log_ratio;
-  const double w2 = -std::log1p(-s2) * lc.inv_log_ratio;
-  lc.kwin = (int)std::ceil(w1 > w2 ? w1 : w2) + 2;
-  lc.nladder = (int)ladder.size();
+// Line-of-sight parameters every K5 entry point checks before any device work.
+static int check_los_params(nx_ctx* ctx, const LosParams& lp) {
+  const std::string e = los_dphi_error(lp.dphi);
+  if (!e.empty()) { ctx->err = e; return -1; }
+  if (lp.quantity != 1) { ctx->err = "Other quantities not set up."; return -1; }   // compute_iteration.py:213
+  if (ctx->gtables.n == 0) { ctx->err = "no g-value tables uploaded"; return -1; }
+  return 0;
 }
 
-// Host version of the per-line preparation (nx_los_used; the accumulate calls do the same on
-// the device: k_los_prepare / k_los_finish in nx_los_grid.cu).
-static void los_prepare(const double* los, long long nlos, const LosParams& lp,
-                        std::vector<int>& nball, std::vector<double>& ladder,
-                        std::vector<double>& wid2, LosConsts& lc) {
-  std::vector<double> dd(nlos);
-  double ddmax = 0.0;
-  for (long long i = 0; i < nlos; ++i) {
-    const double x = los[i], y = los[nlos + i], z = los[2 * nlos + i];
-    const double bx = los[3 * nlos + i], by = los[4 * nlos + i], bz = los[5 * nlos + i];
-    const double b = 2 * ((x * bx + y * by) + z * bz);
-    const double nrm = std::sqrt((x * x + y * y) + z * z);
-    const double c = nrm * nrm - lp.outeredge * lp.outeredge;
-    dd[i] = (-b + std::sqrt(b * b - 4 * 1 * c)) / 2;
-    if (dd[i] > ddmax) ddmax = dd[i];
+// The ladder, then the squared ball radii, into d_dst (2 * ladder.size() doubles) through the
+// context's pinned staging, at most NX_LADDER_STAGE bytes at a time: a ladder of millions of
+// entries (arcsecond cones) does not grow the staging buffer.
+#define NX_LADDER_STAGE ((size_t)4 << 20)
+static int stage_ladder(nx_ctx* ctx, double* d_dst, const std::vector<double>& ladder,
+                        const std::vector<double>& wid2) {
+  const size_t nl = ladder.size(), total = 2 * nl, per = NX_LADDER_STAGE / sizeof(double);
+  { int r0 = pinned_staging(ctx, (total < per ? total : per) * sizeof(double)); if (r0) return r0; }
+  double* st = static_cast<double*>(ctx->pinned);
+  for (size_t a = 0; a < total; a += per) {
+    const size_t b = total - a < per ? total : a + per;
+    // the previous chunk has left the staging buffer (the stream is idle on the first one)
+    if (a) CK(cudaStreamSynchronize(ctx->stream));
+    for (size_t i = a; i < b; ++i) st[i - a] = i < nl ? ladder[i] : wid2[i - nl];
+    CK(cudaMemcpyAsync(d_dst + a, st, (b - a) * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
   }
-  los_constants(lp, ddmax, ladder, wid2, lc);
-  nball.resize(nlos);
-  for (long long i = 0; i < nlos; ++i) {
-    // first k with t_k >= dd is the last ladder entry; NaN dd -> single entry
-    int k = 0;
-    if (dd[i] == dd[i]) {
-      k = (int)(std::lower_bound(ladder.begin(), ladder.end(), dd[i]) - ladder.begin());
-      if (k >= (int)ladder.size()) k = (int)ladder.size() - 1;
-    }
-    nball[i] = k + 1;
-  }
+  return 0;
 }
 
 static int los_run(nx_ctx* ctx, long long n, long long nlos, const double* los_dev,
@@ -1610,15 +1576,10 @@ static int los_run(nx_ctx* ctx, long long n, long long nlos, const double* los_d
   CK(cudaStreamSynchronize(ctx->stream));
   std::vector<double> ladder, wid2;
   LosConsts lc;
-  los_constants(lp, ddmax, ladder, wid2, lc);
-  // ladder + wid2 through the context's pinned staging: the copies outlive this scope's vectors
-  { int r0 = pinned_staging(ctx, 2 * ladder.size() * sizeof(double)); if (r0) return r0; }
-  double* st_ladder = static_cast<double*>(ctx->pinned);
-  std::memcpy(st_ladder, ladder.data(), ladder.size() * sizeof(double));
-  std::memcpy(st_ladder + ladder.size(), wid2.data(), wid2.size() * sizeof(double));
+  { const std::string e = los_constants(lp, ddmax, ladder, wid2, lc); if (!e.empty()) { ctx->err = e; return -1; } }
   SCR(SCR_LADDER, d_ladder, 2 * ladder.size());
   d_wid2 = d_ladder + ladder.size();
-  CK(cudaMemcpyAsync(d_ladder, st_ladder, 2 * ladder.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+  { int r0 = stage_ladder(ctx, d_ladder, ladder, wid2); if (r0) return r0; }
   CK(launch_los_finish(ctx->stream, d_dd, d_ladder, (int)ladder.size(), nlos, d_nball, d_key, d_hist,
                        d_order));
   ctx->launches += want_order ? 3 : 2;
@@ -1664,8 +1625,7 @@ int nx_los_accumulate_dev(nx_ctx* ctx, long long n, long long nlos, void* los_de
   if (n > resident_rows(ctx)) { ctx->err = "n exceeds resident packets"; return -1; }
   LosParams lp;
   std::memcpy(&lp, lp_, sizeof(lp));
-  if (lp.quantity != 1) { ctx->err = "Other quantities not set up."; return -1; }   // compute_iteration.py:213
-  if (ctx->gtables.n == 0) { ctx->err = "no g-value tables uploaded"; return -1; }
+  { int r0 = check_los_params(ctx, lp); if (r0) return r0; }
   if (n == 0 || nlos == 0) return 0;
   return los_run(ctx, n, nlos, (const double*)los_dev, (const double*)dist_dev, lp,
                  (double*)radiance_dev, (unsigned long long*)npackets_dev,
@@ -1679,8 +1639,7 @@ int nx_los_accumulate(nx_ctx* ctx, long long n, long long nlos, const double* lo
   if (n > resident_rows(ctx)) { ctx->err = "n exceeds resident packets"; return -1; }
   LosParams lp;
   std::memcpy(&lp, lp_, sizeof(lp));
-  if (lp.quantity != 1) { ctx->err = "Other quantities not set up."; return -1; }
-  if (ctx->gtables.n == 0) { ctx->err = "no g-value tables uploaded"; return -1; }
+  { int r0 = check_los_params(ctx, lp); if (r0) return r0; }
   double *d_los = nullptr, *d_dist = nullptr, *d_rad = nullptr;
   unsigned long long* d_np = nullptr;
   unsigned char* d_inc = nullptr;
@@ -1721,8 +1680,7 @@ int nx_los_accumulate_counted(nx_ctx* ctx, long long n, long long nlos, const do
   if (n >= (1LL << 32)) { ctx->err = "more than 2^32 packets per GPU"; return -1; }
   LosParams lp;
   std::memcpy(&lp, lp_, sizeof(lp));
-  if (lp.quantity != 1) { ctx->err = "Other quantities not set up."; return -1; }
-  if (ctx->gtables.n == 0) { ctx->err = "no g-value tables uploaded"; return -1; }
+  { int r0 = check_los_params(ctx, lp); if (r0) return r0; }
   double *d_los = nullptr, *d_dist = nullptr, *d_rad = nullptr;
   unsigned long long *d_np = nullptr, *d_nused = nullptr;
   unsigned char* d_inc = nullptr;
@@ -1762,6 +1720,7 @@ int nx_los_used_fill(nx_ctx* ctx, long long n, long long nlos, const double* los
   if (!used_offsets || !used_indices) { ctx->err = "nx_los_used_fill: null argument"; return -1; }
   LosParams lp;
   std::memcpy(&lp, lp_, sizeof(lp));
+  { const std::string e = los_dphi_error(lp.dphi); if (!e.empty()) { ctx->err = e; return -1; } }
   const nx_ctx::LosKept k = ctx->los_kept;
   const bool reuse = k.np > 0 && k.n == n && k.nlos == nlos && k.bound == ctx->bound &&
                      std::memcmp(&k.lp, &lp, sizeof(lp)) == 0;
@@ -1802,8 +1761,7 @@ int nx_los_used(nx_ctx* ctx, long long n, long long nlos, const double* los,
   if (n > resident_rows(ctx)) { ctx->err = "n exceeds resident packets"; return -1; }
   LosParams lp;
   std::memcpy(&lp, lp_, sizeof(lp));
-  if (lp.quantity != 1) { ctx->err = "Other quantities not set up."; return -1; }
-  if (ctx->gtables.n == 0) { ctx->err = "no g-value tables uploaded"; return -1; }
+  { int r0 = check_los_params(ctx, lp); if (r0) return r0; }
   if (nlos <= 0) return 0;
   if (n <= 0) { for (long long i = 0; i < nlos; ++i) used_count[i] = 0; return 0; }
   if (n >= (1LL << 32)) { ctx->err = "more than 2^32 packets per GPU"; return -1; }
@@ -1811,7 +1769,7 @@ int nx_los_used(nx_ctx* ctx, long long n, long long nlos, const double* los,
   std::vector<int> nball;
   std::vector<double> ladder, wid2;
   LosConsts lc;
-  los_prepare(los, nlos, lp, nball, ladder, wid2, lc);
+  { const std::string e = los_prepare(los, nlos, lp, nball, ladder, wid2, lc); if (!e.empty()) { ctx->err = e; return -1; } }
   const long long total = used_indices ? used_offsets[nlos] : 0;
   double *d_los = nullptr, *d_dist = nullptr, *d_ladder = nullptr, *d_wid2 = nullptr;
   int* d_nball = nullptr;
@@ -1881,8 +1839,7 @@ int nx_los_spectrum(nx_ctx* ctx, long long n, long long nlos, const double* los,
   }
   LosParams lp;
   std::memcpy(&lp, lp_, sizeof(lp));
-  if (lp.quantity != 1) { ctx->err = "Other quantities not set up."; return -1; }
-  if (ctx->gtables.n == 0) { ctx->err = "no g-value tables uploaded"; return -1; }
+  { int r0 = check_los_params(ctx, lp); if (r0) return r0; }
   const size_t ncell = (size_t)(nlos * ncol);
   if (nlos == 0) return 0;
   if (!los || !dist_from_plan || !spectrum || !counts) { ctx->err = "nx_los_spectrum: null argument"; return -1; }

@@ -5,6 +5,7 @@
 
 #include "nx_image.cuh"
 #include "nx_init.cuh"
+#include "nx_los.h"
 #include "nx_physics.cuh"
 #include "nx_surface.cuh"
 
@@ -35,18 +36,6 @@ struct RowSink {
   unsigned long long cap;
   size_t stride;
   int skip_dead, to_f32;
-};
-
-struct LosConsts {
-  double sin_dphi;
-  double cos_margin2;     // (cos(dphi) (1 - 1e-9))^2   conservative reject, exact-order path
-  double cos_loose2;      // (cos(dphi) (1 - 1e-6))^2   conservative reject, FMA path
-  double cos_accept2;     // (cos(dphi) (1 + 1e-9))^2   sure accept, no acos needed
-  int cover;              // 1: in-cone points between the first and last ball centre are in a ball
-  double inv_log_ratio;   // 1 / log(1 + sin dphi)
-  double log_t0;          // log(sin dphi)
-  int kwin;
-  int nladder;
 };
 
 // ---- K5 spatial culling (nx_los_grid.cu) ----
