@@ -221,7 +221,7 @@ int nx_integrate_adaptive_bounce(nx_ctx* ctx, long long n, uint64_t seed, uint64
                                  unsigned long long* accepted_steps,
                                  unsigned long long* bounces);
 
-/* ---- context-owned accumulators (image, cube, deposition, ion production) ------------------
+/* ---- context-owned accumulators (image, cube, deposition, ion production, trajectory) -----
  * Each product below sums on the device into its own accumulator of `nsum` f64 sums and
  * `ncount` i64 counts (the product states the shape), so one product's calls leave the others
  * alone.  Its begin validates the shape and zeroes the accumulator (the device block is reused
@@ -238,7 +238,8 @@ typedef enum {
   NX_PRODUCT_IMAGE = 0,
   NX_PRODUCT_CUBE = 1,
   NX_PRODUCT_DEPOSIT = 2,
-  NX_PRODUCT_IONIZE = 3
+  NX_PRODUCT_IONIZE = 3,
+  NX_PRODUCT_TRACE = 4
 } nx_product;
 int nx_product_fetch(nx_ctx* ctx, nx_product which, double* sums, long long* counts);
 int nx_product_device_ptrs(nx_ctx* ctx, nx_product which, void** sums, void** counts);
@@ -312,6 +313,41 @@ int nx_integrate_adaptive_ionize(nx_ctx* ctx, long long n, uint64_t seed, uint64
                                  unsigned long long* attempted_steps,
                                  unsigned long long* accepted_steps,
                                  unsigned long long* bounces);
+
+/* ---- K2t: images and density grids from every accepted step (ModelTrajectoryImage,
+ * ModelTrajectoryDensity) -------------------------------------------------------------------
+ * An extension (the reference has no such product).  nx_integrate_adaptive_trace runs the
+ * adaptive driver on the resident packets exactly as nx_integrate_adaptive_ionize would (the
+ * same preconditions, the same kernel choice: perfect sticking or bounce, deviates keyed by
+ * seed / first_id, the same final state and step totals), and adds every accepted step to the
+ * image and / or grid of nx_trace_begin.  With T = endtime, t0 the packet's time remaining when
+ * the kernel loads it (its release time in an imported or K1 X0), t the time remaining before
+ * the step, h the step, and every operation an f64 op rounded to nearest:
+ *   midpoint   m = (s + s_rk) * 0.5 per component, s the state before the step, s_rk the
+ *              Runge-Kutta state before any surface, moon, escape or vanish handling
+ *   dwell      a = (h * T) / ((T - t0) + (t - 0.5 * h)): the step's length over the chance
+ *              (T - age) / T that a packet released uniformly in (0, T] is still in flight at
+ *              the midpoint's age, so the sums estimate the steady state the snapshot does
+ *   image      K4's pixel and weight w of m (nx_image_accumulate with round_f32 = 0; w carries
+ *              m's frac, and the sunlit mask and g-values for radiance): w * a and one count
+ *   grid       m's position binned as in nx_ionize_begin: frac(m) * a and one count, OUTSIDE
+ *              for a midpoint outside the box or NaN
+ * ModelImage's image is sums * atoms_per_packet; this image is sums * atoms_per_packet / T
+ * with the same expectation.  A step is represented by its midpoint (not split over the pixels
+ * or cells its chord crosses); a step that ends inside the planet counts its full h.
+ * The sink is the NX_PRODUCT_TRACE accumulator, nsum = ncount = (image ? nx * nz : 0) + (grid ?
+ * gx * gy * gz + 1 : 0): the pixels (ix * nz + iz), then the grid's cells (row-major) and
+ * OUTSIDE, each an f64 sum and a count of recorded steps.  begin takes either or both (NULL:
+ * none; both NULL is -1), validates the image (nx, nz >= 1, x0 < x1 and z0 < z1 finite, apix >
+ * 0, quantity 0 or 1) and the grid as nx_ionize_begin does, and keeps copies of both.
+ * nx_integrate_adaptive_trace returns -1 for a run with moons (the forces then depend on the
+ * time, so a step's sample is not the snapshot's state) and for a radiance image without
+ * g-value tables.  Every recorded step is one f64 and one u64 atomic add per product.       */
+int nx_trace_begin(nx_ctx* ctx, const nx_image_params* image, const nx_ion_grid* grid);
+int nx_integrate_adaptive_trace(nx_ctx* ctx, long long n, uint64_t seed, uint64_t first_id,
+                                unsigned long long* attempted_steps,
+                                unsigned long long* accepted_steps,
+                                unsigned long long* bounces);
 
 /* ---- K3: constant-step driver with bounce (Output.py:368-455, bouncepackets.py)
  * Optional fused per-step image accumulation (image_dev / counts_dev device

@@ -3,7 +3,7 @@
 Public API mirrors the reference's ``nexoclom/__init__.py:9-14``.  Importing the
 package needs neither PostgreSQL nor astropy; creating an ``Output`` /
 ``ModelImage`` / ``ModelImageCube`` / ``ModelDensity`` / ``ModelDeposition`` /
-``ModelIonization`` / ``LOSResult`` /
+``ModelIonization`` / ``ModelTrajectoryImage`` / ``ModelTrajectoryDensity`` / ``LOSResult`` /
 ``LOSSpectrum`` needs the built CUDA library and a
 GPU (there is no CPU fallback).
 """
@@ -14,6 +14,7 @@ from .ModelImageCube import ModelImageCube
 from .ModelDensity import ModelDensity
 from .ModelDeposition import ModelDeposition
 from .ModelIonization import ModelIonization
+from .ModelTrajectory import ModelTrajectoryImage, ModelTrajectoryDensity
 from .LOSResult import LOSResult
 from .LOSSpectrum import LOSSpectrum
 from .LOSResultFitted import LOSResultFitted
@@ -21,5 +22,5 @@ from .solarsystem import SSObject
 from .input_classes import InputError
 
 __all__ = ['Input', 'Output', 'ModelImage', 'ModelImageCube', 'ModelDensity', 'ModelDeposition',
-           'ModelIonization', 'LOSResult', 'LOSSpectrum', 'LOSResultFitted', 'SSObject', 'InputError']
+           'ModelIonization', 'ModelTrajectoryImage', 'ModelTrajectoryDensity', 'LOSResult', 'LOSSpectrum', 'LOSResultFitted', 'SSObject', 'InputError']
 __version__ = '0.1.0'

@@ -18,7 +18,7 @@ c_u32_p = C.POINTER(C.c_uint32)
 c_u8_p = C.POINTER(C.c_uint8)
 
 # nx_product: the context-owned accumulators
-NX_PRODUCT_IMAGE, NX_PRODUCT_CUBE, NX_PRODUCT_DEPOSIT, NX_PRODUCT_IONIZE = 0, 1, 2, 3
+NX_PRODUCT_IMAGE, NX_PRODUCT_CUBE, NX_PRODUCT_DEPOSIT, NX_PRODUCT_IONIZE, NX_PRODUCT_TRACE = range(5)
 
 
 class RunParams(C.Structure):
@@ -175,6 +175,9 @@ def load():
         'nx_integrate_adaptive_deposit': [vp, i64, u64, u64, C.POINTER(u64), C.POINTER(u64),
                                           C.POINTER(u64)],
         'nx_ionize_begin': [vp, C.POINTER(IonGrid)],
+        'nx_trace_begin': [vp, C.POINTER(ImageParams), C.POINTER(IonGrid)],
+        'nx_integrate_adaptive_trace': [vp, i64, u64, u64, C.POINTER(u64), C.POINTER(u64),
+                                        C.POINTER(u64)],
         'nx_integrate_adaptive_ionize': [vp, i64, u64, u64, C.POINTER(u64), C.POINTER(u64),
                                          C.POINTER(u64)],
         'nx_product_fetch': [vp, C.c_int, c_double_p, c_i64_p],

@@ -135,8 +135,12 @@ struct nx_ctx {
   // cudaFree (an implicit device synchronisation each) on the calls LOSResult / ModelImage
   // make once per output file, and nothing to leak on an error path
   struct Scratch { void* p = nullptr; size_t bytes = 0; } scr[32];
-  Accum accum[NX_PRODUCT_IONIZE + 1];    // one per nx_product
+  Accum accum[NX_PRODUCT_TRACE + 1];     // one per nx_product
   IonOut ion_axes{};                     // the grid of nx_ionize_begin (axes only)
+  // nx_trace_begin's image (trace_npix > 0) and grid (trace_grid.n[0] > 0, axes only)
+  ImageParams trace_ip{};
+  long long trace_npix = 0;
+  IonOut trace_grid{};
   void* pinned = nullptr;      // grow-only pinned staging for small D2H results (image, LOS columns)
   size_t pinned_bytes = 0;
   unsigned* cmp_tiles = nullptr;     // compaction scratch (tile counts)
@@ -318,15 +322,16 @@ static int pinned_staging(nx_ctx* ctx, size_t bytes) {
   return 0;
 }
 
-// ---- context-owned accumulators (image, cube, deposition, ion production) -------------------
+// ---- context-owned accumulators (image, cube, deposition, ion production, trajectory) -------
 // None of these calls ENTER: nothing here changes what the line-of-sight kernels read, so the
 // candidate pairs nx_los_accumulate_counted keeps stay valid.
 static const char* const accum_begin_name[] = {"nx_image_begin", "nx_cube_begin",
-                                               "nx_deposit_begin", "nx_ionize_begin"};
+                                               "nx_deposit_begin", "nx_ionize_begin",
+                                               "nx_trace_begin"};
 
 // The accumulator of `which` when its begin has run; else NULL with the error set.
 static Accum* accum_of(nx_ctx* ctx, int which) {
-  if (which < NX_PRODUCT_IMAGE || which > NX_PRODUCT_IONIZE) {
+  if (which < NX_PRODUCT_IMAGE || which > NX_PRODUCT_TRACE) {
     ctx->err = "unknown nx_product";
     return nullptr;
   }
@@ -928,10 +933,11 @@ static int check_status(nx_ctx* ctx) {
 // S != nullptr: packets bounce (nx_integrate_adaptive_bounce); the cost model then budgets
 // every packet's remaining time, since reaching the surface no longer ends its flight.
 // dep != nullptr: the SINK build of the same kernel (nx_integrate_adaptive_deposit);
-// ion != nullptr: its ion build (nx_integrate_adaptive_ionize).
+// ion != nullptr: its ion build (nx_integrate_adaptive_ionize); trace != nullptr: its trace
+// build (nx_integrate_adaptive_trace).
 static int adaptive_resident(nx_ctx* ctx, long long n, const Spline2D* S, uint64_t seed,
                              uint64_t first_id, const DepositOut* dep = nullptr,
-                             const IonOut* ion = nullptr) {
+                             const IonOut* ion = nullptr, const TraceOut* trace = nullptr) {
   const bool order = ctx->order_packets && n >= 4096;
   const bool to_surface = !S || perfect_sticking(ctx->params);
   if (order)
@@ -941,7 +947,8 @@ static int adaptive_resident(nx_ctx* ctx, long long n, const Spline2D* S, uint64
                                ctx->params,
                                ctx->radpres.view, ctx->radpres.fast,
                                order ? ctx->perm : nullptr, ctx->scalars, ctx->scalars + 1,
-                               ctx->att, ctx->acc, ctx->status, S, seed, first_id, dep, ion));
+                               ctx->att, ctx->acc, ctx->status, S, seed, first_id, dep, ion,
+                               trace));
   return end_timed(ctx, order ? 4 : 1);
 }
 
@@ -1095,26 +1102,37 @@ int nx_integrate_adaptive_deposit(nx_ctx* ctx, long long n, uint64_t seed, uint6
 // resident packets: the same final state and step totals, plus the loss added to the grid.
 static_assert(sizeof(nx_ion_grid) == 64, "nx_ion_grid layout");
 
-int nx_ionize_begin(nx_ctx* ctx, const nx_ion_grid* grid) {
-  CK(cudaSetDevice(ctx->device));
-  if (!grid) { ctx->err = "nx_ionize_begin: grid is NULL"; return -1; }
+// The axes of a valid grid in *g (cells + OUTSIDE in *nslot); -1 with the error set, naming
+// the caller `who`, otherwise.
+static int ion_grid_axes(nx_ctx* ctx, const char* who, const nx_ion_grid* grid, IonOut* g,
+                         long long* nslot) {
+  const std::string name(who);
+  if (!grid) { ctx->err = name + ": grid is NULL"; return -1; }
   double ncell = 1.0;
   for (int a = 0; a < 3; ++a) {
-    if (grid->n[a] < 1) { ctx->err = "nx_ionize_begin: n must be >= 1 on every axis"; return -1; }
+    if (grid->n[a] < 1) { ctx->err = name + ": n must be >= 1 on every axis"; return -1; }
     if (!(std::isfinite(grid->lo[a]) && std::isfinite(grid->hi[a]) && grid->lo[a] < grid->hi[a])) {
-      ctx->err = "nx_ionize_begin: lo < hi, both finite, on every axis";
+      ctx->err = name + ": lo < hi, both finite, on every axis";
       return -1;
     }
     ncell *= grid->n[a];
   }
   if (ncell + 1.0 >= 2147483648.0) {
-    ctx->err = "nx_ionize_begin: nx * ny * nz + 1 must be < 2^31";
+    ctx->err = name + ": nx * ny * nz + 1 must be < 2^31";
     return -1;
   }
-  IonOut g{};
-  for (int a = 0; a < 3; ++a) { g.lo[a] = grid->lo[a]; g.hi[a] = grid->hi[a]; g.n[a] = grid->n[a]; }
-  ion_steps(g);
-  const long long n = (long long)ncell + 1;
+  *g = IonOut{};
+  for (int a = 0; a < 3; ++a) { g->lo[a] = grid->lo[a]; g->hi[a] = grid->hi[a]; g->n[a] = grid->n[a]; }
+  ion_steps(*g);
+  *nslot = (long long)ncell + 1;
+  return 0;
+}
+
+int nx_ionize_begin(nx_ctx* ctx, const nx_ion_grid* grid) {
+  CK(cudaSetDevice(ctx->device));
+  IonOut g;
+  long long n = 0;
+  if (ion_grid_axes(ctx, "nx_ionize_begin", grid, &g, &n)) return -1;
   int r = accum_begin(ctx, NX_PRODUCT_IONIZE, n, n, g.n[0], g.n[1], g.n[2]);
   if (r == 0) ctx->ion_axes = g;
   return r;
@@ -1148,6 +1166,105 @@ int nx_integrate_adaptive_ionize(nx_ctx* ctx, long long n, uint64_t seed, uint64
     if ((r = begin_timed(ctx))) return r;
     if ((r = adaptive_resident(ctx, n, bounce ? &ctx->spline : nullptr, seed, first_id, nullptr,
                                &g)))
+      return r;
+    ctx->fresh = false;
+  }
+  unsigned long long h[4] = {0, 0, 0, 0};
+  CK(cudaMemcpyAsync(h, ctx->scalars, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
+  r = check_status(ctx);
+  if (r < 0) return r;
+  if (attempted) *attempted = h[1];
+  if (accepted) *accepted = h[2];
+  if (bounces) *bounces = h[3];
+  return r;
+}
+
+// ---- K2t: images and density grids from every accepted step ----------------------------------
+// The sink is the NX_PRODUCT_TRACE accumulator: the image's pixels (ix * nz + iz), then the
+// grid's cells, row-major (nx, ny, nz), and OUTSIDE, in the sums and in the counts.
+// nx_integrate_adaptive_trace runs k_trace_adaptive, the build of the kernel
+// nx_integrate_adaptive (perfect sticking) or nx_integrate_adaptive_bounce would run, on the
+// resident packets: the same final state and step totals, plus every accepted step added to the
+// image and / or the grid.
+int nx_trace_begin(nx_ctx* ctx, const nx_image_params* image, const nx_ion_grid* grid) {
+  CK(cudaSetDevice(ctx->device));
+  if (!image && !grid) { ctx->err = "nx_trace_begin: neither an image nor a grid"; return -1; }
+  ImageParams ip{};
+  long long npix = 0;
+  if (image) {
+    std::memcpy(&ip, image, sizeof(ip));
+    if (ip.nx < 1 || ip.nz < 1 || (double)ip.nx * ip.nz >= 1073741824.0) {
+      ctx->err = "nx_trace_begin: image dims must be >= 1 and nx * nz < 2^30";
+      return -1;
+    }
+    if (!(std::isfinite(ip.x0) && std::isfinite(ip.x1) && ip.x0 < ip.x1 && std::isfinite(ip.z0) &&
+          std::isfinite(ip.z1) && ip.z0 < ip.z1)) {
+      ctx->err = "nx_trace_begin: image range x0 < x1, z0 < z1, all finite";
+      return -1;
+    }
+    if (!(ip.apix > 0.0 && std::isfinite(ip.apix))) {
+      ctx->err = "nx_trace_begin: apix must be finite and > 0";
+      return -1;
+    }
+    if (ip.quantity != 0 && ip.quantity != 1) {
+      ctx->err = "nx_trace_begin: quantity must be 0 (column) or 1 (radiance)";
+      return -1;
+    }
+    npix = (long long)ip.nx * ip.nz;
+  }
+  IonOut g{};
+  long long nslot = 0;
+  if (grid && ion_grid_axes(ctx, "nx_trace_begin", grid, &g, &nslot)) return -1;
+  const long long n = npix + nslot;
+  int r = accum_begin(ctx, NX_PRODUCT_TRACE, n, n, ip.nx, ip.nz, grid ? 1 : 0);
+  if (r == 0) { ctx->trace_ip = ip; ctx->trace_npix = npix; ctx->trace_grid = g; }
+  return r;
+}
+
+int nx_integrate_adaptive_trace(nx_ctx* ctx, long long n, uint64_t seed, uint64_t first_id,
+                                unsigned long long* attempted, unsigned long long* accepted,
+                                unsigned long long* bounces) {
+  ENTER(ctx);
+  const Accum* sink = accum_of(ctx, NX_PRODUCT_TRACE);
+  if (!sink) return -1;
+  if (!ctx->have_params) { ctx->err = "nx_tables_upload not called"; return -1; }
+  ctx->bound = nullptr;            // integrators work on the slab
+  if (n < 0 || n > ctx->cap) { ctx->err = "n exceeds resident packets"; return -1; }
+  const RunParams& p = ctx->params;
+  if (p.nmoons != 0) {
+    ctx->err = "nx_integrate_adaptive_trace: runs with moons are not supported (the forces "
+               "depend on the time, a step's sample is not the snapshot's state)";
+    return -1;
+  }
+  if (ctx->trace_npix > 0 && ctx->trace_ip.quantity == 1 && ctx->gtables.n == 0) {
+    ctx->err = "radiance image requested but no g-value tables uploaded";
+    return -1;
+  }
+  const bool bounce = !perfect_sticking(p);
+  if (bounce && p.accomfactor != 0.0 && !ctx->spl_c) {
+    ctx->err = "accommodation enabled but no speed spline uploaded";
+    return -1;
+  }
+  CK(cudaMemsetAsync(ctx->scalars, 0, 8 * sizeof(unsigned long long), ctx->stream));
+  int r;
+  if (n > 0) {
+    TraceOut t{};
+    if (ctx->trace_npix > 0) {
+      t.img_sum = sink->sums();
+      t.img_cnt = sink->counts();
+      t.ip = ctx->trace_ip;
+      t.is = image_steps(t.ip);
+      t.G = ctx->gtables;
+    }
+    if (ctx->trace_grid.n[0] > 0) {
+      t.grid = ctx->trace_grid;
+      t.grid.sum = sink->sums() + ctx->trace_npix;
+      t.grid.cnt = sink->counts() + ctx->trace_npix;
+    }
+    t.endtime = p.endtime;
+    if ((r = begin_timed(ctx))) return r;
+    if ((r = adaptive_resident(ctx, n, bounce ? &ctx->spline : nullptr, seed, first_id, nullptr,
+                               nullptr, &t)))
       return r;
     ctx->fresh = false;
   }

@@ -204,6 +204,64 @@ NX_HD int image_packet_fast(const ImageParams& ip, const GTables& G, const Image
   return ix * ip.nz + iz;
 }
 
+// The trajectory sink of one launch (k_trace_adaptive, a __grid_constant__ kernel parameter
+// the lanes read through TraceSink::o): the image (img_sum == nullptr: none) with K4's
+// parameters and g-value tables (their records stay in global memory), and the grid
+// (grid.sum == nullptr: none), whose OUTSIDE slot is index n[0] * n[1] * n[2].
+struct TraceOut {
+  double* img_sum;
+  unsigned long long* img_cnt;
+  ImageParams ip;
+  ImageSteps is;
+  GTables G;
+  IonOut grid;
+  double endtime;           // T
+};
+
+// One accepted step of the trajectory sink (declared in nx_physics.cuh).  The dwell of the
+// step, weighted by the inverse probability that a packet of its age is still in flight,
+//   a = (h * T) / (age0 + (t - 0.5 * h)),   age0 = T - t0,
+// every operation an f64 op rounded to nearest (both terms of the sum are >= 0, the second
+// > 0).  The image adds w * a at the midpoint's pixel, w being K4's weight of the midpoint
+// (image_packet_fast, which carries the frac), and one count; the grid adds frac * a at the
+// midpoint's cell (ion_cell) and one count, or to the lane's OUTSIDE share.
+template <class Sink>
+NX_COLD void trace_record(Sink& Tr, double x, double y, double z, double vy, double frac,
+                          double h, double t) {
+  const TraceOut& o = *Tr.o;
+  const double a = div_rn(mul_rn(h, o.endtime), add_rn(Tr.age0, sub_rn(t, mul_rn(0.5, h))));
+  if (o.img_sum) {
+    double w;
+    const int pix = image_packet_fast(o.ip, o.G, o.is, x, y, z, vy, frac, w);
+    if (pix >= 0) {
+      const double v = mul_rn(w, a);
+#if defined(__CUDA_ARCH__)
+      if (v != 0.0) atomicAdd(o.img_sum + pix, v);
+      atomicAdd(o.img_cnt + pix, 1ull);
+#else
+      o.img_sum[pix] += v;
+      o.img_cnt[pix] += 1;
+#endif
+    }
+  }
+  if (o.grid.sum) {
+    const double d = mul_rn(frac, a);
+    const long long c = ion_cell(o.grid, x, y, z);
+    if (c < 0) {
+      Tr.out_sum += d;
+      Tr.out_n += 1;
+      return;
+    }
+#if defined(__CUDA_ARCH__)
+    atomicAdd(o.grid.sum + c, d);
+    atomicAdd(o.grid.cnt + c, 1ull);
+#else
+    o.grid.sum[c] += d;
+    o.grid.cnt[c] += 1;
+#endif
+  }
+}
+
 // ---------------------------------------------------------------------------
 // Lines of sight
 // ---------------------------------------------------------------------------

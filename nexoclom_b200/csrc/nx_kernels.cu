@@ -304,15 +304,21 @@ struct PacketFeeder {
 // ION: the ion-production sink (ModelIonization, k_ionize_adaptive): the attempts record the
 // frac every accepted step loses in flight (ion_record), each lane its OUTSIDE share, reduced
 // here; Ion is unused otherwise.  The final state and the step totals are again unchanged.
-// The persistent lane loop of both kernels (feeder, refill, step totals), inlined into each.
-template <int MODE, bool BOUNCE, bool SINK, bool ION>
+// TRACE: the trajectory sink (ModelTrajectoryImage / ModelTrajectoryDensity,
+// k_trace_adaptive): the lane keeps T - t0 of its packet from the moment it loads it, the
+// attempts record every accepted step (trace_record) into *Tro, each lane its OUTSIDE share of
+// the grid, reduced here; Tro is unused otherwise.  The final state and the step totals are
+// again unchanged.
+// The persistent lane loop of the kernels (feeder, refill, step totals), inlined into each.
+template <int MODE, bool BOUNCE, bool SINK, bool ION, bool TRACE = false>
 __device__ __forceinline__ void
 adaptive_lanes(const StateCols& In, const StateCols& P, long long n, const RunParams& p,
                const InterpTable& Tg, const FastTable& Fg, const unsigned* __restrict__ perm,
                unsigned long long* __restrict__ queue, unsigned long long* __restrict__ totals,
                unsigned* __restrict__ att_out, unsigned* __restrict__ acc_out,
                int* __restrict__ status, unsigned table_bytes, const Spline2D& S, uint64_t seed,
-               uint64_t first_id, const DepositOut& Dep, const IonOut& Ion) {
+               uint64_t first_id, const DepositOut& Dep, const IonOut& Ion,
+               const TraceOut* Tro = nullptr) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   InterpTable T;
   FastTable F;
@@ -341,6 +347,8 @@ adaptive_lanes(const StateCols& In, const StateCols& P, long long n, const RunPa
   }
   IonSink I;                     // ION: lives in local memory, the grid read by ion_record
   if (ION) { I.g = Ion; I.out_sum = 0.0; I.out_n = 0; }
+  TraceSink Tr;                  // TRACE: lives in local memory, the launch's sink read through o
+  if (TRACE) { Tr.o = Tro; Tr.age0 = 0.0; Tr.out_sum = 0.0; Tr.out_n = 0; }
 #ifdef NX_STREAM_DEBUG
   unsigned long long dbg_iters = 0;
 #endif
@@ -360,6 +368,7 @@ adaptive_lanes(const StateCols& In, const StateCols& P, long long n, const RunPa
         idx = feed.ids[feed.buf * 32 + slot];
         att = 0; acc = 0;
         have = (s[0] > p.resolution) && (s[7] > 0.0);
+        if (TRACE && have) Tr.age0 = sub_rn(Tro->endtime, s[0]);
         if (SINK && s[7] > 0.0) {
           D.sum[DEP_SOURCE] += s[7]; ++D.n[DEP_SOURCE];
           if (!have) { D.sum[DEP_REMAINING] += s[7]; ++D.n[DEP_REMAINING]; }
@@ -384,13 +393,16 @@ adaptive_lanes(const StateCols& In, const StateCols& P, long long n, const RunPa
     if (have) {
       int fl;
       if (MODE < 0)
-        fl = adaptive_attempt<true, BOUNCE, SINK, ION>(p, T, s, step, &S, seed, first_id + idx,
-                                                       acc + 1, SINK ? &D : nullptr,
-                                                       ION ? &I : nullptr);
+        fl = adaptive_attempt<true, BOUNCE, SINK, ION, TRACE>(p, T, s, step, &S, seed,
+                                                              first_id + idx, acc + 1,
+                                                              SINK ? &D : nullptr,
+                                                              ION ? &I : nullptr,
+                                                              TRACE ? &Tr : nullptr);
       else
         fl = adaptive_attempt_fast<(MODE >> 3) & 1, (MODE >> 2) & 1, MODE & 3, (MODE >> 4) & 1, BOUNCE,
-                                   SINK, ION>(p, F, s, step, &S, seed, first_id + idx, acc + 1,
-                                              SINK ? &D : nullptr, ION ? &I : nullptr);
+                                   SINK, ION, TRACE>(p, F, s, step, &S, seed, first_id + idx,
+                                                     acc + 1, SINK ? &D : nullptr,
+                                                     ION ? &I : nullptr, TRACE ? &Tr : nullptr);
       ++att;
       if (fl & ATT_ACCEPTED) ++acc;
       if (BOUNCE && (fl & ATT_BOUNCED)) ++tot_bnc;
@@ -455,6 +467,21 @@ adaptive_lanes(const StateCols& In, const StateCols& P, long long n, const RunPa
       atomicAdd(Ion.cnt + out, c);
     }
   }
+  if (TRACE && Tro->grid.sum) {
+    double v = Tr.out_sum;
+    unsigned long long c = Tr.out_n;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      v += __shfl_xor_sync(FULL_MASK, v, o);
+      c += __shfl_xor_sync(FULL_MASK, c, o);
+    }
+    if (lane == 0 && c) {
+      const IonOut& g = Tro->grid;
+      const long long out = (long long)g.n[0] * g.n[1] * g.n[2];
+      atomicAdd(g.sum + out, v);
+      atomicAdd(g.cnt + out, c);
+    }
+  }
 }
 
 template <int MODE, bool BOUNCE = false, bool SINK = false>
@@ -485,6 +512,23 @@ k_ionize_adaptive(StateCols In, StateCols P, long long n, RunParams p, InterpTab
   adaptive_lanes<MODE, BOUNCE, false, true>(In, P, n, p, Tg, Fg, perm, queue, totals, att_out,
                                             acc_out, status, table_bytes, S, seed, first_id,
                                             DepositOut{}, Ion);
+}
+
+// K2t: the adaptive driver with the trajectory sink (ModelTrajectoryImage /
+// ModelTrajectoryDensity).  Built for every kernel the dispatch selects for a run without
+// moons: the fast MODEs without bit 16, with and without bounce, and the strict kernel.
+template <int MODE, bool BOUNCE>
+__global__ void __launch_bounds__(NX_INT_THREADS, NX_INT_MINBLOCKS)
+k_trace_adaptive(StateCols In, StateCols P, long long n, RunParams p, InterpTable Tg,
+                 FastTable Fg, const unsigned* __restrict__ perm,
+                 unsigned long long* __restrict__ queue,
+                 unsigned long long* __restrict__ totals,
+                 unsigned* __restrict__ att_out, unsigned* __restrict__ acc_out,
+                 int* __restrict__ status, unsigned table_bytes, Spline2D S, uint64_t seed,
+                 uint64_t first_id, const __grid_constant__ TraceOut Tro) {
+  adaptive_lanes<MODE, BOUNCE, false, false, true>(In, P, n, p, Tg, Fg, perm, queue, totals,
+                                                   att_out, acc_out, status, table_bytes, S, seed,
+                                                   first_id, DepositOut{}, IonOut{}, &Tro);
 }
 
 // ---------------------------------------------------------------------------
@@ -1611,6 +1655,8 @@ static cudaError_t persistent_grid(K kernel, int device, size_t smem, int* block
 constexpr bool ion_build(int mode) {
   return mode < 0 || (mode & 3) == LOSS_LIFETIME || (mode & 3) == LOSS_PHOTO;
 }
+// the trace builds: the kernels without a moon (MODE bit 16) and the strict kernels
+constexpr bool trace_build(int mode) { return mode < 0 || !(mode & 16); }
 
 template <typename K, typename... Args>
 static cudaError_t launch_lanes(K kernel, cudaStream_t st, int device, size_t smem, long long n,
@@ -1625,7 +1671,8 @@ static cudaError_t launch_lanes(K kernel, cudaStream_t st, int device, size_t sm
 }
 
 // Ion != nullptr: the same run through k_ionize_adaptive<MODE, BOUNCE> (SINK false, MODE with
-// a loss term), so the ion run selects its build by the dispatch of the plain run.
+// a loss term), so the ion run selects its build by the dispatch of the plain run; Trace !=
+// nullptr: through k_trace_adaptive<MODE, BOUNCE> (SINK false, MODE without a moon) alike.
 template <int MODE, bool BOUNCE = false, bool SINK = false>
 static cudaError_t launch_adaptive_mode(cudaStream_t st, int device, StateCols In, StateCols P,
                                         long long n,
@@ -1635,7 +1682,7 @@ static cudaError_t launch_adaptive_mode(cudaStream_t st, int device, StateCols I
                                         unsigned long long* totals, unsigned* att, unsigned* acc,
                                         int* status, const Spline2D& S, uint64_t seed,
                                         uint64_t first_id, const DepositOut& Dep,
-                                        const IonOut* Ion) {
+                                        const IonOut* Ion, const TraceOut* Trace) {
   const size_t tbytes = (MODE < 0) ? table_smem_bytes(T) : fast_table_smem_bytes(F);
   const size_t smem = tbytes + (size_t)(NX_INT_THREADS / 32) * NX_FEED_BYTES_PER_WARP;
   if constexpr (!SINK && ion_build(MODE)) {
@@ -1645,6 +1692,13 @@ static cudaError_t launch_adaptive_mode(cudaStream_t st, int device, StateCols I
                           first_id, *Ion);
   }
   if (Ion) return cudaErrorInvalidValue;         // no ion build: a run without loss
+  if constexpr (!SINK && trace_build(MODE)) {
+    if (Trace)
+      return launch_lanes(k_trace_adaptive<MODE, BOUNCE>, st, device, smem, n, In, P, n, p, T, F,
+                          perm, queue, totals, att, acc, status, (unsigned)tbytes, S, seed,
+                          first_id, *Trace);
+  }
+  if (Trace) return cudaErrorInvalidValue;       // no trace build: a run with a moon
   return launch_lanes(k_integrate_adaptive<MODE, BOUNCE, SINK>, st, device, smem, n, In, P, n, p,
                       T, F, perm, queue, totals, att, acc, status, (unsigned)tbytes, S, seed,
                       first_id, Dep);
@@ -1752,7 +1806,8 @@ cudaError_t launch_cost_order(cudaStream_t st, int device, StateCols P, long lon
 }
 
 // K2 / K2b kernel selection; SINK builds exist for every kernel it can select, ion builds
-// (Ion != nullptr, SINK false) for those of them with a loss term.
+// (Ion != nullptr, SINK false) for those of them with a loss term, trace builds (Trace !=
+// nullptr, SINK false) for those of them without a moon.
 template <bool SINK>
 static cudaError_t dispatch_adaptive(cudaStream_t st, int device, StateCols In, StateCols P,
                                      long long n, const RunParams& p, const InterpTable& T,
@@ -1760,9 +1815,10 @@ static cudaError_t dispatch_adaptive(cudaStream_t st, int device, StateCols In, 
                                      unsigned long long* queue, unsigned long long* totals,
                                      unsigned* att, unsigned* acc, int* status,
                                      const Spline2D* S, uint64_t seed, uint64_t first_id,
-                                     const DepositOut& Dep, const IonOut* Ion) {
+                                     const DepositOut& Dep, const IonOut* Ion,
+                                     const TraceOut* Trace) {
 #define NX_ARGS st, device, In, P, n, p, T, F, perm, queue, totals, att, acc, status, \
-                S ? *S : Spline2D{}, seed, first_id, Dep, Ion
+                S ? *S : Spline2D{}, seed, first_id, Dep, Ion, Trace
   if (S) {
     // bounce builds: the strict kernel, and the fast kernels with gravity (one moon too);
     // runs without gravity or with more moons take the strict kernel
@@ -1817,13 +1873,14 @@ cudaError_t launch_integrate_adaptive(cudaStream_t st, int device, StateCols In,
                                       unsigned long long* queue, unsigned long long* totals,
                                       unsigned* att, unsigned* acc, int* status,
                                       const Spline2D* S, uint64_t seed, uint64_t first_id,
-                                      const DepositOut* dep, const IonOut* ion) {
-  if (dep && ion) return cudaErrorInvalidValue;
+                                      const DepositOut* dep, const IonOut* ion,
+                                      const TraceOut* trace) {
+  if ((dep != nullptr) + (ion != nullptr) + (trace != nullptr) > 1) return cudaErrorInvalidValue;
   if (dep)
     return dispatch_adaptive<true>(st, device, In, P, n, p, T, F, perm, queue, totals, att, acc,
-                                   status, S, seed, first_id, *dep, nullptr);
+                                   status, S, seed, first_id, *dep, nullptr, nullptr);
   return dispatch_adaptive<false>(st, device, In, P, n, p, T, F, perm, queue, totals, att, acc,
-                                  status, S, seed, first_id, DepositOut{}, ion);
+                                  status, S, seed, first_id, DepositOut{}, ion, trace);
 }
 
 template <int MODE>

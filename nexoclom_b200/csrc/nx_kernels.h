@@ -148,6 +148,8 @@ struct DepositOut {
 // dep != nullptr: the same run through the kernel's SINK build, which adds its events to *dep.
 // ion != nullptr (dep == nullptr, a run with a loss term): the same run through
 // k_ionize_adaptive, which adds the frac lost in flight to the grid *ion.
+// trace != nullptr (the others nullptr, a run without moons): the same run through
+// k_trace_adaptive, which adds every accepted step to the image and / or grid of *trace.
 cudaError_t launch_integrate_adaptive(cudaStream_t st, int device, StateCols In, StateCols P,
                                       long long n, const RunParams& p, const InterpTable& T,
                                       const FastTable& F, const unsigned* perm,
@@ -155,7 +157,8 @@ cudaError_t launch_integrate_adaptive(cudaStream_t st, int device, StateCols In,
                                       unsigned* att, unsigned* acc, int* status,
                                       const Spline2D* S = nullptr, uint64_t seed = 0,
                                       uint64_t first_id = 0, const DepositOut* dep = nullptr,
-                                      const IonOut* ion = nullptr);
+                                      const IonOut* ion = nullptr,
+                                      const TraceOut* trace = nullptr);
 #define NX_STREAM_GROUP 128          // == NX_GROUP: segment sizes are multiples of this
 #define NX_STREAM_MAX_SEG 32
 #define NX_STREAM_CURSORS 256        // >= NX_NCLASS x 32 u64 cursors

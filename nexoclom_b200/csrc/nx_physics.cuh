@@ -477,6 +477,26 @@ struct IonSink {
 template <class Sink>
 NX_COLD void ion_record(Sink& I, double loss, double x, double y, double z);
 
+// The trajectory sink (TRACE builds of the adaptive driver, ModelTrajectoryImage /
+// ModelTrajectoryDensity): an image and / or a grid that every accepted step adds to, weighted
+// by the time the packet spends on it.  TraceOut (nx_image.cuh) is the launch's image, grid and
+// g-value tables; the lane keeps age0 = T - t0 of the packet it holds (T = endtime, t0 = its
+// initial time remaining) and its OUTSIDE share of the grid, reduced when the kernel ends.
+struct TraceOut;
+struct TraceSink {
+  const TraceOut* o;
+  double age0;
+  double out_sum;
+  unsigned long long out_n;
+};
+
+// Records one accepted step of length h from time remaining t, at the midpoint (x, y, z, vy,
+// frac) of the state before it and the Runge-Kutta state.  Defined in nx_image.cuh, an
+// out-of-line call like ion_record().
+template <class Sink>
+NX_COLD void trace_record(Sink& Tr, double x, double y, double z, double vy, double frac,
+                          double h, double t);
+
 // BOUNCE = false: the reference's driver (a packet that hits the surface sticks, Q6).
 // BOUNCE = true: accepted steps that end inside the planet go through adaptive_surface()
 // unless the sticking is perfect; S / seed / id / k feed it (unused otherwise).
@@ -485,10 +505,15 @@ NX_COLD void ion_record(Sink& I, double loss, double x, double y, double z);
 // ION = true: every accepted step that changes the frac goes to ion_record(*I) with
 // frac before - frac of the Runge-Kutta step, at the midpoint of the step's chord (before a
 // bounce moves the packet); the state is again the same as without it.
-template <bool STRICT, bool BOUNCE = false, bool SINK = false, bool ION = false>
+// TRACE = true: every accepted step goes to trace_record(*Tr) with its length, the time
+// remaining before it and the midpoint of the state before it and the Runge-Kutta state (each
+// component (s + s_rk) * 0.5, before any surface, moon, escape or vanish handling).
+template <bool STRICT, bool BOUNCE = false, bool SINK = false, bool ION = false,
+          bool TRACE = false>
 NX_HD int adaptive_attempt(const RunParams& p, const InterpTable& T, double* s, double& step,
                            const Spline2D* S = nullptr, uint64_t seed = 0, uint64_t id = 0,
-                           uint32_t k = 0, DepositSink* D = nullptr, IonSink* I = nullptr) {
+                           uint32_t k = 0, DepositSink* D = nullptr, IonSink* I = nullptr,
+                           TraceSink* Tr = nullptr) {
   const double res = p.resolution;
   const double resv = mul_rn(0.1, res);
   const double h = fmin(s[0], step);
@@ -519,6 +544,10 @@ NX_HD int adaptive_attempt(const RunParams& p, const InterpTable& T, double* s, 
         ion_record(*I, loss, mul_rn(add_rn(s[1], nx[1]), 0.5), mul_rn(add_rn(s[2], nx[2]), 0.5),
                    mul_rn(add_rn(s[3], nx[3]), 0.5));
     }
+    if (TRACE)
+      trace_record(*Tr, mul_rn(add_rn(s[1], nx[1]), 0.5), mul_rn(add_rn(s[2], nx[2]), 0.5),
+                   mul_rn(add_rn(s[3], nx[3]), 0.5), mul_rn(add_rn(s[5], nx[5]), 0.5),
+                   mul_rn(add_rn(s[7], nx[7]), 0.5), h, s[0]);
     const double r2 = add_rn(add_rn(mul_rn(nx[1], nx[1]), mul_rn(nx[2], nx[2])), mul_rn(nx[3], nx[3]));
     double f = nx[7];
     double dep = 0.0, ff = 0.0;            // SINK: deposited frac, frac of the fate event

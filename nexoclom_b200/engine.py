@@ -12,7 +12,7 @@ import numpy as np
 from . import _lib
 from ._lib import (RunParams, SourceParams, ImageParams, LosParams, SpectrumParams, as_f64,
                    dptr, c_double_p, NX_PRODUCT_IMAGE, NX_PRODUCT_CUBE, NX_PRODUCT_DEPOSIT,
-                   NX_PRODUCT_IONIZE)
+                   NX_PRODUCT_IONIZE, NX_PRODUCT_TRACE)
 
 STATE_COLS = ('time', 'x', 'y', 'z', 'vx', 'vy', 'vz', 'frac')
 X0_COLS = ('time', 'x', 'y', 'z', 'vx', 'vy', 'vz', 'frac', 'v', 'longitude', 'latitude',
@@ -622,6 +622,63 @@ class Engine:
     def ionize_end(self):
         """Release the ion-production grid's device memory."""
         self._product_end(NX_PRODUCT_IONIZE)
+
+    def trace_begin(self, image_params=None, grid=None):
+        """Allocate and zero the context-owned trajectory sink: an image (``image_params``, an
+        ``ImageParams``, or None) and / or a grid (``grid`` = (lo, hi, dims) as for
+        ``ionize_begin``, or None), until ``trace_end``."""
+        g = None
+        if grid is not None:
+            lo, hi, dims = grid
+            g = _lib.IonGrid()
+            for k in range(3):
+                g.lo[k], g.hi[k], g.n[k] = float(lo[k]), float(hi[k]), int(dims[k])
+        self._check(self.lib.nx_trace_begin(self.ctx,
+                                            None if image_params is None else C.byref(image_params),
+                                            None if g is None else C.byref(g)), 'nx_trace_begin')
+        self._trace_shape = ((0, 0) if image_params is None else
+                             (int(image_params.nx), int(image_params.nz)),
+                             None if grid is None else tuple(int(d) for d in grid[2]))
+
+    def integrate_adaptive_trace(self, seed, first_id=0, n=None):
+        """K2 on the resident packets through its trajectory sink: the run
+        ``integrate_adaptive_ionize`` would make, every accepted step added to the image and / or
+        grid of ``trace_begin`` at its midpoint, weighted by its age-weighted dwell.  Returns
+        (attempted, accepted, bounces)."""
+        att, acc, bnc = C.c_ulonglong(), C.c_ulonglong(), C.c_ulonglong()
+        n = self.n if n is None else n
+        self._check(self.lib.nx_integrate_adaptive_trace(self.ctx, int(n), int(seed),
+                                                         int(first_id), C.byref(att),
+                                                         C.byref(acc), C.byref(bnc)),
+                    'nx_integrate_adaptive_trace')
+        return int(att.value), int(acc.value), int(bnc.value)
+
+    def trace_fetch(self):
+        """(image, image_counts, grid, grid_counts, outside, outside_count): the (nx, nz) image
+        sums (float64) and recorded steps (int64), the (gx, gy, gz) grid's sums and steps, then
+        OUTSIDE's sum and count; the parts ``trace_begin`` did not ask for are None."""
+        (nx, nz), gdims = self._trace_shape
+        npix = nx * nz
+        ncell = 0 if gdims is None else gdims[0] * gdims[1] * gdims[2]
+        nslot = npix + (0 if gdims is None else ncell + 1)
+        sums, cnt = self._product_fetch(NX_PRODUCT_TRACE, (nslot,))
+        img = img_n = grid = grid_n = outside = outside_n = None
+        if npix:
+            img, img_n = sums[:npix].reshape(nx, nz), cnt[:npix].reshape(nx, nz)
+        if gdims is not None:
+            grid = sums[npix:npix + ncell].reshape(gdims)
+            grid_n = cnt[npix:npix + ncell].reshape(gdims)
+            outside, outside_n = float(sums[npix + ncell]), int(cnt[npix + ncell])
+        return img, img_n, grid, grid_n, outside, outside_n
+
+    def trace_allreduce(self, comm, total):
+        """Sum the trajectory sink over the ranks of ``comm`` in place, with one scalar riding
+        along; returns the summed scalar."""
+        return self._product_allreduce(NX_PRODUCT_TRACE, comm, total)
+
+    def trace_end(self):
+        """Release the trajectory sink's device memory."""
+        self._product_end(NX_PRODUCT_TRACE)
 
     # -- context-owned accumulators (nx_product) --------------------------------
     def _product_fetch(self, which, shape):
